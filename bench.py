@@ -6,10 +6,11 @@ such frames per step.
 
     python bench.py --gpus N --steps K --warmup W          # ours (CUDA, sm_100a)
     python bench.py --impl reference ...                    # reference CPU path on host cores
+    python bench.py ... --dump-outputs DIR                  # + the last timed step's results as DIR/<name>.npy
 
 One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for the definition of every
-field.  Nothing here reads /root/reference; the CPU arms use oracle/_ref (the reference's
-own ops, prebuilt) and the oracle restatement of the seeker loop.
+field.  Nothing here reads the reference's source tree; the CPU arms use oracle/_ref (the
+reference's own ops, prebuilt) and the oracle restatement of the seeker loop.
 """
 import argparse
 import collections
@@ -30,7 +31,7 @@ sys.path.insert(0, os.path.join(ROOT, "oracle"))
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 20)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default="cfg2")
@@ -40,7 +41,7 @@ def parse():
     ap.add_argument("--distinct", type=int, default=256, help="distinct synthetic frames per rank (weak scaling) / in the pool (--total-frames)")
     ap.add_argument("--total-frames", type=int, default=0,
                     help="strong scaling, BASELINE.json configs[3]: this many frames in all, sharded rank::world "
-                         "(6019 = the nuScenes val sweep); steps = ceil(shard / frames), --steps is ignored")
+                         "(6019 = the nuScenes val sweep); steps = ceil(shard / frames), so --steps is refused")
     ap.add_argument("--layout", default="xyz", choices=["xyz", "rows"],
                     help="point table the loader hands over: x,y,z as its own array (12 B/point, no gather) or the "
                          "reference's rows (5 columns; the e2e arm gathers x,y,z on the host)")
@@ -52,7 +53,67 @@ def parse():
     ap.add_argument("--pack-threads", type=int, default=None)
     ap.add_argument("--slots", type=int, default=3, help="batches in flight on the device (streams + arenas), resident arm")
     ap.add_argument("--opt", action="append", default=[], help="name=value tuning switch (fnp_set_option), A/B runs only")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step of the timed (resident) run returned -- "
+                         "proposals, per-candidate results, recall counters -- as DIR/<name>.npy (float32 / float64, "
+                         "rank 0), to compare two builds output for output; a seeded sample of the frames above 64 MB")
+    a = ap.parse_args()
+    if a.total_frames > 0 and a.steps is not None:
+        ap.error("--total-frames sets the number of timed steps; leave out --steps")
+    if a.impl == "reference" and a.dump_outputs:
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl ours)")
+    a.steps = 20 if a.steps is None else a.steps
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return a
+
+
+# --------------------------------------------------------------------------- outputs
+def dump_outputs(out_dir, res, plan, limit=64 << 20):
+    """SeekerEngine.finish's result of one batch as .npy files: per proposal (frames back to back) boxes, 2D scores,
+    labels, stage-4 keep flags; per candidate frustum validity, point / valid-hypothesis counts and the best
+    hypothesis (zero where invalid; with topk > 1 these hold slot 0, the per-proposal arrays every slot); the recall
+    counters in the engine's order (RECALL_KEYS, then RECALL_PER_THRESH per IoU threshold).  Integers are stored as
+    float64 (exact).  Above `limit` bytes, the frames are a seeded sample (frame_index says which); the recall
+    counters always count the whole batch."""
+    n_frames = len(res["frames"])
+    fcs = plan["frame_cand_start"]
+
+    def arrays(frames):
+        fr = [res["frames"][b] for b in frames]
+        cand = np.concatenate([np.arange(fcs[b], fcs[b + 1]) for b in frames]).astype(np.int64)
+        valid = res["cand_valid"][cand]
+        f64 = lambda x: np.asarray(x, np.float64)                               # noqa: E731
+        out = {
+            "frame_index": f64(frames),
+            "frame_pred_count": f64([f["pred_boxes"].shape[0] for f in fr]),
+            "frame_cand_count": f64(np.diff(fcs)[frames]),
+            "pred_boxes": np.concatenate([f["pred_boxes"] for f in fr]).astype(np.float32).reshape(-1, 7),
+            "pred_scores": np.concatenate([f["pred_scores"] for f in fr]).astype(np.float32),
+            "pred_labels": f64(np.concatenate([f["pred_labels"] for f in fr])),
+            "cand_valid": valid.astype(np.float32),
+            "cand_npts": f64(res["cand_npts"][cand]),
+            "cand_nvalid": f64(res["cand_nvalid"][cand]),
+            "cand_boxes": np.where(valid[:, None], res["cand_boxes"][cand], 0).astype(np.float32),
+            "cand_score2": np.where(valid, res["cand_score2"][cand], 0).astype(np.float32),
+            "cand_best": f64(np.where(valid, res["cand_best"][cand], 0)),
+            "cand_count": f64(np.where(valid, res["cand_count"][cand], 0)),
+        }
+        if fr and "nms_keep" in fr[0]:
+            out["pred_nms_keep"] = np.concatenate([f["nms_keep"] for f in fr]).astype(np.float32)
+        if "recall" in res:
+            out["recall"] = f64(list(res["recall"].values()))
+        return out
+
+    frames = np.arange(n_frames)
+    out = arrays(frames)
+    rng = np.random.default_rng(0)
+    while sum(v.nbytes for v in out.values()) > limit and len(frames) > 1:
+        frames = np.sort(rng.choice(n_frames, len(frames) // 2, replace=False))
+        out = arrays(frames)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 # --------------------------------------------------------------------------- clocks
@@ -460,12 +521,13 @@ def run_ours(a):
         return xbuf["allp"], xbuf["allc"], rc
 
     def drain(prev):
+        """Finishes the batches still in flight; returns (result, plan) of the newest one."""
         last = None
         while prev:
             old = prev.popleft()
-            last = eng.finish(old)
+            last = eng.finish(old), old["plan"]
             if world > 1:
-                exchange_add(last, old["plan"])
+                exchange_add(last[0], old["plan"])
         return last
 
     gathered = {}
@@ -749,6 +811,8 @@ def run_ours(a):
         if cpu is not None:
             line["cpu_baseline"] = cpu
         print(json.dumps(line), flush=True)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, *last)
     if world > 1:
         dist.destroy_process_group()
 

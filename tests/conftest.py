@@ -20,10 +20,14 @@ def golden_dir():
 
 @pytest.fixture(scope="session")
 def ref_ops():
-    """The reference's own compiled ops (oracle/_ref); skip when they were not built."""
+    """The reference's own compiled ops (oracle/_ref), or None where they were not built: the tests then compare with
+    the reference's outputs stored in tests/golden and with the C oracle, and say so in a warning."""
+    import warnings
+
     import build_ref
     try:
         return build_ref.load("roiaware_pool3d_cuda"), build_ref.load("iou3d_nms_cuda")
-    except ImportError as e:  # pragma: no cover
-        pytest.skip(str(e))
+    except ImportError as e:
+        warnings.warn("%s: the op tests compare with the reference's stored outputs and the C oracle only" % e)
+        return None
 

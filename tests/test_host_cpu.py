@@ -204,13 +204,31 @@ def test_batch_planner_in_c_equals_the_numpy_path():
     assert fis[0]._prep is None and fis[0].prepare() is not p0
 
 
-def test_cpu_op_box_constants_reproduce_the_reference_cpu_op(ref_ops):
+def test_cpu_op_box_constants_reproduce_the_reference_cpu_op(ref_ops, golden_dir):
     """fnp_host_prep_boxes_cpu (the host half of the device-executed points_in_boxes_cpu): with its constants, the
     rounded fp32 arithmetic the device kernel performs -- emulated here in numpy, one rounding per operation --
-    gives the reference-compiled CPU op's matrix bit for bit, also for points within a few ulp of dx/2 + 1e-2."""
+    gives the reference-compiled CPU op's matrix bit for bit, also for points within a few ulp of dx/2 + 1e-2.
+    Without the compiled op: its matrix on the stored inputs (tests/golden), and the oracle's port of it on these."""
     import ctypes as C
+    import oracle as O
     from findnpropagate_b200 import _lib
-    ref_rp, _ = ref_ops
+
+    def emulated(boxes, pts):
+        n = boxes.shape[0]
+        prep = np.zeros((n, 8), np.float32)
+        assert _lib.lib.fnp_host_prep_boxes_cpu(C.c_void_p(boxes.ctypes.data), C.c_void_p(prep.ctypes.data), n) == 0
+        f = np.float32
+        sx = (pts[None, :, 0] - prep[:, None, 0]).astype(f)
+        sy = (pts[None, :, 1] - prep[:, None, 1]).astype(f)
+        sz = (pts[None, :, 2] - prep[:, None, 2]).astype(f)
+        cosa, sina = prep[:, None, 4], prep[:, None, 5]
+        lxx = ((sx * cosa).astype(f) + (sy * -sina).astype(f)).astype(f)
+        lyy = ((sx * sina).astype(f) + (sy * cosa).astype(f)).astype(f)
+        inside = ~(np.abs(sz) > prep[:, None, 3]) & (np.abs(lxx) <= prep[:, None, 6]) & (np.abs(lyy) <= prep[:, None, 7])
+        return inside.astype(np.int32)
+
+    g = np.load(os.path.join(golden_dir, "ops_cpu_reference.npz"))
+    assert np.array_equal(emulated(np.ascontiguousarray(g["boxes"]), g["pts"]), g["pib_cpu"])
     rng = np.random.default_rng(3)
     n = 40
     boxes = np.zeros((n, 7), np.float32)
@@ -225,20 +243,15 @@ def test_cpu_op_box_constants_reproduce_the_reference_cpu_op(ref_ops):
     ca, sa = np.cos(b[:, 6]), np.sin(b[:, 6])
     pts = np.stack([b[:, 0] + lx * ca - ly * sa, b[:, 1] + lx * sa + ly * ca, b[:, 2] + rng.uniform(-0.5, 0.5, 4000) * b[:, 5]], 1)
     pts = np.concatenate([pts, rng.uniform(-25, 25, (4000, 3))]).astype(np.float32)
-    want = torch.zeros((n, pts.shape[0]), dtype=torch.int32)
-    ref_rp.points_in_boxes_cpu(torch.from_numpy(boxes), torch.from_numpy(pts), want)
-    prep = np.zeros((n, 8), np.float32)
-    assert _lib.lib.fnp_host_prep_boxes_cpu(C.c_void_p(boxes.ctypes.data), C.c_void_p(prep.ctypes.data), n) == 0
-    f = np.float32
-    sx = (pts[None, :, 0] - prep[:, None, 0]).astype(f)
-    sy = (pts[None, :, 1] - prep[:, None, 1]).astype(f)
-    sz = (pts[None, :, 2] - prep[:, None, 2]).astype(f)
-    cosa, sina = prep[:, None, 4], prep[:, None, 5]
-    lxx = ((sx * cosa).astype(f) + (sy * -sina).astype(f)).astype(f)
-    lyy = ((sx * sina).astype(f) + (sy * cosa).astype(f)).astype(f)
-    got = ~(np.abs(sz) > prep[:, None, 3]) & (np.abs(lxx) <= prep[:, None, 6]) & (np.abs(lyy) <= prep[:, None, 7])
-    assert np.array_equal(got.astype(np.int32), want.numpy()), int((got.astype(np.int32) != want.numpy()).sum())
-    assert want.numpy().sum() > 2000
+    if ref_ops is not None:
+        want = torch.zeros((n, pts.shape[0]), dtype=torch.int32)
+        ref_ops[0].points_in_boxes_cpu(torch.from_numpy(boxes), torch.from_numpy(pts), want)
+        want = want.numpy()
+    else:
+        want = O.points_in_boxes_cpu(pts, boxes)
+    got = emulated(boxes, pts)
+    assert np.array_equal(got, want), int((got != want).sum())
+    assert want.sum() > 2000
 
 
 def test_shipped_yaml_params_equal_the_hard_coded_ones():
