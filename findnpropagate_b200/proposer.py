@@ -73,6 +73,10 @@ class PreprocessedGLIP:
             self.token_to_id[image['token']] = img_id
             self.path_to_id[image['file_name']] = img_id
 
+    def has_image(self, path) -> bool:
+        """Whether ``infer_nusc`` finds the camera image ``path`` in the prediction file."""
+        return str(path) in self.path_to_id
+
     def infer_nusc(self, batch_dict):
         labels, boxes, scores, idx, cam_idx = [], [], [], [], []
         for b in range(batch_dict['batch_size']):
@@ -167,9 +171,15 @@ class PreprocessedDetector:
                 torch.from_numpy(np.concatenate(scores)), torch.from_numpy(np.concatenate(idx)),
                 torch.from_numpy(np.concatenate(cam)))
 
+    def _image_name(self, path) -> str:
+        return os.path.basename(str(path)) if self.incl_ext else os.path.splitext(os.path.basename(str(path)))[0]
+
+    def has_image(self, path) -> bool:
+        """Whether the result files list the camera image ``path``."""
+        return self._image_name(path) in self.by_name
+
     def infer_nusc(self, batch_dict):
-        names = [[(os.path.basename(str(p)) if self.incl_ext else os.path.splitext(os.path.basename(str(p)))[0])
-                  for p in batch_dict['image_paths'][b]] for b in range(batch_dict['batch_size'])]
+        names = [[self._image_name(p) for p in batch_dict['image_paths'][b]] for b in range(batch_dict['batch_size'])]
         return self._collect(names, [range(len(n)) for n in names])
 
     def infer_kitti(self, batch_dict):

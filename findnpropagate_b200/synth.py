@@ -325,6 +325,30 @@ def write_nuscenes_tree(root, frames):
     return infos
 
 
+def write_glip_predictions(frames, pred_pth, meta_coco):
+    """Write the detections of synthetic frames as the GLIP prediction file (a pickled list of BoxList, one per camera
+    image) and its COCO meta json (``images`` with ``token`` and ``file_name``) that proposer.PreprocessedGLIP
+    reads (preprocessed_detector.py:11-45)."""
+    import json
+    import os
+    from .proposer import BoxList, install_boxlist_shim
+    install_boxlist_shim()
+    lists, images = [], []
+    for f in frames:
+        for c in range(6):
+            m = np.asarray(f.det_cam_idx) == c
+            bl = BoxList(torch.from_numpy(np.asarray(f.det_boxes, np.float32)[m].reshape(-1, 4)), (IMG_W, IMG_H))
+            bl.extra_fields = dict(scores=torch.from_numpy(np.asarray(f.det_scores, np.float32)[m]),
+                                   labels=torch.from_numpy(np.asarray(f.det_labels, np.int64)[m]))
+            lists.append(bl)
+            images.append(dict(id=len(images), token=f.token, file_name=str(f.image_paths[c])))
+    for p in (pred_pth, meta_coco):
+        os.makedirs(os.path.dirname(os.path.abspath(p)), exist_ok=True)
+    torch.save(lists, pred_pth)
+    with open(meta_coco, "w") as fh:
+        json.dump(dict(images=images, categories=[dict(id=i + 1, name=n) for i, n in enumerate(CLASS_NAMES)]), fh)
+
+
 def make_kitti_frame(index):
     """A KITTI-shaped frame: points in front of the sensor, P2 / R0 / Tr_velo2cam, x-y-w-h 2D boxes of the visible
     synthetic objects, labels 1..7 (the KITTI head's seven anchors)."""
