@@ -575,6 +575,54 @@ __global__ void __launch_bounds__(256) recall_kernel(const float *__restrict__ p
     }
 }
 
+// Precision counters: per valid proposal the largest IoU3D over its frame's GT boxes (the IoU of recall_kernel),
+// thresholded.  One CTA per frame.
+__global__ void __launch_bounds__(256) precision_kernel(const float *__restrict__ pred, const int32_t *__restrict__ pred_valid,
+                                                        const int32_t *__restrict__ pred_start,
+                                                        const float *__restrict__ gt, const int32_t *__restrict__ gt_start,
+                                                        int n_thresh, float t0, float t1, float t2, float t3, float t4,
+                                                        float t5, float t6, float t7, long long *__restrict__ counters)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const float thr[8] = {t0, t1, t2, t3, t4, t5, t6, t7};
+    const int fr = blockIdx.x;
+    const int p0 = pred_start[fr], K = pred_start[fr + 1] - p0;
+    const int g0 = gt_start[fr], G = gt_start[fr + 1] - g0;
+    if (K <= 0) return;
+    RBox *s_g = reinterpret_cast<RBox *>(smem);          // [G]
+    RBox *s_p = s_g + G;                                  // [K]
+    int *s_best = reinterpret_cast<int *>(s_p + K);       // [K] float bits; IoU >= 0 orders like int
+    for (int i = threadIdx.x; i < G; i += blockDim.x) s_g[i] = prep_rbox(gt + (size_t)(g0 + i) * 8);
+    for (int i = threadIdx.x; i < K; i += blockDim.x) {
+        s_p[i] = prep_rbox(pred + (size_t)(p0 + i) * 7);
+        if (pred_valid && pred_valid[p0 + i] < 0) s_p[i].pad = -1.f;   // not a proposal
+        s_best[i] = __float_as_int(-1.f);
+    }
+    __syncthreads();
+    for (int q = threadIdx.x; q < G * K; q += blockDim.x) {
+        const int k = q / G, gi = q - k * G;
+        if (s_p[k].pad < 0.f) continue;
+        float iou = 0.f;
+        if (!surely_disjoint(s_p[k], s_g[gi]))
+            iou = iou3d_from_overlap(pred + (size_t)(p0 + k) * 7, gt + (size_t)(g0 + gi) * 8, box_overlap(s_p[k], s_g[gi]));
+        if (iou >= 0.f) atomicMax(&s_best[k], __float_as_int(iou));
+    }
+    __syncthreads();
+    long long local[1 + 8];
+    for (int i = 0; i < 1 + 8; i++) local[i] = 0;
+    for (int k = threadIdx.x; k < K; k += blockDim.x) {
+        if (s_p[k].pad < 0.f) continue;
+        local[0]++;
+        const float best = __int_as_float(s_best[k]);
+        for (int t = 0; t < n_thresh; t++) local[1 + t] += best > thr[t];
+    }
+    for (int i = 0; i < 1 + n_thresh; i++) {
+        long long v = local[i];
+        for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if ((threadIdx.x & 31) == 0 && v) atomicAdd(reinterpret_cast<unsigned long long *>(counters + i), (unsigned long long)v);
+    }
+}
+
 // Small host->device upload executed by SMs: `src` is pinned (page-locked, UVA-mapped) host
 // memory.  Used for the per-batch metadata so that it does not queue behind a large point
 // copy in the H2D copy engine (copies of different streams are not served in issue order).
@@ -793,6 +841,25 @@ extern "C" int fnp_recall_counters(const float *pred, const int32_t *pred_valid,
     cudaFuncSetAttribute(recall_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     recall_kernel<<<n_frames, 256, smem, (cudaStream_t)stream>>>(pred, pred_valid, pred_start, gt, gt_start, n_thresh, t[0], t[1],
                                                                  t[2], t[3], t[4], t[5], t[6], t[7], counters);
+    FNP_LAUNCH_CHECK();
+    return FNP_OK;
+}
+
+extern "C" int fnp_precision_counters(const float *pred, const int32_t *pred_valid, const int32_t *pred_start, const float *gt,
+                                      const int32_t *gt_start, int n_frames, int max_pred_per_frame, int max_gt_per_frame,
+                                      const float *thresh_host, int n_thresh, long long *counters, void *stream)
+{
+    if (n_frames < 0 || n_thresh < 0 || n_thresh > 8 || max_pred_per_frame < 0 || max_gt_per_frame < 0) return FNP_EINVAL;
+    if (n_frames == 0 || max_pred_per_frame == 0) return FNP_OK;
+    if (!pred || !pred_start || !gt_start || !counters || (n_thresh && !thresh_host) || (max_gt_per_frame && !gt))
+        return FNP_EINVAL;
+    float t[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    for (int i = 0; i < n_thresh; i++) t[i] = thresh_host[i];
+    const size_t smem = (size_t)(max_pred_per_frame + max_gt_per_frame) * sizeof(RBox) + (size_t)max_pred_per_frame * 4 + 16;
+    if (smem > 200 * 1024) return FNP_EINVAL;
+    cudaFuncSetAttribute(precision_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    precision_kernel<<<n_frames, 256, smem, (cudaStream_t)stream>>>(pred, pred_valid, pred_start, gt, gt_start, n_thresh, t[0],
+                                                                    t[1], t[2], t[3], t[4], t[5], t[6], t[7], counters);
     FNP_LAUNCH_CHECK();
     return FNP_OK;
 }

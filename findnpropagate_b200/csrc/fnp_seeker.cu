@@ -1831,10 +1831,9 @@ __device__ __forceinline__ float block_max128(float v, float *s4, const int lane
     return v;
 }
 
-// Block-wide arg-max of (score, index) over 128 threads, lowest index on ties; every thread gets the result.
+// Warp-wide arg-max of (score, index), lowest index on ties; every lane gets the result.
 // besti == 0x7fffffff means "no entry".
-__device__ __forceinline__ void block_argmax128(float &best, int &besti, float *s_f, int *s_i, const int lane,
-                                                const int warp)
+__device__ __forceinline__ void warp_argmax(float &best, int &besti)
 {
 #pragma unroll
     for (int o = 16; o; o >>= 1) {
@@ -1842,6 +1841,13 @@ __device__ __forceinline__ void block_argmax128(float &best, int &besti, float *
         const int oi = __shfl_xor_sync(0xffffffffu, besti, o);
         if (oi != 0x7fffffff && (besti == 0x7fffffff || ob > best || (ob == best && oi < besti))) { best = ob; besti = oi; }
     }
+}
+
+// Block-wide arg-max of (score, index) over 128 threads, lowest index on ties; every thread gets the result.
+__device__ __forceinline__ void block_argmax128(float &best, int &besti, float *s_f, int *s_i, const int lane,
+                                                const int warp)
+{
+    warp_argmax(best, besti);
     if (lane == 0) { s_f[warp] = best; s_i[warp] = besti; }
     __syncthreads();
     best = s_f[0]; besti = s_i[0];
@@ -1855,6 +1861,38 @@ __device__ __forceinline__ void block_argmax128(float &best, int &besti, float *
 }
 
 constexpr int kSelectMaxTopkH = 32768;   // hypotheses per frustum the suppression bitmask of topk > 1 covers
+
+// The weights and switches of the second-stage score.  Every stage-3 kernel forms the score with hyp_score, so
+// that a setting scored by select_multi_kernel gets the bits select_kernel gives it.
+struct ScoreTerms {
+    float dns_w, iou_w, dst_w, ego_w, occl_w;
+    bool kitti, mult, occl_mult, use_dist, use_occl_w, use_ego;
+};
+
+// Second-stage score of one hypothesis (frustum_proposals_v1.py:996-1026; FrustumProposerOGKITTI :650-654).
+// count / den: its point count over the frustum's normaliser; dist, dmin, dden: the distance term (read only with
+// use_dist); fail / fden: its occlusion score and the normaliser max + 1e-6 (use_occl_w, occl_mult); ego / emx: the
+// norm of its centre and the largest such norm (use_ego).
+__device__ __forceinline__ float hyp_score(const ScoreTerms &t, const int count, const float den, const float iou,
+                                           const float dist, const float dmin, const float dden, const float fail,
+                                           const float fden, const float ego, const float emx)
+{
+    const float dens = __fdiv_rn((float)count, den);
+    const float dr = t.use_dist ? __fsub_rn(1.0f, __fdiv_rn(__fsub_rn(dist, dmin), dden)) : 1.0f;
+    float sc;
+    if (t.kitti)
+        sc = __fadd_rn(__fadd_rn(__fadd_rn(t.dns_w, dens), __fmul_rn(t.iou_w, iou)), __fmul_rn(dr, t.dst_w));
+    else if (t.mult)
+        sc = __fmul_rn(__fmul_rn(__fmul_rn(__fmul_rn(__fmul_rn(dens, t.dns_w), iou), t.iou_w), dr), t.dst_w);
+    else {
+        sc = __fadd_rn(__fmul_rn(dens, t.dns_w), __fmul_rn(iou, t.iou_w));
+        if (t.use_dist) sc = __fadd_rn(sc, __fmul_rn(dr, t.dst_w));
+    }
+    if (t.use_occl_w) sc = __fadd_rn(sc, __fmul_rn(t.occl_w, __fsub_rn(1.0f, __fdiv_rn(fail, fden))));
+    if (t.use_ego) sc = __fadd_rn(sc, __fmul_rn(t.ego_w, __fdiv_rn(ego, emx)));
+    if (t.occl_mult) sc = __fmul_rn(__fmul_rn(dens, iou), fail);
+    return sc;
+}
 
 // EXTRAS = false is the shipped configuration (density + IoU, top-1): the optional terms, the score table and
 // the suppression bitmask of topk > 1 are compiled out.
@@ -1914,25 +1952,15 @@ __global__ void __launch_bounds__(128) select_kernel(const fnp_seeker_batch b, c
         dden = __fadd_rn(__fsub_rn(st[14], dmin), 1e-8f);
     }
     // argmax of score, lowest index wins ties (stable descending sort + top-1)
+    const ScoreTerms terms = {cfg.dns_w, cfg.iou_w, cfg.dst_w, cfg.ego_w, cfg.occl_w, kitti, mult, occl_mult, use_dist,
+                              use_occl_w, use_ego};
     float best = -__int_as_float(0x7f800000);
     int besti = 0x7fffffff;
     for (int r = tid; r < nv; r += blockDim.x) {
-        const float dens = __fdiv_rn((float)cbase[r], den);
-        const float iou = b.hyp_iou[(size_t)f * H + r];
-        const float dr = use_dist ? __fsub_rn(1.0f, __fdiv_rn(__fsub_rn(b.hyp_dist[(size_t)f * H + r], dmin), dden)) : 1.0f;
-        float sc;
-        if (kitti)
-            sc = __fadd_rn(__fadd_rn(__fadd_rn(cfg.dns_w, dens), __fmul_rn(cfg.iou_w, iou)), __fmul_rn(dr, cfg.dst_w));
-        else if (mult)
-            sc = __fmul_rn(__fmul_rn(__fmul_rn(__fmul_rn(__fmul_rn(dens, cfg.dns_w), iou), cfg.iou_w), dr), cfg.dst_w);
-        else {
-            sc = __fadd_rn(__fmul_rn(dens, cfg.dns_w), __fmul_rn(iou, cfg.iou_w));
-            if (use_dist) sc = __fadd_rn(sc, __fmul_rn(dr, cfg.dst_w));
-        }
-        if (use_occl_w) sc = __fadd_rn(sc, __fmul_rn(cfg.occl_w, __fsub_rn(1.0f, __fdiv_rn(FNP_FAIL(r), fden))));
-        if (use_ego)
-            sc = __fadd_rn(sc, __fmul_rn(cfg.ego_w, __fdiv_rn(norm3(pbase[r * 8], pbase[r * 8 + 1], pbase[r * 8 + 2]), emx)));
-        if (occl_mult) sc = __fmul_rn(__fmul_rn(dens, iou), FNP_FAIL(r));
+        const float sc = hyp_score(terms, cbase[r], den, b.hyp_iou[(size_t)f * H + r],
+                                   use_dist ? b.hyp_dist[(size_t)f * H + r] : 0.f, dmin, dden,
+                                   (use_occl_w || occl_mult) ? FNP_FAIL(r) : 0.f, fden,
+                                   use_ego ? norm3(pbase[r * 8], pbase[r * 8 + 1], pbase[r * 8 + 2]) : 0.f, emx);
         if (T > 1) b.hyp_score[(size_t)f * H + r] = sc;
         if (sc > best || besti == 0x7fffffff) { best = sc; besti = r; }
     }
@@ -1978,6 +2006,102 @@ __global__ void __launch_bounds__(128) select_kernel(const fnp_seeker_batch b, c
                 b.out_best[(size_t)f * T + kk] = -1; b.out_score[(size_t)f * T + kk] = 0.f; b.out_count[(size_t)f * T + kk] = 0;
             }
             break;
+        }
+    }
+}
+
+// Stage 3 for many select-level settings over one execution of stages 1-2c (fnp_seeker_select_multi).  One CTA
+// per frustum stages the frustum's per-hypothesis inputs in shared memory once -- count and IoU, and the planes some
+// setting reads: distance, occlusion score, centre norm -- then warp w scores settings w, w + 8, ...: the setting's
+// valid set is the compacted hypotheses with iou > its min_cam_iou, the count / occlusion / ego normalisers are
+// maxima over that set, and the arg-max of hyp_score over it breaks ties on the lowest index (compaction keeps the
+// original order, so that is also the lowest original index: select_kernel's choice for a cfg with those values).
+constexpr int kMultiThreads = 256;
+constexpr int kMultiPlaneDist = 1, kMultiPlaneFail = 2, kMultiPlaneEgo = 4;
+
+struct SelectSettings {
+    fnp_select_setting s[FNP_SELECT_MAX_SETTINGS];
+};
+
+__global__ void __launch_bounds__(kMultiThreads) select_multi_kernel(const fnp_seeker_batch b, const int J, const int H,
+                                                                    const SelectSettings set, const int n_set,
+                                                                    const int planes, float *out_boxes, float *out_score,
+                                                                    int32_t *out_best, int32_t *out_count)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int f = blockIdx.x, F = b.n_cands;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int nv = (b.status[0] & 2) ? 0 : b.hyp_nvalid[f];
+    int *s_cnt = reinterpret_cast<int *>(smem);
+    float *s_iou = reinterpret_cast<float *>(s_cnt + H);
+    float *p_next = s_iou + H;
+    float *s_dist = (planes & kMultiPlaneDist) ? p_next : nullptr;
+    p_next += s_dist ? H : 0;
+    float *s_fail = (planes & kMultiPlaneFail) ? p_next : nullptr;
+    p_next += s_fail ? H : 0;
+    float *s_ego = (planes & kMultiPlaneEgo) ? p_next : nullptr;
+    const size_t fH = (size_t)f * H;
+    const float *pbase = b.hyp_prep + fH * 8;
+    const long long npts = b.cand_npts[f];
+    for (int r = threadIdx.x; r < nv; r += kMultiThreads) {
+        const int c = b.counts[fH + r];
+        s_cnt[r] = c;
+        s_iou[r] = b.hyp_iou[fH + r];
+        if (s_dist) s_dist[r] = b.hyp_dist[fH + r];
+        // the reference's occlusion score n_far * n_out, as select_kernel's FNP_FAIL forms it
+        if (s_fail) s_fail[r] = __ll2float_rn((long long)b.hyp_nfar[fH + r] * (npts - (long long)c));
+        if (s_ego) s_ego[r] = norm3(pbase[r * 8], pbase[r * 8 + 1], pbase[r * 8 + 2]);
+    }
+    float dmin = 0.f, dden = 1.f;
+    if (s_dist) {
+        const float *st = b.cand_stats + (size_t)f * kStatsFloats;
+        dmin = st[13];
+        dden = __fadd_rn(__fsub_rn(st[14], dmin), 1e-8f);
+    }
+    __syncthreads();
+    const float *bb_tab = b.base_boxes + (size_t)(b.cand_label[f] - 1) * J * 7;
+    for (int si = warp; si < n_set; si += kMultiThreads / 32) {
+        const fnp_select_setting p = set.s[si];
+        const bool mult = (p.flags & FNP_SEEKER_MULT) != 0, occl_mult = (p.flags & FNP_SEEKER_OCCL_MULT) != 0;
+        const ScoreTerms t = {p.dns_w, p.iou_w, p.dst_w, p.ego_w, p.occl_w, false, mult, occl_mult,
+                              (p.dst_w != 0.f) || mult, p.occl_w > 0.f, p.ego_w > 0.f};
+        const bool use_fail = t.use_occl_w || occl_mult;
+        const float thr = p.min_cam_iou;
+        int mxi = 0;
+        float fmx = 0.f, emx = 0.f;
+        for (int r = lane; r < nv; r += 32) {
+            if (!(s_iou[r] > thr)) continue;
+            mxi = max(mxi, s_cnt[r]);
+            if (use_fail) fmx = fmaxf(fmx, s_fail[r]);
+            if (t.use_ego) emx = fmaxf(emx, s_ego[r]);
+        }
+        const float den = __fadd_rn(warp_max((float)mxi), 1e-8f);
+        const float fden = use_fail ? __fadd_rn(warp_max(fmx), 1e-6f) : 1.f;
+        if (t.use_ego) emx = warp_max(emx);
+        float best = -__int_as_float(0x7f800000);
+        int besti = 0x7fffffff;
+        for (int r = lane; r < nv; r += 32) {
+            if (!(s_iou[r] > thr)) continue;
+            const float sc = hyp_score(t, s_cnt[r], den, s_iou[r], t.use_dist ? s_dist[r] : 0.f, dmin, dden,
+                                       use_fail ? s_fail[r] : 0.f, fden, t.use_ego ? s_ego[r] : 0.f, emx);
+            if (sc > best || besti == 0x7fffffff) { best = sc; besti = r; }
+        }
+        warp_argmax(best, besti);
+        // every lane writes lane 0's choice: the lanes agree after warp_argmax unless scores are unordered (NaN)
+        best = __shfl_sync(0xffffffffu, best, 0);
+        besti = __shfl_sync(0xffffffffu, besti, 0);
+        const size_t o = (size_t)si * F + f;
+        if (lane < 7) {
+            float v = 0.f;      // a frustum without a hypothesis valid for the setting: zeros, best -1
+            if (besti != 0x7fffffff)
+                v = lane < 3 ? pbase[(size_t)besti * 8 + lane] : bb_tab[(size_t)(b.hyp_index[fH + besti] % J) * 7 + lane];
+            out_boxes[o * 7 + lane] = v;
+        }
+        if (lane == 0) {
+            const bool none = besti == 0x7fffffff;
+            out_best[o] = none ? -1 : besti;
+            out_score[o] = none ? 0.f : best;
+            out_count[o] = none ? 0 : s_cnt[besti];
         }
     }
 }
@@ -2211,6 +2335,39 @@ extern "C" int fnp_seeker_select(const fnp_seeker_cfg *cfg, const fnp_seeker_bat
         select_kernel<true><<<b->n_cands, 128, 0, (cudaStream_t)stream>>>(*b, *cfg);
     else
         select_kernel<false><<<b->n_cands, 128, 0, (cudaStream_t)stream>>>(*b, *cfg);
+    FNP_LAUNCH_CHECK();
+    return FNP_OK;
+}
+
+extern "C" int fnp_seeker_select_multi(const fnp_seeker_cfg *cfg, const fnp_seeker_batch *b,
+                                       const fnp_select_setting *settings_host, int n_settings, float *out_boxes,
+                                       float *out_score, int32_t *out_best, int32_t *out_count, void *stream)
+{
+    int rc = check_batch(cfg, b);
+    if (rc) return rc;
+    if (!settings_host || n_settings < 1 || n_settings > FNP_SELECT_MAX_SETTINGS) return FNP_EINVAL;
+    // KITTI: first-match counts depend on the valid set; topk > 1: the suppression pass is not repeated per setting
+    if (cfg->topk > 1 || cfg->variant == FNP_VARIANT_KITTI) return FNP_EINVAL;
+    SelectSettings set = {};
+    int planes = 0;
+    for (int i = 0; i < n_settings; i++) {
+        const fnp_select_setting &s = settings_host[i];
+        if (s.flags & ~(FNP_SEEKER_MULT | FNP_SEEKER_OCCL_MULT)) return FNP_EINVAL;
+        if (!(s.min_cam_iou >= cfg->min_cam_iou)) return FNP_EINVAL;    // compacted at cfg's threshold
+        if ((s.dst_w != 0.f) || (s.flags & FNP_SEEKER_MULT)) planes |= kMultiPlaneDist;
+        if ((s.occl_w > 0.f) || (s.flags & FNP_SEEKER_OCCL_MULT)) planes |= kMultiPlaneFail;
+        if (s.ego_w > 0.f) planes |= kMultiPlaneEgo;
+        set.s[i] = s;
+    }
+    if (((planes & kMultiPlaneDist) && !b->hyp_dist) || ((planes & kMultiPlaneFail) && !b->hyp_nfar)) return FNP_EINVAL;
+    if (b->n_cands == 0) return FNP_OK;
+    if (!out_boxes || !out_score || !out_best || !out_count || !b->counts) return FNP_EINVAL;
+    const int J = cfg->num_yaw_size, H = J * cfg->num_mags;
+    const size_t smem = (size_t)H * 4 * (2 + __builtin_popcount(planes));
+    if (smem > 200 * 1024) return FNP_EINVAL;
+    cudaFuncSetAttribute(select_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    select_multi_kernel<<<b->n_cands, kMultiThreads, smem, (cudaStream_t)stream>>>(*b, J, H, set, n_settings, planes,
+                                                                                out_boxes, out_score, out_best, out_count);
     FNP_LAUNCH_CHECK();
     return FNP_OK;
 }

@@ -27,6 +27,26 @@ def _cfg_get(cfg, key, default=None):
     return getattr(cfg, key, default) if not hasattr(cfg, "get") else cfg.get(key, default)
 
 
+# PARAMS keys the head reads besides the constructor's own (:160-165)
+EXTRA_PARAMS = ('aln_w', 'ego_w', 'occl_w', 'rand_center', 'search_depth')
+
+
+def head_params(model_cfg, defaults=None):
+    """The parameters FrustumProposerOG runs with: ``defaults`` (the constructor's, DEFAULTS when None), overridden by
+    ``model_cfg.PARAMS`` (:167-196), plus the model_cfg-level switches MULTICAM_IOU / OCCL_MULT / MULT (:154-156)."""
+    p = dict(DEFAULTS if defaults is None else defaults)
+    params = _cfg_get(model_cfg, 'PARAMS')
+    if params is not None:
+        for k in list(DEFAULTS) + list(EXTRA_PARAMS):
+            if k in params:
+                p[k] = params[k]
+    if _cfg_get(model_cfg, 'SAVE_BLEND', False):
+        raise NotImplementedError("SAVE_BLEND (Blender visualisation dumps) is outside the Box Seeker path")
+    for flag in ('MULTICAM_IOU', 'OCCL_MULT', 'MULT'):
+        p[flag] = bool(_cfg_get(model_cfg, flag, False))
+    return p
+
+
 # ----------------------------------------------------------------------------- feeders
 class BoxList:
     """Unpickling shim for maskrcnn_benchmark.structures.bounding_box.BoxList (GLIP's
@@ -237,15 +257,7 @@ class FrustumProposerOG(nn.Module):
                  size_max=size_max, ry_min=ry_min, ry_max=float(ry_max), cq=cq, num_mags=num_mags, max_dist=max_dist,
                  num_sizes=num_sizes, num_rotations=num_rotations, topk=topk, nms_2d=nms_2d, nms_3d=nms_3d,
                  score_thr=score_thr, nms_normal=nms_normal, clamp_bottom=clamp_bottom)
-        params = _cfg_get(model_cfg, 'PARAMS')
-        if params is not None:                       # PARAMS override the defaults (:167-196)
-            for k in list(DEFAULTS) + ['aln_w', 'ego_w', 'occl_w', 'rand_center', 'search_depth']:
-                if k in params:
-                    p[k] = params[k]
-        if _cfg_get(model_cfg, 'SAVE_BLEND', False):
-            raise NotImplementedError("SAVE_BLEND (Blender visualisation dumps) is outside the Box Seeker path")
-        for flag in ('MULTICAM_IOU', 'OCCL_MULT', 'MULT'):      # model_cfg-level switches (:154-156)
-            p[flag] = bool(_cfg_get(model_cfg, flag, False))
+        p = head_params(model_cfg, p)
         assert p['nms_3d'] == 0, 'DO NOT USE!'          # the reference's own assertion (:209)
         self.params = p
         self.box_fmt = _cfg_get(model_cfg, 'BOX_FORMAT', 'xyxy')

@@ -48,6 +48,9 @@ RECALL_PER_THRESH = ["rcnn", "rcnn_3known", "rcnn_6known", "rcnn_4unknown", "rcn
 
 
 FLAG_KEYS = ("MULT", "OCCL_MULT", "MULTICAM_IOU")     # MODEL.DENSE_HEAD switches, frustum_proposals_v1.py:154-156
+# the parameters only stage 3 reads (with min_cam_iou, which only removes hypotheses): settings that differ in these
+# alone share stages 1-2c (SeekerEngine.evaluate_settings, fnp_seeker_select_multi)
+SELECT_KEYS = ("dns_w", "iou_w", "dst_w", "ego_w", "occl_w", "min_cam_iou", "MULT", "OCCL_MULT")
 
 
 def resolve_params(params: Optional[dict], variant: str = "nuscenes") -> dict:
@@ -86,6 +89,16 @@ def resolve_params(params: Optional[dict], variant: str = "nuscenes") -> dict:
     if unsupported:
         raise NotImplementedError("Box Seeker options outside the supported set: " + ", ".join(unsupported))
     return p
+
+
+def select_setting(p: dict) -> "_lib.SelectSetting":
+    """The fnp_select_setting of a parameter dict (its SELECT_KEYS; the head's defaults for those it leaves out)."""
+    p = dict(dict(DEFAULTS, ego_w=0, occl_w=0, MULT=False, OCCL_MULT=False), **{k: p[k] for k in SELECT_KEYS if k in p})
+    return _lib.SelectSetting(dns_w=float(p["dns_w"]), iou_w=float(p["iou_w"]), dst_w=float(p["dst_w"]),
+                              ego_w=float(p["ego_w"] or 0), occl_w=float(p["occl_w"] or 0),
+                              min_cam_iou=float(p["min_cam_iou"]),
+                              flags=(_lib.SEEKER_MULT if p["MULT"] else 0) | (_lib.SEEKER_OCCL_MULT if p["OCCL_MULT"] else 0),
+                              reserved=0)
 
 
 def build_tables(p: dict, anchors=None):
@@ -553,16 +566,25 @@ class SeekerEngine:
         return {k: base + o for k, o in offs.items()}
 
     def execute(self, plan, points_dev, nms_thresh=None, gt=None, recall_thresh=(0.3, 0.5, 0.7), slot=0,
-                points_ready=None):
+                points_ready=None, settings=None):
         """Enqueue the whole batch on the current stream.  points_dev: CUDA float32 tensor
         holding the rows of all frames back to back.  points_ready: optional CUDA event the
         kernels must wait for (the H2D copy of the points on another stream); the small
         metadata upload is issued *before* that wait so that it does not queue behind the
-        next step's point copy in the H2D engine.  Returns a handle for `finish`."""
+        next step's point copy in the H2D engine.  settings: see evaluate_settings.  Returns a
+        handle for `finish`."""
         t0 = time.perf_counter()
         _lib.require_cuda(points_dev)
         assert points_dev.dtype == torch.float32 and points_dev.is_contiguous()
         F, B, H, M = plan["F"], plan["B"], self.H, self.M
+        S = len(settings) if settings is not None else 0
+        if S:
+            sel = [select_setting(dict(self.p, **s)) for s in settings]     # left-out keys: this engine's values
+            # the workspaces any setting reads, whether or not this engine's own score reads them
+            use_dist = self.use_dist or any(s.dst_w != 0 or s.flags & _lib.SEEKER_MULT for s in sel)
+            use_occl = self.use_occl or any(s.occl_w > 0 or s.flags & _lib.SEEKER_OCCL_MULT for s in sel)
+        else:
+            use_dist, use_occl = self.use_dist, self.use_occl
         dev = self.device
         with torch.cuda.device(dev):
             stream = _lib.current_stream(dev)
@@ -606,12 +628,15 @@ class SeekerEngine:
             FT = F * T
             off_recall = 4 * (10 * FT + 2 * F + 8)
             off_keep = off_recall + 8 * self.N_COUNTERS
-            sizes["out"] = off_keep + _align(FT, 8)
+            # per setting: boxes(7) score best count per candidate, then recall and precision counters per setting
+            off_sel = off_keep + _align(FT, 8)
+            off_sel_counters = off_sel + 40 * S * F
+            sizes["out"] = off_sel_counters + 8 * S * (self.N_COUNTERS + self.N_PRECISION)
             if T > 1:
                 sizes["hyp_score"] = 4 * H * F
-            if self.use_dist:
+            if use_dist:
                 sizes["hyp_dist"] = 4 * H * F
-            if self.use_occl:
+            if use_occl:
                 sizes["hyp_nfar"] = 4 * H * F
             if self.debug:
                 sizes.update(hyp_boxes_dbg=28 * H * F, hyp_iou_dbg=4 * H * F, hyp_valid_dbg=H * F)
@@ -656,7 +681,11 @@ class SeekerEngine:
             handle = dict(plan=plan, batch=b, sp=sp, cap=cap, out_dev=out_dev, out_bytes=sizes["out"], meta=meta,
                           tab_stride=tab_stride, planes=planes,
                           off_recall=off_recall, off_keep=off_keep, has_nms=False, has_recall=False,
-                          recall_thresh=tuple(recall_thresh))
+                          recall_thresh=tuple(recall_thresh), n_settings=S, off_sel=off_sel,
+                          off_sel_counters=off_sel_counters)
+            if S and F:
+                self._select_multi(plan, meta, b, sel, use_occl, gt, recall_thresh, stream, out_dev, off_sel,
+                                   off_sel_counters)
             if nms_thresh is not None and F:
                 self._stage4_nms(plan, meta, o_boxes, o_best, float(nms_thresh), stream, ob + off_keep)
                 handle["has_nms"] = True
@@ -697,6 +726,65 @@ class SeekerEngine:
                                           out_dev.data_ptr() + off, stream)
         _lib.check(rc, "fnp_recall_counters")
         self.launches += 1
+
+    N_PRECISION = 1 + 3             # valid proposals, then hits at 3 IoU thresholds (fnp_precision_counters)
+
+    def _select_multi(self, plan, meta, b, sel, use_occl, gt, thresh, stream, out_dev, off, off_counters):
+        """Stage 3 once per setting over this execution's stages 1-2c, then each setting's recall and precision."""
+        L, F, S = _lib.lib, plan["F"], len(sel)
+        if use_occl and not self.use_occl:      # this engine's own cfg leaves stage 2c off
+            cfg = _lib.SeekerCfg.from_buffer_copy(self.cfg)
+            cfg.flags |= _lib.SEEKER_OCCL_MULT
+            _lib.check(L.fnp_seeker_occlusion(C.byref(cfg), C.byref(b), stream), "fnp_seeker_occlusion")
+            self.launches += 1
+        ob = out_dev.data_ptr() + off
+        boxes, best = ob, ob + 32 * S * F
+        # one launch per FNP_SELECT_MAX_SETTINGS settings (the kernel-parameter block), all over the same stages 1-2c
+        for c0 in range(0, S, _lib.SELECT_MAX_SETTINGS):
+            n = min(_lib.SELECT_MAX_SETTINGS, S - c0)
+            chunk = (_lib.SelectSetting * n)(*sel[c0:c0 + n])
+            _lib.check(L.fnp_seeker_select_multi(C.byref(self.cfg), C.byref(b), chunk, n, boxes + 28 * c0 * F,
+                                                 ob + 28 * S * F + 4 * c0 * F, best + 4 * c0 * F,
+                                                 ob + 36 * S * F + 4 * c0 * F, stream), "fnp_seeker_select_multi")
+            self.launches += 1
+        if gt is None:
+            return
+        gt_boxes, gt_start, max_gt = gt
+        out_dev[off_counters:off_counters + 8 * S * (self.N_COUNTERS + self.N_PRECISION)].zero_()
+        th = (C.c_float * len(thresh))(*[float(t) for t in thresh])
+        for s in range(S):
+            for fn, n, base in ((L.fnp_recall_counters, self.N_COUNTERS, off_counters),
+                                (L.fnp_precision_counters, self.N_PRECISION, off_counters + 8 * S * self.N_COUNTERS)):
+                rc = fn(boxes + 28 * s * F, best + 4 * s * F, meta["frame_cand_start"], gt_boxes.data_ptr(),
+                        gt_start.data_ptr(), plan["B"], max(plan["max_cands"], 1), int(max_gt), th, len(thresh),
+                        out_dev.data_ptr() + base + 8 * s * n, stream)
+                _lib.check(rc, fn.__name__)
+        self.launches += 2 * S
+
+    def evaluate_settings(self, plan, points_dev, gt, settings, recall_thresh=(0.3, 0.5, 0.7)):
+        """Scores several select-level settings on one batch: stages 1-2c run once with this engine's parameters, then
+        stage 3 once per setting (fnp_seeker_select_multi), and its recall and precision counters.  settings: dicts of
+        SELECT_KEYS (a key a setting leaves out takes this engine's value), any number of them: stage 3 runs for up to
+        256 settings per launch; each min_cam_iou must be at least this engine's, whose compaction every setting
+        filters further.  plan / points_dev / gt as for execute (gt from
+        upload_gt).  Returns finish()'s dict, whose "settings" holds per setting: proposals, recall (recall_dict),
+        precision (proposals, then "hits_<t>": proposals with a GT IoU3D > t), and per candidate cand_best (index among
+        the compacted hypotheses, -1: none), cand_score2, cand_count, cand_boxes.  One D2H; on a page-pool overflow
+        the pool grows and the batch runs again."""
+        if self.T != 1 or self.variant != "nuscenes" or self.rand_center:
+            raise NotImplementedError("evaluate_settings runs the nuScenes head with topk = 1 and no rand_center")
+        if not settings:
+            raise ValueError("evaluate_settings needs at least one setting")
+        for s in settings:
+            if np.float32(s.get("min_cam_iou", self.p["min_cam_iou"])) < np.float32(self.p["min_cam_iou"]):
+                raise ValueError("setting %r: min_cam_iou below the engine's %s" % (s, self.p["min_cam_iou"]))
+        while True:
+            h = self.execute(plan, points_dev, gt=gt, recall_thresh=recall_thresh, settings=settings)
+            try:
+                return self.finish(h)
+            except OverflowError as e:
+                need = int(e.args[0])
+                self.pts_factor = max(self.pts_factor * 1.5, 1.25 * need / max(plan["total_rows"], 1))
 
     def finish(self, handle):
         """Wait for the batch and assemble per-frame results (reference output format)."""
@@ -740,6 +828,25 @@ class SeekerEngine:
         if handle["has_recall"]:
             o = handle["off_recall"]
             res["recall"] = self.recall_dict(raw[o:o + 8 * self.N_COUNTERS].view(np.int64), handle["recall_thresh"])
+        S = handle["n_settings"]
+        if S:
+            o, oc = handle["off_sel"], handle["off_sel_counters"]
+            sb = raw[o:o + 28 * S * F].view(np.float32).reshape(S, F, 7)
+            ss = raw[o + 28 * S * F:o + 32 * S * F].view(np.float32).reshape(S, F)
+            si = raw[o + 32 * S * F:o + 40 * S * F].view(np.int32).reshape(2, S, F)
+            rec = raw[oc:oc + 8 * S * self.N_COUNTERS].view(np.int64).reshape(S, self.N_COUNTERS)
+            oc += 8 * S * self.N_COUNTERS
+            prec = raw[oc:oc + 8 * S * self.N_PRECISION].view(np.int64).reshape(S, self.N_PRECISION)
+            th = handle["recall_thresh"]
+            res["settings"] = []
+            for s in range(S):
+                d = dict(proposals=int((si[0, s] >= 0).sum()), cand_best=si[0, s].copy(), cand_score2=ss[s].copy(),
+                         cand_count=si[1, s].copy(), cand_boxes=sb[s].copy())
+                if handle["has_recall"]:
+                    d["recall"] = self.recall_dict(rec[s], th)
+                    d["precision"] = dict(proposals=int(prec[s, 0]),
+                                          **{"hits_%s" % t: int(prec[s, 1 + i]) for i, t in enumerate(th)})
+                res["settings"].append(d)
         self.host_s["finish"] += time.perf_counter() - t0
         return res
 

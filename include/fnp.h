@@ -285,6 +285,38 @@ int fnp_seeker_select(const fnp_seeker_cfg *cfg, const fnp_seeker_batch *b, void
 /* All stages back to back on `stream`. */
 int fnp_seeker_run(const fnp_seeker_cfg *cfg, const fnp_seeker_batch *b, void *stream);
 
+/* Stage 3 for many "select-level" settings at once, for tuning the score.  Stages 1-2c do not read the score weights,
+ * a hypothesis's point count does not depend on which other hypotheses are valid, and min_cam_iou only removes
+ * hypotheses; so settings that differ only in the fields below can share one execution of stages 1-2c and differ in
+ * stage 3 alone.  For every setting s and candidate f the call writes what fnp_seeker_select writes at topk = 1 when
+ * the stages run with s's values in cfg, bit for bit:
+ *   out_boxes (S,F,7), out_score (S,F), out_best (S,F) and out_count (S,F), slot s*F + f.  out_best is the
+ *   index among b's compacted hypotheses (b->hyp_index maps it to the original one), -1 when no hypothesis of the
+ *   frustum is valid for s; such a slot has a zero box, score 0 and count 0.
+ * Setting s's valid set is the compacted hypotheses with hyp_iou > s.min_cam_iou; the count, occlusion and ego
+ * normalisers are maxima over that set, while the distance term keeps cand_stats[13..14] (every hypothesis within
+ * max_dist, whatever its IoU).  Ties go to the lowest index.
+ * Call it after fnp_seeker_run (or the stages up to fnp_seeker_occlusion) on the same b.  settings_host is a HOST
+ * array of n_settings (1..FNP_SELECT_MAX_SETTINGS) entries, passed by value as kernel parameters (256 x 32 B = 8 KB
+ * of the 32 KB parameter space; the library allocates nothing).  Each CTA stages a frustum's counts and IoUs, plus
+ * the distance, occlusion and centre-norm planes when some setting reads them: 4 H bytes per plane, at most 200 KB
+ * (6-15 KB at H = 768).  A caller with more settings makes one call per 256 over the same stages 1-2c.
+ * Build record (nvcc 12.9, -Xptxas -v, sm_100a): select_multi_kernel 256 threads, 48 registers, 8-byte stack frame,
+ * 4 bytes of spill stores / loads, no static shared memory.
+ * FNP_EINVAL: cfg->topk > 1; the KITTI variant (its first-match counts depend on the valid set); a flag other than
+ * FNP_SEEKER_MULT / FNP_SEEKER_OCCL_MULT; a setting's min_cam_iou below cfg->min_cam_iou (the compaction was done
+ * at cfg's threshold); a setting that needs hyp_dist (dst_w != 0, MULT) or hyp_nfar (occl_w > 0, OCCL_MULT) on a
+ * batch without it -- hyp_nfar is formed by fnp_seeker_occlusion, which runs only when cfg itself turns occlusion on. */
+#define FNP_SELECT_MAX_SETTINGS 256
+typedef struct fnp_select_setting {
+    float dns_w, iou_w, dst_w, ego_w, occl_w, min_cam_iou;
+    int32_t flags;           /* FNP_SEEKER_MULT | FNP_SEEKER_OCCL_MULT */
+    int32_t reserved;
+} fnp_select_setting;
+int fnp_seeker_select_multi(const fnp_seeker_cfg *cfg, const fnp_seeker_batch *b, const fnp_select_setting *settings_host,
+                            int n_settings, float *out_boxes, float *out_score, int32_t *out_best, int32_t *out_count,
+                            void *stream);
+
 /* Stage 4: batched rotated-BEV bitmask NMS in shared memory.  Segment s covers boxes
  * [seg_start[s], seg_start[s+1]) (<= max_seg_boxes <= FNP_SEG_NMS_MAX each, in priority order: an earlier
  * kept box suppresses later ones with IoU > thresh, and if label != NULL only boxes of the
@@ -309,6 +341,17 @@ int fnp_seg_nms_rotated(const float *boxes, const int32_t *label, const int32_t 
 int fnp_recall_counters(const float *pred, const int32_t *pred_valid, const int32_t *pred_start, const float *gt,
                         const int32_t *gt_start, int n_frames, int max_pred_per_frame, int max_gt_per_frame,
                         const float *thresh_host, int n_thresh, long long *counters, void *stream);
+
+/* Precision counters, the companion of fnp_recall_counters with the same arguments: recall counts the GT boxes some
+ * proposal finds, this counts the proposals that find something -- what a looser filter costs.  counters (int64):
+ * [0] = valid proposals (pred_valid[i] >= 0, or every row when pred_valid is NULL), then per threshold t:
+ * [1+t] = valid proposals whose largest IoU3D over their frame's GT boxes is > thresh[t] (the IoU of
+ * fnp_recall_counters, box_overlap + iou3d_from_overlap).  ACCUMULATED (caller zeroes them).  Shared memory:
+ * 64 (max_pred + max_gt) + 4 max_pred bytes, at most 200 KB.  Build record (nvcc 12.9, -Xptxas -v, sm_100a):
+ * precision_kernel 256 threads, 73 registers, 304-byte stack frame (box_overlap's vertex arrays), no spills. */
+int fnp_precision_counters(const float *pred, const int32_t *pred_valid, const int32_t *pred_start, const float *gt,
+                           const int32_t *gt_start, int n_frames, int max_pred_per_frame, int max_gt_per_frame,
+                           const float *thresh_host, int n_thresh, long long *counters, void *stream);
 
 /* ------------------------------------------------------------- host-side planning
  * (runs on the CPU, touches no device memory: every pointer here is a HOST pointer)
