@@ -128,6 +128,11 @@ lib.fnp_seeker_select_multi.argtypes = [C.POINTER(SeekerCfg), C.POINTER(SeekerBa
 for _n in ("fnp_recall_counters", "fnp_precision_counters"):
     getattr(lib, _n).restype = _i
     getattr(lib, _n).argtypes = [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, C.POINTER(_f), _i, _vp, _vp]
+lib.fnp_quality_counters.restype = _i
+lib.fnp_quality_counters.argtypes = [_vp, C.c_longlong, _vp, C.c_longlong, _vp, _vp, _i, _vp, _vp, _i, _i, _i, _i,
+                                     C.POINTER(_f), _i, C.POINTER(_f), _i, _vp, _vp]
+lib.fnp_quality_smem_bytes.restype = C.c_size_t
+lib.fnp_quality_smem_bytes.argtypes = [_i, _i, _i, _i, _i]
 
 lib.fnp_host_select_candidates.restype = _i
 lib.fnp_host_select_candidates.argtypes = [_vp, _vp, _vp, _vp, _vp, _i, _i, _f, _f, _vp, _vp]
@@ -160,7 +165,8 @@ EXPORTED = [
     "fnp_boxes_iou_bev", "fnp_boxes_aligned_overlap_bev", "fnp_nms_workspace_bytes", "fnp_nms_rotated",
     "fnp_nms_normal", "fnp_seeker_cull", "fnp_seeker_frustum_stats", "fnp_seeker_hypotheses",
     "fnp_seeker_score", "fnp_seeker_score_mode", "fnp_seeker_occlusion", "fnp_seeker_select", "fnp_seeker_run", "fnp_seg_nms_rotated", "fnp_seeker_mask_words", "fnp_seeker_cell_mask_bytes",
-    "fnp_recall_counters", "fnp_precision_counters", "fnp_seeker_select_multi", "fnp_host_select_candidates", "fnp_host_pack_xyz", "fnp_host_pack_xyz_begin",
+    "fnp_recall_counters", "fnp_precision_counters", "fnp_quality_counters", "fnp_quality_smem_bytes",
+    "fnp_seeker_select_multi", "fnp_host_select_candidates", "fnp_host_pack_xyz", "fnp_host_pack_xyz_begin",
     "fnp_host_pack_wait", "fnp_host_nms_order", "fnp_host_pack_xyz_multi_begin", "fnp_host_plan_sizes", "fnp_host_plan",
     "fnp_points_in_boxes_matrix", "fnp_host_prep_boxes_cpu", "fnp_boxes_iou3d", "fnp_boxes_aligned_iou3d", "fnp_set_option", "fnp_seeker_cull_tile",
 ]

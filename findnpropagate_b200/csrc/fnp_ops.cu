@@ -623,6 +623,129 @@ __global__ void __launch_bounds__(256) precision_kernel(const float *__restrict_
     }
 }
 
+// Quality counters: recall and precision per (class, BEV range bin), for many settings of proposals over the same
+// frames and GT.  One CTA per (frame, chunk of kQualitySettingsPerCta settings): the frame's GT is staged once, then
+// per setting the proposals are staged and every (GT, proposal) pair is computed once; its IoU feeds the four
+// per-box maxima (GT: over all / same-label proposals, proposal: over all / same-class GT).  The counters are
+// gathered in shared memory and flushed once per setting.
+constexpr int kQualitySettingsPerCta = 8;
+constexpr int kQualityMaxThresh = 8, kQualityMaxBins = 8, kQualityMaxClasses = 32;
+
+struct QualityParams {
+    float thr[kQualityMaxThresh];
+    float edges[kQualityMaxBins - 1];
+    int n_thresh, n_edges, n_classes;
+};
+
+// Range bin of a box centre: the number of edges <= sqrt(x*x + y*y), each operation rounded on its own
+__device__ __forceinline__ int range_bin(const float *__restrict__ b, const QualityParams &q)
+{
+    const float r = __fsqrt_rn(__fadd_rn(__fmul_rn(b[0], b[0]), __fmul_rn(b[1], b[1])));
+    int bin = 0;
+    for (int e = 0; e < q.n_edges; e++) bin += q.edges[e] <= r;
+    return bin;
+}
+
+__global__ void __launch_bounds__(256) quality_kernel(const float *__restrict__ pred, long long pred_setting_stride,
+                                                      const int32_t *__restrict__ pred_valid, long long valid_setting_stride,
+                                                      const int32_t *__restrict__ pred_label,
+                                                      const int32_t *__restrict__ pred_start, int n_settings,
+                                                      const float *__restrict__ gt, const int32_t *__restrict__ gt_start,
+                                                      const QualityParams q, long long *__restrict__ counters)
+{
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int fr = blockIdx.x;
+    const int s_begin = blockIdx.y * kQualitySettingsPerCta;
+    const int s_end = min(n_settings, s_begin + kQualitySettingsPerCta);
+    const int p0 = pred_start[fr], K = pred_start[fr + 1] - p0;
+    const int g0 = gt_start[fr];
+    int G = gt_start[fr + 1] - g0;
+    // strip trailing all-zero GT rows (recall_kernel's rule)
+    while (G > 0) {
+        const float *g = gt + (size_t)(g0 + G - 1) * 8;
+        float s = 0.f;
+        for (int k = 0; k < 8; k++) s += g[k];
+        if (s != 0.f) break;
+        G--;
+    }
+    if (K <= 0 && G == 0) return;
+    const int R = q.n_edges + 1, W = 1 + 2 * q.n_thresh;      // counters per (class, bin)
+    const int n_block = q.n_classes * R * W;                  // one block: recall, then one: precision
+    RBox *s_g = reinterpret_cast<RBox *>(smem);               // [G]
+    RBox *s_p = s_g + G;                                      // [K]
+    int *s_gbest = reinterpret_cast<int *>(s_p + K);          // [2G]: best IoU (float bits) over all / same-label
+    int *s_pbest = s_gbest + 2 * G;                           // [2K]
+    int *s_gcell = s_pbest + 2 * K;                           // [G] (class - 1) * R + bin, -1: not counted
+    int *s_plab = s_gcell + G;                                // [K] label
+    int *s_pcell = s_plab + K;                                // [K] (label - 1) * R + bin, -1: not a proposal
+    int *s_cnt = s_pcell + K;                                 // [2 n_block]
+    for (int i = threadIdx.x; i < G; i += blockDim.x) {
+        const float *g = gt + (size_t)(g0 + i) * 8;
+        s_g[i] = prep_rbox(g);
+        const int lab = (int)g[7];
+        s_gcell[i] = (lab >= 1 && lab <= q.n_classes) ? (lab - 1) * R + range_bin(g, q) : -1;
+    }
+    for (int k = threadIdx.x; k < K; k += blockDim.x) s_plab[k] = pred_label[p0 + k];
+    for (int s = s_begin; s < s_end; s++) {
+        const float *P = pred + (size_t)s * pred_setting_stride * 7;
+        const int32_t *V = pred_valid ? pred_valid + (size_t)s * valid_setting_stride : nullptr;
+        for (int i = threadIdx.x; i < G; i += blockDim.x) s_gbest[2 * i] = s_gbest[2 * i + 1] = __float_as_int(-1.f);
+        for (int k = threadIdx.x; k < K; k += blockDim.x) {
+            const float *p = P + (size_t)(p0 + k) * 7;
+            s_p[k] = prep_rbox(p);
+            s_pbest[2 * k] = s_pbest[2 * k + 1] = __float_as_int(-1.f);
+            const int lab = s_plab[k];
+            const bool ok = (!V || V[p0 + k] >= 0) && lab >= 1 && lab <= q.n_classes;
+            if (!ok) s_p[k].pad = -1.f;                       // not a proposal
+            s_pcell[k] = ok ? (lab - 1) * R + range_bin(p, q) : -1;
+        }
+        for (int i = threadIdx.x; i < 2 * n_block; i += blockDim.x) s_cnt[i] = 0;
+        __syncthreads();
+        // the IoU of recall_kernel / precision_kernel, bit for bit
+        for (int w = threadIdx.x; w < G * K; w += blockDim.x) {
+            const int gi = w / K, k = w - gi * K;
+            if (s_p[k].pad < 0.f) continue;
+            float iou = 0.f;
+            if (!surely_disjoint(s_p[k], s_g[gi]))
+                iou = iou3d_from_overlap(P + (size_t)(p0 + k) * 7, gt + (size_t)(g0 + gi) * 8, box_overlap(s_p[k], s_g[gi]));
+            if (!(iou >= 0.f)) continue;
+            const int bits = __float_as_int(iou);
+            atomicMax(&s_gbest[2 * gi], bits);
+            atomicMax(&s_pbest[2 * k], bits);
+            if (s_plab[k] == (int)gt[(size_t)(g0 + gi) * 8 + 7]) {
+                atomicMax(&s_gbest[2 * gi + 1], bits);
+                atomicMax(&s_pbest[2 * k + 1], bits);
+            }
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < G; i += blockDim.x) {
+            if (s_gcell[i] < 0) continue;
+            int *c = s_cnt + s_gcell[i] * W;
+            const float ba = __int_as_float(s_gbest[2 * i]), bl = __int_as_float(s_gbest[2 * i + 1]);
+            atomicAdd(c, 1);
+            for (int t = 0; t < q.n_thresh; t++) {
+                if (ba > q.thr[t]) atomicAdd(c + 1 + t, 1);
+                if (bl > q.thr[t]) atomicAdd(c + 1 + q.n_thresh + t, 1);
+            }
+        }
+        for (int k = threadIdx.x; k < K; k += blockDim.x) {
+            if (s_pcell[k] < 0) continue;
+            int *c = s_cnt + n_block + s_pcell[k] * W;
+            const float ba = __int_as_float(s_pbest[2 * k]), bl = __int_as_float(s_pbest[2 * k + 1]);
+            atomicAdd(c, 1);
+            for (int t = 0; t < q.n_thresh; t++) {
+                if (ba > q.thr[t]) atomicAdd(c + 1 + t, 1);
+                if (bl > q.thr[t]) atomicAdd(c + 1 + q.n_thresh + t, 1);
+            }
+        }
+        __syncthreads();
+        long long *out = counters + (size_t)s * 2 * n_block;
+        for (int i = threadIdx.x; i < 2 * n_block; i += blockDim.x)
+            if (s_cnt[i]) atomicAdd(reinterpret_cast<unsigned long long *>(out + i), (unsigned long long)s_cnt[i]);
+        __syncthreads();
+    }
+}
+
 // Small host->device upload executed by SMs: `src` is pinned (page-locked, UVA-mapped) host
 // memory.  Used for the per-batch metadata so that it does not queue behind a large point
 // copy in the H2D copy engine (copies of different streams are not served in issue order).
@@ -860,6 +983,46 @@ extern "C" int fnp_precision_counters(const float *pred, const int32_t *pred_val
     cudaFuncSetAttribute(precision_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     precision_kernel<<<n_frames, 256, smem, (cudaStream_t)stream>>>(pred, pred_valid, pred_start, gt, gt_start, n_thresh, t[0],
                                                                     t[1], t[2], t[3], t[4], t[5], t[6], t[7], counters);
+    FNP_LAUNCH_CHECK();
+    return FNP_OK;
+}
+
+extern "C" size_t fnp_quality_smem_bytes(int max_pred_per_frame, int max_gt_per_frame, int n_classes, int n_edges, int n_thresh)
+{
+    const size_t n_block = (size_t)n_classes * (n_edges + 1) * (1 + 2 * n_thresh);
+    return (size_t)max_pred_per_frame * (sizeof(RBox) + 16) + (size_t)max_gt_per_frame * (sizeof(RBox) + 12) + 8 * n_block + 16;
+}
+
+extern "C" int fnp_quality_counters(const float *pred, long long pred_setting_stride, const int32_t *pred_valid,
+                                    long long valid_setting_stride, const int32_t *pred_label, const int32_t *pred_start,
+                                    int n_settings, const float *gt, const int32_t *gt_start, int n_frames,
+                                    int max_pred_per_frame, int max_gt_per_frame, int n_classes, const float *range_edges_host,
+                                    int n_edges, const float *thresh_host, int n_thresh, long long *counters, void *stream)
+{
+    if (n_settings < 0 || n_frames < 0 || max_pred_per_frame < 0 || max_gt_per_frame < 0 || pred_setting_stride < 0 ||
+        valid_setting_stride < 0)
+        return FNP_EINVAL;
+    if (n_thresh < 0 || n_thresh > kQualityMaxThresh || n_edges < 0 || n_edges > kQualityMaxBins - 1 || n_classes < 1 ||
+        n_classes > kQualityMaxClasses)
+        return FNP_EINVAL;
+    if ((n_thresh && !thresh_host) || (n_edges && !range_edges_host)) return FNP_EINVAL;
+    QualityParams q;
+    q.n_thresh = n_thresh; q.n_edges = n_edges; q.n_classes = n_classes;
+    for (int i = 0; i < kQualityMaxThresh; i++) q.thr[i] = i < n_thresh ? thresh_host[i] : 0.f;
+    for (int i = 0; i < kQualityMaxBins - 1; i++) q.edges[i] = i < n_edges ? range_edges_host[i] : 0.f;
+    for (int i = 0; i < n_edges; i++)
+        if (!(q.edges[i] > 0.f) || (i && !(q.edges[i] > q.edges[i - 1]))) return FNP_EINVAL;
+    const size_t smem = fnp_quality_smem_bytes(max_pred_per_frame, max_gt_per_frame, n_classes, n_edges, n_thresh);
+    if (smem > 200 * 1024) return FNP_EINVAL;
+    if (n_settings == 0 || n_frames == 0 || (max_pred_per_frame == 0 && max_gt_per_frame == 0)) return FNP_OK;
+    if (!pred_start || !gt_start || !counters || (max_pred_per_frame && (!pred || !pred_label)) || (max_gt_per_frame && !gt))
+        return FNP_EINVAL;
+    const int chunks = divup(n_settings, kQualitySettingsPerCta);
+    if (chunks > 65535) return FNP_EINVAL;
+    cudaFuncSetAttribute(quality_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    quality_kernel<<<dim3(n_frames, chunks), 256, smem, (cudaStream_t)stream>>>(
+        pred, pred_setting_stride, pred_valid, valid_setting_stride, pred_label, pred_start, n_settings, gt, gt_start, q,
+        counters);
     FNP_LAUNCH_CHECK();
     return FNP_OK;
 }

@@ -205,8 +205,16 @@ class NuScenesFeed:
     def __len__(self):
         return len(self.infos)
 
-    def _prepare(self, d: dict) -> dict:
-        """DatasetTemplate.prepare_data (dataset.py:159-220); returns None when the frame has to be re-drawn."""
+    def _load_gt(self, info: dict, d: dict):
+        """The info's GT with the min-points filter (nuscenes_dataset.py:252-258) into d."""
+        if 'gt_boxes' in info:
+            mask = (info['num_lidar_pts'] > self.filter_min_points_in_gt - 1) if self.filter_min_points_in_gt else None
+            d['gt_names'] = info['gt_names'] if mask is None else info['gt_names'][mask]
+            d['gt_boxes'] = info['gt_boxes'] if mask is None else info['gt_boxes'][mask]
+
+    def _prepare_gt(self, d: dict):
+        """The GT part of _prepare: class filter, class column, and in training mode the heading wrap and the range
+        filter."""
         if self.training:
             assert 'gt_boxes' in d, 'gt_boxes should be provided for training'      # dataset.py:182
             # DataAugmentor.forward with an empty queue (data_augmentor.py:380-394): headings wrapped, then the
@@ -214,17 +222,30 @@ class NuScenesFeed:
             keep = np.array([n in self.class_names for n in d['gt_names']], dtype=np.bool_)
             d['gt_boxes'][:, 6] = limit_period(d['gt_boxes'][:, 6], offset=0.5, period=2 * np.pi)
             d['gt_boxes'], d['gt_names'] = d['gt_boxes'][keep], d['gt_names'][keep]
-        d['lidar_aug_matrix'] = np.eye(4)                                   # set_lidar_aug_matrix, no augmentation
         if d.get('gt_boxes', None) is not None:
             sel = np.array([i for i, n in enumerate(d['gt_names']) if n in self.class_names], dtype=np.int64)
             d['gt_boxes'] = d['gt_boxes'][sel]
             d['gt_names'] = d['gt_names'][sel]
             cls = np.array([self.class_names.index(n) + 1 for n in d['gt_names']], dtype=np.int32)
             d['gt_boxes'] = np.concatenate((d['gt_boxes'], cls.reshape(-1, 1).astype(np.float32)), axis=1)
-        d['use_lead_xyz'] = True                                            # absolute_coordinates_encoding
-        d['points'] = d['points'][mask_points_by_range(d['points'], self.range)]
         if self.training and d.get('gt_boxes', None) is not None:          # REMOVE_OUTSIDE_BOXES, data_processor.py:88-93
             d['gt_boxes'] = d['gt_boxes'][mask_boxes_outside_range(d['gt_boxes'], self.range)]
+
+    def _finish_gt(self, info: dict, d: dict):
+        """NaN velocities zeroed, and the velocity columns dropped without PRED_VELOCITY (nuscenes_dataset.py:269-277)."""
+        if self.set_nan_velocity_to_zeros and 'gt_boxes' in info:
+            g = d['gt_boxes']
+            g[np.isnan(g)] = 0
+            d['gt_boxes'] = g
+        if not self.pred_velocity and 'gt_boxes' in d:
+            d['gt_boxes'] = d['gt_boxes'][:, [0, 1, 2, 3, 4, 5, 6, -1]]
+
+    def _prepare(self, d: dict) -> dict:
+        """DatasetTemplate.prepare_data (dataset.py:159-220); returns None when the frame has to be re-drawn."""
+        self._prepare_gt(d)
+        d['lidar_aug_matrix'] = np.eye(4)                                   # set_lidar_aug_matrix, no augmentation
+        d['use_lead_xyz'] = True                                            # absolute_coordinates_encoding
+        d['points'] = d['points'][mask_points_by_range(d['points'], self.range)]
         if self.training and len(d['gt_boxes']) == 0 and self.skip_no_gt:   # dataset.py:213-215
             return None
         d.pop('gt_names', None)
@@ -234,10 +255,7 @@ class NuScenesFeed:
         info = copy.deepcopy(self.infos[index])
         d = {'points': lidar_with_sweeps(self.root, info, self.max_sweeps, self.rng),
              'frame_id': Path(info['lidar_path']).stem, 'metadata': {'token': info['token']}}
-        if 'gt_boxes' in info:
-            mask = (info['num_lidar_pts'] > self.filter_min_points_in_gt - 1) if self.filter_min_points_in_gt else None
-            d['gt_names'] = info['gt_names'] if mask is None else info['gt_names'][mask]
-            d['gt_boxes'] = info['gt_boxes'] if mask is None else info['gt_boxes'][mask]
+        self._load_gt(info, d)
         d.update(camera_info(info))
         fH, fW = self.final_dim
         d['ori_shape'] = [fW, fH]
@@ -245,13 +263,21 @@ class NuScenesFeed:
         d = self._prepare(d)
         if d is None:        # SKIP_NO_GT: the reference returns another, randomly drawn frame in this one's place
             d = self[int((np.random if self.rng is None else self.rng).randint(len(self)))]
-        if self.set_nan_velocity_to_zeros and 'gt_boxes' in info:
-            g = d['gt_boxes']
-            g[np.isnan(g)] = 0
-            d['gt_boxes'] = g
-        if not self.pred_velocity and 'gt_boxes' in d:
-            d['gt_boxes'] = d['gt_boxes'][:, [0, 1, 2, 3, 4, 5, 6, -1]]
+        self._finish_gt(info, d)
         return d
+
+    def gt_boxes(self, index: int) -> np.ndarray:
+        """The frame's gt_boxes as ``self[index]`` produces them, without reading its LiDAR file.  A frame left
+        without GT gives an empty array here: no other frame is drawn in its place (SKIP_NO_GT), because a caller
+        that scores frame by frame must see this frame's GT.  A frame whose info has no GT gives a (0, 8) array."""
+        info = self.infos[index]
+        if 'gt_boxes' not in info:
+            return np.zeros((0, 8), np.float32)
+        d = {k: copy.deepcopy(info[k]) for k in ('gt_boxes', 'gt_names', 'num_lidar_pts') if k in info}
+        self._load_gt(d, d)
+        self._prepare_gt(d)
+        self._finish_gt(info, d)
+        return d['gt_boxes']
 
     # ---------------------------------------------------------------- seeker inputs
     def frame_input(self, index: int, detector, xyz_only: bool = False):

@@ -43,14 +43,11 @@ def pseudo_path(folder, frame_id):
     return os.path.join(str(folder), "%s.pth" % str(frame_id).replace('.', '_'))
 
 
-def load_pseudos(folder, frame_id, labels=None, nms_thresh=None):
-    """(K, 8) float32 [box7, label] and (K,) float32 scores of one frame, as load_pseudos returns
-    them with filter_by_score=False; a missing file gives empty arrays (the reference prints and
-    does the same).  labels: keep only these class labels (the reference's unknowns_only);
-    nms_thresh: apply bev_nms at that threshold (reference: PSEUDO_NMS_THRESH)."""
-    path = pseudo_path(folder, frame_id)
+def read_pseudos(path):
+    """(boxes (K,7) f32, scores (K,) f32, labels (K,)) of one proposal file -- a list of length 1 holding the dict, or
+    the bare dict; pred_boxes may have more than 7 columns -- or None when the file does not exist."""
     if not os.path.exists(path):
-        return np.zeros((0, 8), np.float32), np.zeros((0,), np.float32)
+        return None
     preds = torch.load(path, map_location='cpu', weights_only=False)
     if isinstance(preds, dict):
         pred = preds
@@ -59,7 +56,18 @@ def load_pseudos(folder, frame_id, labels=None, nms_thresh=None):
         pred = preds[0]
     boxes = pred['pred_boxes'].numpy().astype(np.float32)[:, :7]
     scores = pred['pred_scores'].numpy().astype(np.float32)
-    lab = pred['pred_labels'].numpy()
+    return boxes, scores, pred['pred_labels'].numpy()
+
+
+def load_pseudos(folder, frame_id, labels=None, nms_thresh=None):
+    """(K, 8) float32 [box7, label] and (K,) float32 scores of one frame, as load_pseudos returns
+    them with filter_by_score=False; a missing file gives empty arrays (the reference prints and
+    does the same).  labels: keep only these class labels (the reference's unknowns_only);
+    nms_thresh: apply bev_nms at that threshold (reference: PSEUDO_NMS_THRESH)."""
+    got = read_pseudos(pseudo_path(folder, frame_id))
+    if got is None:
+        return np.zeros((0, 8), np.float32), np.zeros((0,), np.float32)
+    boxes, scores, lab = got
     if labels is not None:
         m = np.isin(lab, np.asarray(list(labels)))
         boxes, scores, lab = boxes[m], scores[m], lab[m]

@@ -566,12 +566,12 @@ class SeekerEngine:
         return {k: base + o for k, o in offs.items()}
 
     def execute(self, plan, points_dev, nms_thresh=None, gt=None, recall_thresh=(0.3, 0.5, 0.7), slot=0,
-                points_ready=None, settings=None):
+                points_ready=None, settings=None, quality=None):
         """Enqueue the whole batch on the current stream.  points_dev: CUDA float32 tensor
         holding the rows of all frames back to back.  points_ready: optional CUDA event the
         kernels must wait for (the H2D copy of the points on another stream); the small
         metadata upload is issued *before* that wait so that it does not queue behind the
-        next step's point copy in the H2D engine.  settings: see evaluate_settings.  Returns a
+        next step's point copy in the H2D engine.  settings, quality: see evaluate_settings.  Returns a
         handle for `finish`."""
         t0 = time.perf_counter()
         _lib.require_cuda(points_dev)
@@ -632,6 +632,9 @@ class SeekerEngine:
             off_sel = off_keep + _align(FT, 8)
             off_sel_counters = off_sel + 40 * S * F
             sizes["out"] = off_sel_counters + 8 * S * (self.N_COUNTERS + self.N_PRECISION)
+            off_quality = sizes["out"]
+            if quality is not None:             # per setting: the class x range counters (quality.QualitySpec)
+                sizes["out"] += 8 * S * quality.n_counters
             if T > 1:
                 sizes["hyp_score"] = 4 * H * F
             if use_dist:
@@ -682,10 +685,13 @@ class SeekerEngine:
                           tab_stride=tab_stride, planes=planes,
                           off_recall=off_recall, off_keep=off_keep, has_nms=False, has_recall=False,
                           recall_thresh=tuple(recall_thresh), n_settings=S, off_sel=off_sel,
-                          off_sel_counters=off_sel_counters)
+                          off_sel_counters=off_sel_counters, quality=None, off_quality=off_quality)
             if S and F:
                 self._select_multi(plan, meta, b, sel, use_occl, gt, recall_thresh, stream, out_dev, off_sel,
                                    off_sel_counters)
+                if quality is not None and gt is not None:
+                    self._quality(plan, meta, S, gt, quality, stream, out_dev, off_sel, off_quality)
+                    handle["quality"] = quality
             if nms_thresh is not None and F:
                 self._stage4_nms(plan, meta, o_boxes, o_best, float(nms_thresh), stream, ob + off_keep)
                 handle["has_nms"] = True
@@ -761,7 +767,20 @@ class SeekerEngine:
                 _lib.check(rc, fn.__name__)
         self.launches += 2 * S
 
-    def evaluate_settings(self, plan, points_dev, gt, settings, recall_thresh=(0.3, 0.5, 0.7)):
+    def _quality(self, plan, meta, S, gt, spec, stream, out_dev, off, off_quality):
+        """One fnp_quality_counters launch over every setting's proposals (the boxes and flags _select_multi wrote);
+        labels are the candidates' 2D labels, shared by the settings."""
+        from . import quality
+        F = plan["F"]
+        gt_boxes, gt_start, max_gt = gt
+        out_dev[off_quality:off_quality + 8 * S * spec.n_counters].zero_()
+        ob = out_dev.data_ptr() + off
+        quality.launch(spec, ob, meta["cand_label"], meta["frame_cand_start"], gt_boxes, gt_start, plan["B"],
+                       max(plan["max_cands"], 1), int(max_gt), out_dev.data_ptr() + off_quality, n_settings=S,
+                       pred_valid=ob + 32 * S * F, pred_stride=F, valid_stride=F, stream=stream)
+        self.launches += 1
+
+    def evaluate_settings(self, plan, points_dev, gt, settings, recall_thresh=(0.3, 0.5, 0.7), quality=None):
         """Scores several select-level settings on one batch: stages 1-2c run once with this engine's parameters, then
         stage 3 once per setting (fnp_seeker_select_multi), and its recall and precision counters.  settings: dicts of
         SELECT_KEYS (a key a setting leaves out takes this engine's value), any number of them: stage 3 runs for up to
@@ -769,8 +788,9 @@ class SeekerEngine:
         filters further.  plan / points_dev / gt as for execute (gt from
         upload_gt).  Returns finish()'s dict, whose "settings" holds per setting: proposals, recall (recall_dict),
         precision (proposals, then "hits_<t>": proposals with a GT IoU3D > t), and per candidate cand_best (index among
-        the compacted hypotheses, -1: none), cand_score2, cand_count, cand_boxes.  One D2H; on a page-pool overflow
-        the pool grows and the batch runs again."""
+        the compacted hypotheses, -1: none), cand_score2, cand_count, cand_boxes.  quality (a quality.QualitySpec): one
+        more launch, fnp_quality_counters over every setting, and each setting gains "quality", its flat counters
+        (quality.tables reads them).  One D2H; on a page-pool overflow the pool grows and the batch runs again."""
         if self.T != 1 or self.variant != "nuscenes" or self.rand_center:
             raise NotImplementedError("evaluate_settings runs the nuScenes head with topk = 1 and no rand_center")
         if not settings:
@@ -778,8 +798,12 @@ class SeekerEngine:
         for s in settings:
             if np.float32(s.get("min_cam_iou", self.p["min_cam_iou"])) < np.float32(self.p["min_cam_iou"]):
                 raise ValueError("setting %r: min_cam_iou below the engine's %s" % (s, self.p["min_cam_iou"]))
+        if quality is not None:
+            from .quality import check_labels
+            check_labels(quality, plan["cand_label"], gt[0].cpu().numpy(), gt[1].cpu().numpy())
+            quality.check_size(plan["max_cands"], gt[2], "the largest frame of the batch")
         while True:
-            h = self.execute(plan, points_dev, gt=gt, recall_thresh=recall_thresh, settings=settings)
+            h = self.execute(plan, points_dev, gt=gt, recall_thresh=recall_thresh, settings=settings, quality=quality)
             try:
                 return self.finish(h)
             except OverflowError as e:
@@ -838,6 +862,10 @@ class SeekerEngine:
             oc += 8 * S * self.N_COUNTERS
             prec = raw[oc:oc + 8 * S * self.N_PRECISION].view(np.int64).reshape(S, self.N_PRECISION)
             th = handle["recall_thresh"]
+            spec = handle.get("quality")
+            if spec is not None:
+                oq = handle["off_quality"]
+                qc = raw[oq:oq + 8 * S * spec.n_counters].view(np.int64).reshape(S, spec.n_counters)
             res["settings"] = []
             for s in range(S):
                 d = dict(proposals=int((si[0, s] >= 0).sum()), cand_best=si[0, s].copy(), cand_score2=ss[s].copy(),
@@ -846,6 +874,8 @@ class SeekerEngine:
                     d["recall"] = self.recall_dict(rec[s], th)
                     d["precision"] = dict(proposals=int(prec[s, 0]),
                                           **{"hits_%s" % t: int(prec[s, 1 + i]) for i, t in enumerate(th)})
+                if spec is not None:
+                    d["quality"] = qc[s].copy()
                 res["settings"].append(d)
         self.host_s["finish"] += time.perf_counter() - t0
         return res

@@ -123,10 +123,12 @@ def group_settings(base_params, settings):
     return out
 
 
-def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, workers=4, box_format="xyxy", device=None):
+def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, workers=4, box_format="xyxy", device=None,
+                  quality=None):
     """Scores every setting over every frame of ``feed``: each batch is read once (NuScenesFeed.prefetch) and uploaded
     once, then every group of ``group_settings`` runs on it.  Returns (per setting dict(proposals, recall, precision)
-    summed over the frames, groups)."""
+    summed over the frames, groups).  quality (a quality.QualitySpec): each setting's dict also holds "quality", its
+    summed fnp_quality_counters counters."""
     import numpy as np
     import torch
     from .extract import THRESH, recall_keys
@@ -140,12 +142,15 @@ def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, worker
     prec_keys = ["proposals"] + ["hits_%s" % t for t in THRESH]
     totals = [dict(proposals=0, recall=dict.fromkeys(recall_keys(), 0), precision=dict.fromkeys(prec_keys, 0))
               for _ in settings]
+    if quality is not None:
+        for t in totals:
+            t["quality"] = np.zeros(quality.n_counters, np.int64)
     for frames, _, _ in feed.prefetch(range(len(feed)), detector, batch_frames=batch_frames, workers=workers,
                                       xyz_only=True):
         points = torch.from_numpy(np.concatenate([f.points for f in frames])).to(engines[0].device)
         gt = engines[0].upload_gt(frames)
         for g, eng in zip(groups, engines):
-            res = eng.evaluate_settings(eng.plan(frames), points, gt, g["settings"], recall_thresh=THRESH)
+            res = eng.evaluate_settings(eng.plan(frames), points, gt, g["settings"], recall_thresh=THRESH, quality=quality)
             for i, r in zip(g["members"], res["settings"]):
                 t = totals[i]
                 t["proposals"] += r["proposals"]
@@ -153,6 +158,8 @@ def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, worker
                     t["recall"][k] += v
                 for k, v in r.get("precision", {}).items():
                     t["precision"][k] += v
+                if "quality" in r:
+                    t["quality"] += r["quality"]
     return totals, groups
 
 
@@ -166,6 +173,10 @@ def parse_args(argv=None):
     p.add_argument("--batch_frames", type=int, default=64, help="frames per batch on the GPU")
     p.add_argument("--workers", type=int, default=4, help="loader threads")
     p.add_argument("--out", default=None, help="also write the JSON lines to this file")
+    p.add_argument("--breakdown", action="store_true",
+                   help="add per class and range bin counters to each line (classes; see eval_pseudo_labels)")
+    p.add_argument("--range_edges", type=float, nargs="*", default=[20.0, 30.0, 40.0],
+                   help="with --breakdown: BEV range bin edges in metres (default: 20 30 40)")
     p.add_argument("--set", dest="set_cfgs", default=None, nargs=argparse.REMAINDER, metavar="KEY VALUE",
                    help="config overrides applied to every setting, e.g. --set DATA_CONFIG.MAX_SWEEPS 1")
     return p.parse_args(argv)
@@ -192,6 +203,11 @@ def main(argv=None):
         settings = [{names[k]: v for k, v in s.items()} for s in grid]
         base = head_params(cfg.MODEL.DENSE_HEAD)
         groups = group_settings(base, settings)
+        spec = None
+        if args.breakdown:
+            from .nuscenes_feed import CLASS_NAMES
+            from .quality import QualitySpec
+            spec = QualitySpec(cfg.get("CLASS_NAMES") or CLASS_NAMES, range_edges=args.range_edges)
     except (OSError, KeyError, ValueError, NotImplementedError) as e:
         _fail(e.args[-1] if isinstance(e, KeyError) else e)
     print("%d settings in %d groups" % (len(settings), len(groups)))
@@ -207,7 +223,8 @@ def main(argv=None):
     feed = build_feed(cfg, infos=[all_frames.infos[i] for i, c in zip(picked, codes) if c == 0])
     print("frames scored: %d, failed frames: %d" % (len(feed), sum(1 for c in codes if c)))
     totals, groups = evaluate_grid(feed, head.image_detector, base, settings, batch_frames=args.batch_frames,
-                                   workers=args.workers, box_format=head.box_fmt, device=head.engine.device)
+                                   workers=args.workers, box_format=head.box_fmt, device=head.engine.device,
+                                   quality=spec)
     group_of = {i: gi for gi, g in enumerate(groups) for i in g["members"]}
     lines = []
     for i, (s, t) in enumerate(zip(grid, totals)):
@@ -215,6 +232,9 @@ def main(argv=None):
         lines.append(dict(setting=s, group=group_of[i], proposals=t["proposals"], recall=rec,
                           ar={str(th): rec["rcnn_%s" % th] / n_gt for th in extract.THRESH},
                           precision={str(th): t["precision"]["hits_%s" % th] / n_prop for th in extract.THRESH}))
+        if spec is not None:
+            from .quality import tables
+            lines[-1]["classes"] = tables(t["quality"], spec)
     lines.sort(key=lambda d: -d["ar"]["0.5"])       # stable: equal AR keeps grid order
     text = [json.dumps(d) for d in lines]
     for t in text:

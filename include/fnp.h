@@ -353,6 +353,33 @@ int fnp_precision_counters(const float *pred, const int32_t *pred_valid, const i
                            const int32_t *gt_start, int n_frames, int max_pred_per_frame, int max_gt_per_frame,
                            const float *thresh_host, int n_thresh, long long *counters, void *stream);
 
+/* Quality counters: recall and precision per class and per BEV range bin, for n_settings sets of proposals over the
+ * same frames and GT, in one launch.  The IoU of a (GT, proposal) pair is that of fnp_recall_counters, bit for bit,
+ * and each pair is computed once.
+ *   pred: setting s's rows start at pred + 7 * s * pred_setting_stride (0: every setting reads the same rows);
+ *   pred_valid (nullable): setting s's flags at pred_valid + s * valid_setting_stride, rows < 0 are not proposals;
+ *   pred_label (1-based class), pred_start (n_frames+1): shared by every setting;
+ *   gt (sum G,8) = box7 + 1-based class with gt_start (n_frames+1); trailing all-zero GT rows of a frame are dropped
+ *   as in fnp_recall_counters.
+ * Range: r = sqrt(x*x + y*y) of the box centre, each operation rounded in fp32; bin b = number of range edges <= r
+ * (edges strictly increasing, > 0).  A GT box is binned by its centre, a proposal by its own.
+ * T = n_thresh <= 8, R = n_edges + 1 <= 8, C = n_classes <= 32, W = 1 + 2T.  counters (int64), ACCUMULATED (caller
+ * zeroes them), 2 C R W per setting: setting s starts at counters + 2 C R W s, then
+ *   recall    [c][b][w], c = GT class - 1, b = GT bin:   w = 0 GT boxes;  1+t: best IoU over all valid proposals of
+ *             the frame > thresh[t];  1+T+t: the same over the proposals with the GT's label;
+ *   precision [c][b][w], c = label - 1, b = proposal bin: w = 0 valid proposals;  1+t: best IoU over the frame's GT
+ *             > thresh[t];  1+T+t: the same over the GT boxes of the proposal's class.
+ * Labels must lie in 1..C (the caller checks them; a box with another label is not counted).  Shared memory:
+ * fnp_quality_smem_bytes(...) <= 200 KB.  FNP_EINVAL: T, R or C out of range, bad edges, shared memory, a negative
+ * size or stride, a missing pointer.  Build record (nvcc 12.9, -Xptxas -v, sm_100a): quality_kernel 256 threads,
+ * 71 registers, 272-byte stack frame (box_overlap's vertex arrays), no spills; one CTA per (frame, 8 settings). */
+int fnp_quality_counters(const float *pred, long long pred_setting_stride, const int32_t *pred_valid,
+                         long long valid_setting_stride, const int32_t *pred_label, const int32_t *pred_start,
+                         int n_settings, const float *gt, const int32_t *gt_start, int n_frames, int max_pred_per_frame,
+                         int max_gt_per_frame, int n_classes, const float *range_edges_host, int n_edges,
+                         const float *thresh_host, int n_thresh, long long *counters, void *stream);
+size_t fnp_quality_smem_bytes(int max_pred_per_frame, int max_gt_per_frame, int n_classes, int n_edges, int n_thresh);
+
 /* ------------------------------------------------------------- host-side planning
  * (runs on the CPU, touches no device memory: every pointer here is a HOST pointer)
  *
