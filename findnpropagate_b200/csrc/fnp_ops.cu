@@ -755,6 +755,246 @@ __global__ void __launch_bounds__(256) upload_kernel(uint4 *__restrict__ dst, co
         dst[i] = src[i];
 }
 
+// ======================================================================================
+// Crop points in boxes: each point to the first box of its frame that contains it (the
+// predicate of points_in_boxes_kernel), then every box's points copied out contiguously, in
+// input order, with the box centre subtracted from x, y, z.
+//
+// A frame's points are cut into tiles of kCropTile rows.  Per frame the workspace holds a
+// tiles x boxes int32 matrix: crop_assign_kernel counts each tile's points per box in it,
+// crop_prefix_kernel turns every box's column into exclusive offsets over the tiles (and
+// writes the box's count), crop_starts_kernel scans the counts into row starts, and
+// crop_scatter_kernel copies each tile's points in order, one warp per tile, ranking points
+// of the same box within 32 rows with __match_any_sync.  Counting atomics only add; no
+// atomic decides a position, so the output is the same on every run.
+// ======================================================================================
+constexpr int kCropTile = 1024;
+constexpr int kCropThreads = 256;
+constexpr int kCropPerThread = kCropTile / kCropThreads;
+constexpr int kCropScanThreads = 1024;
+
+struct CropWs {                 // the workspace, carved as fnp_crop_workspace_bytes sizes it
+    int64_t *mat_start;         // (n_frames + 1): frame f's matrix at mat + mat_start[f]
+    int64_t *tile_start;        // (n_frames + 1): frame f's tiles are tile_start[f] ..
+    int32_t *box_of_pt;         // (n_points): box index within the frame, or -1
+    int32_t *mat;               // (mat_cap)
+    long long mat_cap, n_points, n_boxes;
+};
+
+// The starts end at the sizes the call was given and the matrix fits: otherwise no kernel
+// touches the outputs past counts (all zero), so a wrong call cannot write out of bounds.
+__device__ __forceinline__ bool crop_ok(const int64_t *__restrict__ row_start, const int64_t *__restrict__ box_start,
+                                        int n_frames, const CropWs &ws)
+{
+    return ws.mat_start[n_frames] <= ws.mat_cap && row_start[0] == 0 && box_start[0] == 0 &&
+           row_start[n_frames] == ws.n_points && box_start[n_frames] == ws.n_boxes;
+}
+
+__device__ __forceinline__ int crop_frame_of(const int64_t *__restrict__ start, int n_frames, long long v)
+{
+    int lo = 0, hi = n_frames - 1;      // last f with start[f] <= v
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (start[mid] <= v) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(kCropScanThreads) crop_plan_kernel(const int64_t *__restrict__ row_start,
+                                                                     const int64_t *__restrict__ box_start, int n_frames,
+                                                                     CropWs ws)
+{
+    __shared__ long long s_carry[2];
+    __shared__ long long s_warp[2][kCropScanThreads / 32];
+    if (threadIdx.x == 0) { s_carry[0] = 0; s_carry[1] = 0; }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int f0 = 0; f0 <= n_frames; f0 += kCropScanThreads) {
+        const int f = f0 + threadIdx.x;
+        long long v[2] = {0, 0};
+        if (f < n_frames) {
+            const long long tiles = (row_start[f + 1] - row_start[f] + kCropTile - 1) / kCropTile;
+            v[0] = tiles * (long long)(box_start[f + 1] - box_start[f]);
+            v[1] = tiles;
+        }
+        __syncthreads();
+        long long incl[2];
+        for (int k = 0; k < 2; k++) {
+            incl[k] = v[k];
+            for (int o = 1; o < 32; o <<= 1) {
+                const long long u = __shfl_up_sync(0xffffffffu, incl[k], o);
+                if (lane >= o) incl[k] += u;
+            }
+            if (lane == 31) s_warp[k][warp] = incl[k];
+        }
+        __syncthreads();
+        for (int k = 0; k < 2; k++) {
+            long long before = s_carry[k];
+            for (int w = 0; w < warp; w++) before += s_warp[k][w];
+            if (f <= n_frames) (k ? ws.tile_start : ws.mat_start)[f] = before + incl[k] - v[k];
+        }
+        __syncthreads();
+        if (threadIdx.x == 0)
+            for (int k = 0; k < 2; k++)
+                for (int w = 0; w < kCropScanThreads / 32; w++) s_carry[k] += s_warp[k][w];
+    }
+}
+
+// Tile -> (frame, first row, rows); false for a grid slot past the last tile or a matrix that
+// does not fit the workspace.
+__device__ __forceinline__ bool crop_tile(const int64_t *__restrict__ row_start, const int64_t *__restrict__ box_start,
+                                          int n_frames, const CropWs &ws, long long tile, int &f, long long &r0, int &n)
+{
+    if (n_frames == 0 || tile >= ws.tile_start[n_frames] || !crop_ok(row_start, box_start, n_frames, ws)) return false;
+    f = crop_frame_of(ws.tile_start, n_frames, tile);
+    const long long t = tile - ws.tile_start[f];
+    r0 = row_start[f] + t * kCropTile;
+    n = (int)min((long long)kCropTile, row_start[f + 1] - r0);
+    return true;
+}
+
+__global__ void __launch_bounds__(kCropThreads) crop_assign_kernel(const float *__restrict__ pts, int n_cols,
+                                                                   const int64_t *__restrict__ row_start,
+                                                                   const float *__restrict__ boxes,
+                                                                   const int64_t *__restrict__ box_start, int n_frames,
+                                                                   CropWs ws)
+{
+    __shared__ BoxPrep s_box[kCropThreads];
+    int f, n;
+    long long r0;
+    if (!crop_tile(row_start, box_start, n_frames, ws, blockIdx.x, f, r0, n)) return;
+    const long long b0 = box_start[f];
+    const int T = (int)(box_start[f + 1] - b0);
+    float x[kCropPerThread], y[kCropPerThread], z[kCropPerThread];
+    int found[kCropPerThread];
+#pragma unroll
+    for (int j = 0; j < kCropPerThread; j++) {
+        const int i = j * kCropThreads + threadIdx.x;
+        found[j] = i < n ? -1 : 0;          // 0: a slot past the tile's end, never tested
+        x[j] = y[j] = z[j] = 0.f;
+        if (i < n) {
+            const float *p = pts + (size_t)(r0 + i) * n_cols;
+            x[j] = p[0]; y[j] = p[1]; z[j] = p[2];
+        }
+    }
+    for (int t0 = 0; t0 < T; t0 += kCropThreads) {
+        const int nt = min(kCropThreads, T - t0);
+        __syncthreads();
+        if ((int)threadIdx.x < nt) s_box[threadIdx.x] = prep_box(boxes + (size_t)(b0 + t0 + threadIdx.x) * 7);
+        __syncthreads();
+        bool done = true;
+#pragma unroll
+        for (int j = 0; j < kCropPerThread; j++) {
+            if (found[j] < 0)
+                for (int k = 0; k < nt; k++)
+                    if (in_box(x[j], y[j], z[j], s_box[k])) { found[j] = t0 + k; break; }
+            done = done && found[j] >= 0;
+        }
+        if (__syncthreads_and(done)) break;
+    }
+    int32_t *row = ws.mat + ws.mat_start[f] + (blockIdx.x - ws.tile_start[f]) * (long long)T;
+#pragma unroll
+    for (int j = 0; j < kCropPerThread; j++) {
+        const int i = j * kCropThreads + threadIdx.x;
+        if (i < n) {
+            ws.box_of_pt[r0 + i] = found[j];
+            if (found[j] >= 0) atomicAdd(row + found[j], 1);
+        }
+    }
+}
+
+// One thread per box: its column of the frame's matrix becomes exclusive offsets over the tiles.
+__global__ void __launch_bounds__(128) crop_prefix_kernel(const int64_t *__restrict__ row_start,
+                                                          const int64_t *__restrict__ box_start, int n_frames,
+                                                          int n_boxes, CropWs ws, int32_t *__restrict__ counts)
+{
+    const int g = blockIdx.x * blockDim.x + threadIdx.x;
+    if (g >= n_boxes) return;
+    if (!crop_ok(row_start, box_start, n_frames, ws)) { counts[g] = 0; return; }
+    const int f = crop_frame_of(box_start, n_frames, g);
+    const long long T = box_start[f + 1] - box_start[f];
+    const long long tiles = ws.tile_start[f + 1] - ws.tile_start[f];
+    int32_t *col = ws.mat + ws.mat_start[f] + (g - box_start[f]);
+    int run = 0;
+    long long t = 0;
+    for (; t + 8 <= tiles; t += 8) {
+        int v[8];
+#pragma unroll
+        for (int k = 0; k < 8; k++) v[k] = col[(t + k) * T];
+#pragma unroll
+        for (int k = 0; k < 8; k++) { col[(t + k) * T] = run; run += v[k]; }
+    }
+    for (; t < tiles; t++) {
+        const int v = col[t * T];
+        col[t * T] = run;
+        run += v;
+    }
+    counts[g] = run;
+}
+
+// starts[g] = counts[0] + ... + counts[g-1] for g = 0 .. n_boxes (one CTA).
+__global__ void __launch_bounds__(kCropScanThreads) crop_starts_kernel(const int32_t *__restrict__ counts, int n_boxes,
+                                                                       int64_t *__restrict__ starts)
+{
+    __shared__ long long s_warp[kCropScanThreads / 32];
+    __shared__ long long s_carry;
+    if (threadIdx.x == 0) s_carry = 0;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int g0 = 0; g0 <= n_boxes; g0 += kCropScanThreads) {
+        const int g = g0 + threadIdx.x;
+        const long long v = g < n_boxes ? counts[g] : 0;
+        long long incl = v;
+        for (int o = 1; o < 32; o <<= 1) {
+            const long long u = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += u;
+        }
+        __syncthreads();
+        if (lane == 31) s_warp[warp] = incl;
+        __syncthreads();
+        long long before = s_carry;
+        for (int w = 0; w < warp; w++) before += s_warp[w];
+        if (g <= n_boxes) starts[g] = before + incl - v;
+        __syncthreads();
+        if (threadIdx.x == 0)
+            for (int w = 0; w < kCropScanThreads / 32; w++) s_carry += s_warp[w];
+    }
+}
+
+// One warp per tile, 32 rows at a time in input order.  The tile's matrix row holds, per box,
+// where its next point goes within the box; only this warp touches it.
+__global__ void __launch_bounds__(32) crop_scatter_kernel(const float *__restrict__ pts, int n_cols,
+                                                          const int64_t *__restrict__ row_start,
+                                                          const double *__restrict__ centres,
+                                                          const int64_t *__restrict__ box_start, int n_frames,
+                                                          CropWs ws, const int64_t *__restrict__ starts,
+                                                          float *__restrict__ rows)
+{
+    int f, n;
+    long long r0;
+    if (!crop_tile(row_start, box_start, n_frames, ws, blockIdx.x, f, r0, n)) return;
+    const long long b0 = box_start[f];
+    const long long T = box_start[f + 1] - b0;
+    int32_t *next = ws.mat + ws.mat_start[f] + (blockIdx.x - ws.tile_start[f]) * T;
+    const unsigned lane = threadIdx.x;
+    for (int i0 = 0; i0 < n; i0 += 32) {
+        const int i = i0 + (int)lane;
+        const int b = i < n ? ws.box_of_pt[r0 + i] : -1;
+        const unsigned same = __match_any_sync(0xffffffffu, b);
+        int base = 0;
+        if (b >= 0) base = next[b];
+        __syncwarp();
+        if (b >= 0 && lane == (unsigned)(__ffs(same) - 1)) next[b] = base + __popc(same);
+        __syncwarp();
+        if (b < 0) continue;
+        const long long g = b0 + b;
+        const long long out = starts[g] + base + __popc(same & ((1u << lane) - 1u));
+        const float *p = pts + (size_t)(r0 + i) * n_cols;
+        float *o = rows + (size_t)out * n_cols;
+#pragma unroll
+        for (int c = 0; c < 3; c++) o[c] = __double2float_rn(__dsub_rn((double)p[c], centres[g * 3 + c]));
+        for (int c = 3; c < n_cols; c++) o[c] = p[c];
+    }
+}
+
 // test hook: the device math routines exactly as this library's kernels see them
 __global__ void dbg_math_kernel(const float *__restrict__ x, const float *__restrict__ y, float *__restrict__ out, int n)
 {
@@ -802,6 +1042,66 @@ extern "C" int fnp_points_in_boxes(const float *boxes, const float *pts, int32_t
     if (B > 65535) return FNP_EINVAL;
     dim3 grid(divup(M, kPibThreads), B);
     points_in_boxes_kernel<<<grid, kPibThreads, 0, (cudaStream_t)stream>>>(boxes, pts, out, T, M);
+    FNP_LAUNCH_CHECK();
+    return FNP_OK;
+}
+
+static size_t crop_head_bytes(long long n_points, int n_frames)
+{
+    return (size_t)2 * (n_frames + 1) * 8 + ((size_t)n_points * 4 + 15) / 16 * 16;
+}
+
+extern "C" size_t fnp_crop_workspace_bytes(const int64_t *row_start_host, const int64_t *box_start_host, int n_frames)
+{
+    if (n_frames < 0 || (n_frames > 0 && (!row_start_host || !box_start_host))) return 0;
+    size_t mat = 0;
+    for (int f = 0; f < n_frames; f++) {
+        const long long n = row_start_host[f + 1] - row_start_host[f], g = box_start_host[f + 1] - box_start_host[f];
+        if (n > 0 && g > 0) mat += (size_t)((n + kCropTile - 1) / kCropTile) * (size_t)g;
+    }
+    return crop_head_bytes(n_frames ? row_start_host[n_frames] : 0, n_frames) + mat * 4 + 16;
+}
+
+extern "C" int fnp_crop_points_in_boxes(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                                        const float *boxes, const double *centres, const int64_t *box_start,
+                                        int n_boxes, int n_frames, int32_t *counts, int64_t *starts, float *rows,
+                                        void *workspace, size_t workspace_bytes, void *stream)
+{
+    if (n_cols < 3 || n_points < 0 || n_boxes < 0 || n_frames < 0 || n_frames > 65535 * 1024) return FNP_EINVAL;
+    if (n_frames == 0 && (n_points || n_boxes)) return FNP_EINVAL;
+    if (!row_start || !box_start || !starts || !workspace || (n_points && !pts) || (n_boxes && (!boxes || !centres || !counts)) ||
+        (n_points && n_boxes && !rows) || (reinterpret_cast<uintptr_t>(workspace) & 15))
+        return FNP_EINVAL;
+    const long long n_tiles = n_points / kCropTile + n_frames;
+    if (n_tiles > 0x7fffffffLL || divup(n_boxes, 128) > 0x7fffffff) return FNP_EINVAL;
+    const size_t head = crop_head_bytes(n_points, n_frames);
+    if (workspace_bytes < head + 16) return FNP_EWORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream;
+    char *w = static_cast<char *>(workspace);
+    CropWs ws;
+    ws.mat_start = reinterpret_cast<int64_t *>(w);
+    ws.tile_start = ws.mat_start + n_frames + 1;
+    ws.box_of_pt = reinterpret_cast<int32_t *>(ws.tile_start + n_frames + 1);
+    ws.mat = reinterpret_cast<int32_t *>(w + head);
+    ws.mat_cap = (long long)((workspace_bytes - head) / 4);
+    ws.n_points = n_points;
+    ws.n_boxes = n_boxes;
+    const cudaError_t e = cudaMemsetAsync(ws.mat, 0, workspace_bytes - head, s);
+    if (e != cudaSuccess) return (int)e;
+    crop_plan_kernel<<<1, kCropScanThreads, 0, s>>>(row_start, box_start, n_frames, ws);
+    FNP_LAUNCH_CHECK();
+    if (n_tiles > 0 && n_boxes > 0)
+        crop_assign_kernel<<<(unsigned)n_tiles, kCropThreads, 0, s>>>(pts, n_cols, row_start, boxes, box_start,
+                                                                      n_frames, ws);
+    FNP_LAUNCH_CHECK();
+    if (n_boxes > 0)
+        crop_prefix_kernel<<<divup(n_boxes, 128), 128, 0, s>>>(row_start, box_start, n_frames, n_boxes, ws, counts);
+    FNP_LAUNCH_CHECK();
+    crop_starts_kernel<<<1, kCropScanThreads, 0, s>>>(counts, n_boxes, starts);
+    FNP_LAUNCH_CHECK();
+    if (n_tiles > 0 && n_boxes > 0)
+        crop_scatter_kernel<<<(unsigned)n_tiles, 32, 0, s>>>(pts, n_cols, row_start, centres, box_start, n_frames, ws,
+                                                             starts, rows);
     FNP_LAUNCH_CHECK();
     return FNP_OK;
 }

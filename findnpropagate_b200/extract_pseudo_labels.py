@@ -83,12 +83,12 @@ def build_feed(cfg, infos=None):
 def check_frame(feed, detector, info) -> int:
     """0, or why the frame cannot run: its LiDAR file is missing; MAX_SWEEPS > 1 and a sweep file its info lists is
     missing (which sweeps the feed reads is drawn only at load time); one of its camera images is not in the
-    detector's predictions."""
+    detector's predictions (not checked when ``detector`` is None)."""
     if not (feed.root / info["lidar_path"]).is_file():
         return LIDAR_MISSING
     if feed.max_sweeps > 1 and not all((feed.root / s["lidar_path"]).is_file() for s in info["sweeps"]):
         return SWEEP_MISSING
-    if not all(detector.has_image(cam["data_path"]) for cam in info["cams"].values()):
+    if detector is not None and not all(detector.has_image(cam["data_path"]) for cam in info["cams"].values()):
         return IMAGE_NOT_PREDICTED
     return 0
 

@@ -6,9 +6,10 @@ per frame, every point is assigned to the FIRST GT box that contains it (one ``p
 of the frame's boxes), the points of each box are written to ``gt_database_<S>sweeps_withvelo/<frame>_<name>_<i>.bin``
 relative to the box centre, and one info dict per box goes into ``nuscenes_dbinfos_<S>sweeps_withvelo.pkl``.
 
-Here the frames of a batch are uploaded together and assigned by ONE ``fnp_points_in_boxes`` launch (B frames x T
-boxes x M points, the op's batched form; shorter frames are padded with a far-away point / an empty box), the rest is
-the same host-side bookkeeping and the same files, byte for byte.
+Here the frames of a batch are uploaded together and cropped by ONE ``fnp_crop_points_in_boxes`` call: the first-match
+assignment of ``fnp_points_in_boxes``, then every box's points in input order with the centre subtracted, on the
+device.  Only the counts and the rows in boxes come back.  The rest is the same host-side bookkeeping and the same
+files, byte for byte.
 """
 import pickle
 from pathlib import Path
@@ -18,30 +19,88 @@ import numpy as np
 import torch
 
 from .nuscenes_feed import lidar_with_sweeps
-from .pcdet_ops import roiaware_pool3d_utils
-
-_FAR = 1.0e6        # padding points lie in no box
 
 
-def assign_points_to_boxes(points_list, boxes_list, device=None):
-    """First containing box per point (or -1) for every frame of a batch, one launch.
-    points_list[b]: (N_b, >=3) float array, boxes_list[b]: (G_b, >=7).  Returns a list of (N_b,) int64 arrays --
-    what ``points_in_boxes_gpu(points[None], boxes[None]).long().squeeze(0).cpu().numpy()`` gives frame by frame."""
+def _starts(name, starts, total):
+    a = starts.numpy() if isinstance(starts, torch.Tensor) else np.asarray(starts)
+    if a.ndim != 1 or a.shape[0] < 1 or not np.issubdtype(a.dtype, np.integer):
+        raise ValueError("%s must be a 1-D integer array of n_frames + 1 entries" % name)
+    a = a.astype(np.int64)
+    if a[0] != 0 or a[-1] != total or (np.diff(a) < 0).any():
+        raise ValueError("%s must rise from 0 to %d, got %s .. %s" % (name, total, a[0], a[-1]))
+    return a
+
+
+def crop_points_in_boxes(points, row_start, boxes, centres, box_start):
+    """Every box's points, cropped on the device in one fnp_crop_points_in_boxes call.
+
+    points (N, C) float32 CUDA, C >= 3, x y z first; boxes (G, 7) float32 and centres (G, 3) float64 on the same
+    device; all contiguous.  row_start / box_start: host integer arrays (or CPU tensors) of n_frames + 1 entries,
+    frame f owning points row_start[f] .. row_start[f+1] and boxes box_start[f] .. box_start[f+1].
+    Each point goes to the first box of its frame that contains it (fnp_points_in_boxes' predicate).  Returns device
+    tensors counts (G,) int32, starts (G+1,) int64 and rows (N, C) float32: box g's points are rows
+    starts[g] .. starts[g] + counts[g], in input order, x y z as float32(float64(p) - centre).  ValueError for a bad
+    argument."""
+    from . import _lib
+    for name, t, dt, w in (("points", points, torch.float32, None), ("boxes", boxes, torch.float32, 7),
+                           ("centres", centres, torch.float64, 3)):
+        if not isinstance(t, torch.Tensor):
+            raise ValueError("%s must be a tensor, got %s" % (name, type(t).__name__))
+        if t.dtype != dt or t.dim() != 2 or (t.shape[1] != w if w else t.shape[1] < 3) or not t.is_contiguous():
+            raise ValueError("%s must be a contiguous (rows, %s) %s tensor, got %s %s"
+                             % (name, w or ">= 3", dt, t.dtype, tuple(t.shape)))
+    if boxes.shape[0] != centres.shape[0]:
+        raise ValueError("boxes and centres differ in length: %d and %d" % (boxes.shape[0], centres.shape[0]))
+    if any(isinstance(t, torch.Tensor) and t.is_cuda for t in (row_start, box_start)):
+        raise ValueError("row_start and box_start are host arrays")
+    N, C, G = points.shape[0], points.shape[1], boxes.shape[0]
+    rs, bs = _starts("row_start", row_start, N), _starts("box_start", box_start, G)
+    if rs.shape != bs.shape:
+        raise ValueError("row_start and box_start differ in length: %d and %d" % (rs.shape[0], bs.shape[0]))
+    dev = points.device
+    if not points.is_cuda or boxes.device != dev or centres.device != dev:
+        raise ValueError("points, boxes and centres must be on one CUDA device, got %s, %s, %s"
+                         % (points.device, boxes.device, centres.device))
+    F = rs.shape[0] - 1
+    ws_bytes = int(_lib.lib.fnp_crop_workspace_bytes(rs.ctypes.data, bs.ctypes.data, F))
+    d_starts = torch.from_numpy(np.concatenate([rs, bs])).to(dev)
+    counts = torch.empty(G, dtype=torch.int32, device=dev)
+    starts = torch.empty(G + 1, dtype=torch.int64, device=dev)
+    rows = torch.empty((N, C), dtype=torch.float32, device=dev)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        rc = _lib.lib.fnp_crop_points_in_boxes(points.data_ptr(), C, d_starts.data_ptr(), N, boxes.data_ptr(),
+                                               centres.data_ptr(), d_starts[F + 1:].data_ptr(), G, F,
+                                               counts.data_ptr(), starts.data_ptr(), rows.data_ptr(), ws.data_ptr(),
+                                               ws_bytes, _lib.current_stream(dev))
+    _lib.check(rc, "fnp_crop_points_in_boxes")
+    return counts, starts, rows
+
+
+def crop_frames(points_list, boxes_list, device=None):
+    """Per frame, the list of its boxes' points (n_i, C) float32, box-centred: ``pts[box_of_pt == i]`` then
+    ``[:, :3] -= boxes[i, :3]`` in the boxes' own precision, as create_groundtruth_database crops them.
+    points_list[b]: (N_b, C >= 3) float32 arrays; boxes_list[b]: (G_b, >= 7) float32 or float64 arrays.  One upload,
+    one crop call; the counts come back first, then only the rows that lie in a box."""
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
-    B = len(points_list)
-    if B == 0:
+    if not points_list:
         return []
-    M = max(max(p.shape[0] for p in points_list), 1)
-    T = max(max(g.shape[0] for g in boxes_list), 1)
-    pts = np.full((B, M, 3), _FAR, np.float32)
-    boxes = np.zeros((B, T, 7), np.float32)
-    boxes[:, :, 0:3] = -_FAR                  # padding boxes: zero size, far from every real and padding point
-    for b in range(B):
-        pts[b, :points_list[b].shape[0]] = np.asarray(points_list[b], np.float32)[:, 0:3]
-        boxes[b, :boxes_list[b].shape[0]] = np.asarray(boxes_list[b], np.float32)[:, 0:7]
-    idx = roiaware_pool3d_utils.points_in_boxes_gpu(torch.from_numpy(pts).to(dev), torch.from_numpy(boxes).to(dev))
-    idx = idx.long().cpu().numpy()
-    return [idx[b, :points_list[b].shape[0]] for b in range(B)]
+    C = points_list[0].shape[1]
+    pts = np.concatenate([np.asarray(p, np.float32).reshape(-1, C) for p in points_list])
+    box = np.concatenate([np.asarray(b)[:, :7] for b in boxes_list])
+    rs = np.concatenate([[0], np.cumsum([p.shape[0] for p in points_list])]).astype(np.int64)
+    bs = np.concatenate([[0], np.cumsum([len(b) for b in boxes_list])]).astype(np.int64)
+    counts, starts, rows = crop_points_in_boxes(
+        torch.from_numpy(pts).to(dev), rs, torch.from_numpy(np.ascontiguousarray(box, np.float32)).to(dev),
+        torch.from_numpy(np.ascontiguousarray(box[:, :3], np.float64)).to(dev), bs)
+    counts = counts.cpu().numpy()
+    total = int(counts.sum())
+    rows = rows[:total].cpu().numpy()
+    ends = np.cumsum(counts)
+    out = []
+    for b in range(len(points_list)):
+        out.append([rows[ends[g] - counts[g]:ends[g]] for g in range(bs[b], bs[b + 1])])
+    return out
 
 
 def create_groundtruth_database(root_path, infos: Sequence[dict], used_classes: Optional[Sequence[str]] = None,
@@ -56,14 +115,13 @@ def create_groundtruth_database(root_path, infos: Sequence[dict], used_classes: 
     for s in range(0, len(infos), batch_frames):
         chunk = list(range(s, min(s + batch_frames, len(infos))))
         points = [lidar_with_sweeps(root, infos[i], max_sweeps, rng) for i in chunk]       # the reference's order of draws
-        assigned = assign_points_to_boxes(points, [infos[i]['gt_boxes'] for i in chunk], device=device)
+        cropped = crop_frames(points, [infos[i]['gt_boxes'] for i in chunk], device=device)
         for k, idx in enumerate(chunk):
-            info, pts, box_of_pt = infos[idx], points[k], assigned[k]
+            info = infos[idx]
             gt_boxes, gt_names = info['gt_boxes'], info['gt_names']
             for i in range(gt_boxes.shape[0]):
                 filepath = db_dir / ('%s_%s_%d.bin' % (idx, gt_names[i], i))
-                gt_points = pts[box_of_pt == i]
-                gt_points[:, :3] -= gt_boxes[i, :3]
+                gt_points = cropped[k][i]
                 with open(filepath, 'w') as f:
                     gt_points.tofile(f)
                 if (used_classes is None) or gt_names[i] in used_classes:

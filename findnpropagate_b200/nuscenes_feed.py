@@ -73,21 +73,32 @@ def load_sweep(root: Path, sweep_info: dict):
     return pts.T, times.T
 
 
-def lidar_with_sweeps(root: Path, info: dict, max_sweeps: int = 1, rng=None) -> np.ndarray:
-    """(N,5) float32 [x, y, z, intensity, time]: the key frame followed by max_sweeps - 1 earlier
-    sweeps drawn without replacement (nuscenes_dataset.py:105-124; the reference draws from the
-    global numpy generator, pass ``rng`` for a private one)."""
+def draw_sweeps(info: dict, max_sweeps: int = 1, rng=None) -> np.ndarray:
+    """Indices into ``info['sweeps']`` of the max_sweeps - 1 earlier sweeps a frame reads, drawn without replacement
+    (nuscenes_dataset.py:105-124; the reference draws from the global numpy generator, pass ``rng`` for a private one)."""
     rng = np.random if rng is None else rng
+    return rng.choice(len(info['sweeps']), max_sweeps - 1, replace=False)
+
+
+def read_lidar_with_sweeps(root: Path, info: dict, sweep_ids) -> np.ndarray:
+    """(N,5) float32 [x, y, z, intensity, time]: the key frame followed by the sweeps ``sweep_ids`` (draw_sweeps)."""
     points = np.fromfile(str(root / info['lidar_path']), dtype=np.float32, count=-1).reshape([-1, 5])[:, :4]
     pts_list = [points]
     times_list = [np.zeros((points.shape[0], 1))]
-    for k in rng.choice(len(info['sweeps']), max_sweeps - 1, replace=False):
+    for k in sweep_ids:
         p, t = load_sweep(root, info['sweeps'][k])
         pts_list.append(p)
         times_list.append(t)
     points = np.concatenate(pts_list, axis=0)
     times = np.concatenate(times_list, axis=0).astype(points.dtype)
     return np.concatenate((points, times), axis=1)
+
+
+def lidar_with_sweeps(root: Path, info: dict, max_sweeps: int = 1, rng=None) -> np.ndarray:
+    """(N,5) float32 [x, y, z, intensity, time]: the key frame followed by max_sweeps - 1 earlier
+    sweeps drawn without replacement (nuscenes_dataset.py:105-124; the reference draws from the
+    global numpy generator, pass ``rng`` for a private one)."""
+    return read_lidar_with_sweeps(root, info, draw_sweeps(info, max_sweeps, rng))
 
 
 def camera_info(info: dict) -> dict:

@@ -39,6 +39,33 @@ def bev_nms(boxes, scores, thresh=0.5):
     return keep.numpy() if is_numpy else keep
 
 
+def seg_nms_keep(boxes_list, scores_list, thresh, device=None):
+    """Per frame, the indices of the rows ``load_pseudos(nms_thresh=thresh)`` keeps, in its order (descending score,
+    ties by row), for many frames in one fnp_seg_nms_rotated launch.  boxes_list[f]: (K_f, >= 7), scores_list[f]:
+    (K_f,).  ValueError for a frame of more than SEG_NMS_MAX boxes."""
+    from . import _lib
+    ks = np.array([len(s) for s in scores_list], np.int64)
+    if ks.max(initial=0) > _lib.SEG_NMS_MAX:
+        raise ValueError("frame %d has %d boxes, the NMS takes at most %d per frame"
+                         % (int(np.argmax(ks)), int(ks.max()), _lib.SEG_NMS_MAX))
+    n = len(ks)
+    start = np.concatenate([[0], np.cumsum(ks)]).astype(np.int32)
+    if start[-1] == 0:
+        return [np.zeros(0, np.int64) for _ in range(n)]
+    boxes = np.ascontiguousarray(np.concatenate([np.asarray(b, np.float32)[:, :7] for b in boxes_list]))
+    scores = np.concatenate([np.asarray(s, np.float32) for s in scores_list])
+    order = np.lexsort((-scores, np.repeat(np.arange(n), ks))).astype(np.int32)    # stable: ties by row
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    d_boxes, d_order, d_start = (torch.from_numpy(a).to(dev) for a in (boxes, order, start))
+    keep = torch.empty(boxes.shape[0], dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib.fnp_seg_nms_rotated(d_boxes.data_ptr(), None, d_order.data_ptr(), None, d_start.data_ptr(),
+                                                n, int(ks.max()), float(thresh), keep.data_ptr(),
+                                                _lib.current_stream(dev)), "fnp_seg_nms_rotated")
+    keep = keep.cpu().numpy().astype(bool)
+    return [order[start[f]:start[f + 1]][keep[order[start[f]:start[f + 1]]]] - start[f] for f in range(n)]
+
+
 def pseudo_path(folder, frame_id):
     return os.path.join(str(folder), "%s.pth" % str(frame_id).replace('.', '_'))
 

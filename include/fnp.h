@@ -64,6 +64,36 @@ int fnp_points_in_boxes(const float *boxes, const float *pts, int32_t *out, int 
 int fnp_count_in_boxes(const float *pts4, const int32_t *pt_start, const float *boxes,
                        const int32_t *box_start, int n_segments, int32_t *counts, void *stream);
 
+/* Points of every box, cropped out of a batch of ragged frames (the crop of create_groundtruth_database,
+ * nuscenes_dataset.py:346-390: pts[box_idxs_of_pts == i], then xyz minus the box centre).
+ *   pts (n_points, n_cols) f32, n_cols >= 3, x y z first; frame f's rows are row_start[f] .. row_start[f+1]
+ *   (int64, n_frames+1, row_start[0] = 0, row_start[n_frames] = n_points);
+ *   boxes (n_boxes, 7) f32 and centres (n_boxes, 3) f64, frame f's boxes box_start[f] .. box_start[f+1] (int64,
+ *   the same rule with n_boxes).
+ * Each point goes to the FIRST box of its frame that contains it, by the predicate of fnp_points_in_boxes
+ * (prep_box / in_box), so the assignment is that op's bit for bit.  Outputs, caller-allocated:
+ *   counts (n_boxes) int32, starts (n_boxes+1) int64 (exclusive scan of counts), rows (n_points, n_cols) f32 of
+ *   which rows starts[b] .. starts[b]+counts[b] are box b's points in input order, x y z as
+ *   (float)((double)p - centre) (numpy's f32_rows[:, :3] -= f64_centre) and the other columns copied.
+ * Each point lands in at most one box, so rows never needs more than n_points rows; there is no cap on points or
+ * boxes per frame.  The order is fixed by per-tile counts, a scan and a per-tile ordered scatter: no atomic picks a
+ * position, and two runs give the same bytes.
+ * workspace: 16-byte aligned, at least fnp_crop_workspace_bytes(host copies of row_start, box_start, n_frames)
+ * bytes (4 bytes per point plus 4 per (1024-point tile, box) pair of each frame); FNP_EWORKSPACE when it cannot
+ * hold the per-point part.  Starts that do not end at n_points / n_boxes, or a workspace too small for the
+ * per-tile part, leave every count 0 and write no row (checked on the device).  FNP_EINVAL: n_cols < 3, a
+ * negative size, frames without n_frames, a missing pointer.  Build record (nvcc 12.9, -Xptxas -v, sm_100a), no
+ * stack, no spills: crop_plan_kernel 1024 threads, 32 registers; crop_assign_kernel 256 threads, 48 registers;
+ * crop_prefix_kernel 128 threads, 61 registers; crop_starts_kernel 1024 threads, 30 registers;
+ * crop_scatter_kernel 32 threads (one warp per tile), 64 registers. */
+int fnp_crop_points_in_boxes(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                             const float *boxes, const double *centres, const int64_t *box_start, int n_boxes,
+                             int n_frames, int32_t *counts, int64_t *starts, float *rows, void *workspace,
+                             size_t workspace_bytes, void *stream);
+/* HOST pointers: row_start_host, box_start_host as passed (on the device) to fnp_crop_points_in_boxes; 0 for a
+ * negative n_frames or a missing pointer. */
+size_t fnp_crop_workspace_bytes(const int64_t *row_start_host, const int64_t *box_start_host, int n_frames);
+
 /* The (N, P) 0/1 matrix of the reference's CPU op points_in_boxes_cpu (roiaware_pool3d.cpp:121-168): NOT
  * the GPU predicate -- the margin is 1e-2 instead of 1e-5 and the products are rounded individually, with
  * the host libm's cosf / sinf.  box_prep (N,8) device = fnp_host_prep_boxes_cpu(boxes) uploaded (the per-box
