@@ -59,24 +59,26 @@ __global__ void __launch_bounds__(kCntThreads) count_segments_kernel(const float
     __shared__ float4 s_pts[kCntTile];
     const int seg = blockIdx.x;
     const int b0 = box_start[seg], nb = box_start[seg + 1] - b0;
-    const int h = blockIdx.y * kCntThreads + threadIdx.x;
-    if ((int)blockIdx.y * kCntThreads >= nb) return;
     const int p0 = pt_start[seg], np = pt_start[seg + 1] - p0;
-    BoxPrep bp;
-    if (h < nb) bp = prep_box(boxes + (size_t)(b0 + h) * 7);
-    else { bp.cx = bp.cy = bp.cz = 0.f; bp.hz = -1.f; bp.cosa = 1.f; bp.sina = 0.f; bp.tx = bp.ty = -1.f; }
-    int cnt = 0;
-    for (int t0 = 0; t0 < np; t0 += kCntTile) {
-        const int m = min(kCntTile, np - t0);
-        __syncthreads();
-        for (int i = threadIdx.x; i < m; i += kCntThreads) s_pts[i] = pts[p0 + t0 + i];
-        __syncthreads();
-        for (int i = 0; i < m; i++) {
-            const float4 q = s_pts[i];
-            count_if(cnt, in_box(q.x, q.y, q.z, bp));
+    // the CTAs of a segment stride over its boxes, gridDim.y * kCntThreads at a time (the bound is uniform per CTA)
+    for (int hb = blockIdx.y * kCntThreads; hb < nb; hb += gridDim.y * kCntThreads) {
+        const int h = hb + threadIdx.x;
+        BoxPrep bp;
+        if (h < nb) bp = prep_box(boxes + (size_t)(b0 + h) * 7);
+        else { bp.cx = bp.cy = bp.cz = 0.f; bp.hz = -1.f; bp.cosa = 1.f; bp.sina = 0.f; bp.tx = bp.ty = -1.f; }
+        int cnt = 0;
+        for (int t0 = 0; t0 < np; t0 += kCntTile) {
+            const int m = min(kCntTile, np - t0);
+            __syncthreads();
+            for (int i = threadIdx.x; i < m; i += kCntThreads) s_pts[i] = pts[p0 + t0 + i];
+            __syncthreads();
+            for (int i = 0; i < m; i++) {
+                const float4 q = s_pts[i];
+                count_if(cnt, in_box(q.x, q.y, q.z, bp));
+            }
         }
+        if (h < nb) counts[b0 + h] = cnt;
     }
-    if (h < nb) counts[b0 + h] = cnt;
 }
 
 // ======================================================================================
@@ -251,13 +253,22 @@ __device__ float box_overlap(const RBox &A, const RBox &B)
     return __fmul_rn(fabsf(area), 0.5f);
 }
 
-// True only when box_overlap(A, B) is exactly 0: the centres are further apart than both half
-// diagonals plus a slack that covers the 1e-2 corner margin of in_box2d and all rounding, so the
-// polygon clipper would find no edge intersection and no contained corner (cnt == 0 -> area 0).
+// |d|/2 + 1e-2 of a box side d from t = fma(d, 0.5, 1e-2): t itself for d >= 0, and 2e-2 - t for d < 0,
+// where t falls below 1e-2 (a negative size spans the same corners as its absolute value)
+__device__ __forceinline__ float abs_half_side(float t)
+{
+    return t >= 1e-2f ? t : 2e-2f - t;
+}
+
+// True only when box_overlap(A, B) is exactly 0, for any finite box (a negative or zero size too): the
+// centres are further apart than both half diagonals plus a slack that covers the 1e-2 corner margin of
+// in_box2d and all rounding, so the polygon clipper would find no edge intersection and no contained
+// corner (cnt == 0 -> area 0).  For sizes >= 0 the radius is tx + ty, bit for bit.
 __device__ __forceinline__ bool surely_disjoint(const RBox &A, const RBox &B)
 {
     const float ddx = A.cx - B.cx, ddy = A.cy - B.cy;
-    const float ra = A.tx + A.ty, rb = B.tx + B.ty;        // >= half diagonal + margin (L1 >= L2)
+    // >= half diagonal + margin (L1 >= L2)
+    const float ra = abs_half_side(A.tx) + abs_half_side(A.ty), rb = abs_half_side(B.tx) + abs_half_side(B.ty);
     const float r = ra + rb + 0.1f;
     return ddx * ddx + ddy * ddy > 1.0001f * r * r;
 }
@@ -1112,7 +1123,7 @@ extern "C" int fnp_count_in_boxes(const float *pts4, const int32_t *pt_start, co
     if (n_segments < 0) return FNP_EINVAL;
     if (n_segments == 0) return FNP_OK;
     if (!pt_start || !box_start || !counts) return FNP_EINVAL;
-    // boxes per segment are not known on the host: cover up to 4096 per segment
+    // boxes per segment are not known on the host: 32 CTAs per segment, each striding over the segment's boxes
     dim3 grid(n_segments, 32);
     count_segments_kernel<<<grid, kCntThreads, 0, (cudaStream_t)stream>>>(
         reinterpret_cast<const float4 *>(pts4), pt_start, boxes, box_start, counts);

@@ -60,7 +60,8 @@ int fnp_points_in_boxes(const float *boxes, const float *pts, int32_t *out, int 
  * pts4[pt_start[s] .. pt_start[s+1]) (float4 x,y,z,_) are tested against boxes
  * boxes[box_start[s] .. box_start[s+1]) (7 floats each); counts[] is indexed like boxes.
  * Same predicate as fnp_points_in_boxes; count = what the reference obtains with one
- * points_in_boxes_gpu call + (idx >= 0).sum() per box (frustum_proposals_v1.py:930-932). */
+ * points_in_boxes_gpu call + (idx >= 0).sum() per box (frustum_proposals_v1.py:930-932).
+ * There is no cap on the points or boxes of a segment: every count is written. */
 int fnp_count_in_boxes(const float *pts4, const int32_t *pt_start, const float *boxes,
                        const int32_t *box_start, int n_segments, int32_t *counts, void *stream);
 
