@@ -152,14 +152,8 @@ def extract_nuscenes(feed, detector, engine, folder: Optional[str] = None, batch
     local, recall = [], {}
 
     def finish(job):
-        h, ids, rerun = job
-        while True:
-            try:
-                res = engine.finish(h)
-                break
-            except OverflowError as e:      # frustum-point buffer too small: grow it, run the batch again
-                engine.pts_factor = max(engine.pts_factor * 1.5, 1.25 * int(e.args[0]) / max(h["plan"]["total_rows"], 1))
-                h = rerun()
+        h, ids = job
+        res = engine.result(h)
         for j, fid in enumerate(ids):
             local.append(res["frames"][j])
             if folder is not None:
@@ -198,12 +192,9 @@ def _pipeline(cur, batches, feeder, engine, stride, stage, finish, nms_thresh):
             stage((k + 1) % 2, nxt[0])                      # gathered while this batch runs
         plan = engine.plan(frames, stride=stride)
         gt = engine.upload_gt(frames)
-        def run(plan=plan, pts=pts, gt=gt, slot=slot, ready=ready):
-            h = engine.execute(plan, pts, nms_thresh=nms_thresh, gt=gt, slot=slot, points_ready=ready)
-            feeder.mark_consumed(slot)
-            return h
-        h = run()
+        h = engine.execute(plan, pts, nms_thresh=nms_thresh, gt=gt, slot=slot, points_ready=ready)
+        feeder.mark_consumed(slot)
         if prev is not None:
             finish(prev)                                    # overlaps the kernels of this batch
-        prev, cur, k = (h, ids, run), nxt, k + 1
+        prev, cur, k = (h, ids), nxt, k + 1
     return prev

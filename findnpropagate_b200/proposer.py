@@ -356,14 +356,7 @@ class FrustumProposerOG(nn.Module):
             bounds.astype(np.int64), stride, xyz_offset, cam_mats, self._np(det_boxes).astype(np.float32).reshape(-1, 4),
             self._np(det_labels).astype(np.int64), self._np(det_scores).astype(np.float32),
             self._np(det_batch_idx).astype(np.int64), self._np(det_cam_idx).astype(np.int64))
-        while True:
-            h = self.engine.execute(plan, pts)
-            try:
-                res = self.engine.finish(h)
-                break
-            except OverflowError as e:
-                self.engine.pts_factor = max(self.engine.pts_factor * 1.5,
-                                             1.25 * int(e.args[0]) / max(plan["total_rows"], 1))
+        res = self.engine.result(self.engine.execute(plan, pts))
         boxes, labels, scores, bi = [], [], [], []
         for b, fr in enumerate(res["frames"]):
             boxes.append(fr["pred_boxes"]); labels.append(fr["pred_labels"]); scores.append(fr["pred_scores"])
@@ -458,14 +451,7 @@ class FrustumProposerOGKITTI(nn.Module):
                                           det_boxes=det_boxes[m], det_labels=det_labels[m], det_scores=det_scores[m],
                                           device=str(dev)))
         plan = self.engine.plan(frames, xyz_offset=1, stride=int(pts.shape[1]))
-        while True:
-            h = self.engine.execute(plan, pts)
-            try:
-                res = self.engine.finish(h)
-                break
-            except OverflowError as e:
-                self.engine.pts_factor = max(self.engine.pts_factor * 1.5,
-                                             1.25 * int(e.args[0]) / max(plan["total_rows"], 1))
+        res = self.engine.result(self.engine.execute(plan, pts))
         boxes, labels, scores, bi = [], [], [], []
         for b, fr in enumerate(res["frames"]):
             boxes.append(fr["pred_boxes"]); labels.append(fr["pred_labels"]); scores.append(fr["pred_scores"])

@@ -18,6 +18,7 @@ per-frame Python loop replaced by five fused CUDA stages over a *batch* of frame
 There is no CPU compute path: the engine raises if CUDA or the extension is missing.
 """
 import ctypes as C
+import math
 import time
 from dataclasses import dataclass
 from typing import List, Optional
@@ -294,6 +295,47 @@ class _FrameResults:
 
 def _align(x, a=256):
     return (x + a - 1) // a * a
+
+
+_F32, _I32, _I64, _U8 = (np.dtype(t) for t in (np.float32, np.int32, np.int64, np.uint8))
+
+
+class OutLayout:
+    """The output block of one execute(), which comes back in one D2H: its regions in this order, each at the next
+    offset aligned for its dtype.  Per proposal slot (F*T of them, T = topk slots per candidate): boxes, score, best
+    (compacted hypothesis index, -1: unused), count; per candidate: npts, nvalid; status (include/fnp.h: 8 int32);
+    the recall counters; the stage-4 keep flags.  Then, for S settings of evaluate_settings: boxes, score, best, count
+    per setting and candidate, the recall and the precision counters per setting, and n_quality quality counters per
+    setting (quality.QualitySpec.n_counters)."""
+
+    def __init__(self, F, T=1, S=0, n_quality=0):
+        FT, NC, NP = F * T, SeekerEngine.N_COUNTERS, SeekerEngine.N_PRECISION
+        self.regions, end = {}, 0            # name -> (byte offset, dtype, shape)
+        for name, dt, shape in (
+                ("boxes", _F32, (FT, 7)), ("score", _F32, (FT,)), ("best", _I32, (FT,)), ("count", _I32, (FT,)),
+                ("npts", _I32, (F,)), ("nvalid", _I32, (F,)), ("status", _I32, (8,)), ("recall", _I64, (NC,)),
+                ("keep", _U8, (FT,)), ("sel_boxes", _F32, (S, F, 7)), ("sel_score", _F32, (S, F)),
+                ("sel_best", _I32, (S, F)), ("sel_count", _I32, (S, F)), ("sel_recall", _I64, (S, NC)),
+                ("sel_precision", _I64, (S, NP)), ("quality", _I64, (S, n_quality))):
+            off = _align(end, dt.itemsize)
+            self.regions[name] = (off, dt, shape)
+            end = off + dt.itemsize * math.prod(shape)
+        self.nbytes = end
+
+    def span(self, first, last=None):
+        """Byte range of region `first`, or of the regions `first` through `last`."""
+        off, dt, shape = self.regions[last or first]
+        return slice(self.regions[first][0], off + dt.itemsize * math.prod(shape))
+
+    def ptr(self, base, name, row=0):
+        """Device address of region `name` (or of its row `row` along the first axis) in the block at `base`."""
+        off, dt, shape = self.regions[name]
+        return base + off + row * dt.itemsize * math.prod(shape[1:])
+
+    def view(self, raw, name):
+        """Region `name` of a host copy of the block (a uint8 array) as a shaped numpy array."""
+        _, dt, shape = self.regions[name]
+        return raw[self.span(name)].view(dt).reshape(shape)
 
 
 class SeekerEngine:
@@ -622,20 +664,7 @@ class SeekerEngine:
                 hyp_iou=4 * H * F, counts=4 * H * F, items=16 * max_items,
                 cand_item_start=4 * (F + 1), sweep_cols=4 * _lib.SWEEP_COL_FLOATS * self.J * F,
                 )
-            # outputs, one D2H: boxes(7) score best count per proposal slot (T per candidate), npts nvalid
-            # per candidate, status(4) + pad(4), recall counters (20 x int64), stage-4 keep flags (F T bytes)
-            T = self.T
-            FT = F * T
-            off_recall = 4 * (10 * FT + 2 * F + 8)
-            off_keep = off_recall + 8 * self.N_COUNTERS
-            # per setting: boxes(7) score best count per candidate, then recall and precision counters per setting
-            off_sel = off_keep + _align(FT, 8)
-            off_sel_counters = off_sel + 40 * S * F
-            sizes["out"] = off_sel_counters + 8 * S * (self.N_COUNTERS + self.N_PRECISION)
-            off_quality = sizes["out"]
-            if quality is not None:             # per setting: the class x range counters (quality.QualitySpec)
-                sizes["out"] += 8 * S * quality.n_counters
-            if T > 1:
+            if self.T > 1:
                 sizes["hyp_score"] = 4 * H * F
             if use_dist:
                 sizes["hyp_dist"] = 4 * H * F
@@ -646,11 +675,10 @@ class SeekerEngine:
             # every slot owns its intermediates, so that batches of different slots may be in flight on
             # different streams at the same time (slot 0 keeps the plain names: debug_views reads them)
             sfx = "" if slot == 0 else "@%d" % slot
-            ptr = {k: self.arena.get(k + sfx, v).data_ptr() for k, v in sizes.items() if k != "out"}
-            out_dev = self.arena.get("out%d" % slot, sizes["out"])
+            ptr = {k: self.arena.get(k + sfx, v).data_ptr() for k, v in sizes.items()}
+            lay = OutLayout(F, self.T, S, quality.n_counters if quality is not None else 0)
+            out_dev = self.arena.get("out%d" % slot, lay.nbytes)
             ob = out_dev.data_ptr()
-            o_boxes, o_score, o_best, o_count = ob, ob + 28 * FT, ob + 32 * FT, ob + 36 * FT
-            o_npts, o_nvalid, o_status = ob + 40 * FT, ob + 40 * FT + 4 * F, ob + 40 * FT + 8 * F
             b = _lib.SeekerBatch(
                 n_frames=B, n_cands=F, n_tiles=plan["n_tiles"], max_cands_per_frame=Cmax,
                 points=points_dev.data_ptr(), point_stride=plan["stride"], xyz_offset=plan["xyz_offset"],
@@ -661,19 +689,20 @@ class SeekerEngine:
                 cand_label=meta["cand_label"], cand_box2d=meta["cand_box2d"],
                 base_boxes=self.base_boxes.data_ptr(), base_corners=self.base_corners.data_ptr(),
                 mags=self.mags.data_ptr(),
-                cell_masks=ptr["cell_masks"], mask_words=W, cand_npts=o_npts, page_tab=ptr["page_tab"],
+                cell_masks=ptr["cell_masks"], mask_words=W, cand_npts=lay.ptr(ob, "npts"), page_tab=ptr["page_tab"],
                 page_tab_stride=tab_stride, page_planes=planes, frustum_pts=ptr["frustum_pts"], pts_capacity=cap,
                 cand_stats=ptr["cand_stats"], centres=ptr["centres"], hyp_prep=ptr["hyp_prep"],
-                hyp_index=ptr["hyp_index"], hyp_iou=ptr["hyp_iou"], hyp_nvalid=o_nvalid,
+                hyp_index=ptr["hyp_index"], hyp_iou=ptr["hyp_iou"], hyp_nvalid=lay.ptr(ob, "nvalid"),
                 hyp_boxes_dbg=ptr.get("hyp_boxes_dbg"), hyp_iou_dbg=ptr.get("hyp_iou_dbg"),
                 hyp_valid_dbg=ptr.get("hyp_valid_dbg"),
                 split_points=sp, max_items=max_items,
                 cand_item_start=ptr["cand_item_start"], items=ptr["items"],
                 counts=ptr["counts"], score_mode=self.score_mode, sweep_cols=ptr["sweep_cols"],
-                out_boxes=o_boxes, out_score=o_score, out_best=o_best, out_count=o_count, status=o_status,
+                out_boxes=lay.ptr(ob, "boxes"), out_score=lay.ptr(ob, "score"), out_best=lay.ptr(ob, "best"),
+                out_count=lay.ptr(ob, "count"), status=lay.ptr(ob, "status"),
                 hyp_dist=ptr.get("hyp_dist"), hyp_nfar=ptr.get("hyp_nfar"), hyp_score=ptr.get("hyp_score"))
             if self.rand_center and F and plan["n_tiles"]:
-                self._run_rand_center(b, stream, F, M, out_dev[40 * FT:40 * FT + 4 * F].view(torch.int32),
+                self._run_rand_center(b, stream, F, M, out_dev[lay.span("npts")].view(torch.int32),
                                       self.arena.bufs["cand_stats" + sfx], self.arena.bufs["centres" + sfx])
             else:
                 rc = _lib.lib.fnp_seeker_run(C.byref(self.cfg), C.byref(b), stream)
@@ -681,25 +710,25 @@ class SeekerEngine:
             mode = _lib.lib.fnp_seeker_score_mode(C.byref(self.cfg), C.byref(b))
             self.last_score_mode = {_lib.SCORE_DIRECT: "direct", _lib.SCORE_SWEEP: "sweep"}.get(mode)
             self.launches += (9 + (mode == _lib.SCORE_SWEEP) + self.use_occl) if F and plan["n_tiles"] else 0
-            handle = dict(plan=plan, batch=b, sp=sp, cap=cap, out_dev=out_dev, out_bytes=sizes["out"], meta=meta,
-                          tab_stride=tab_stride, planes=planes,
-                          off_recall=off_recall, off_keep=off_keep, has_nms=False, has_recall=False,
-                          recall_thresh=tuple(recall_thresh), n_settings=S, off_sel=off_sel,
-                          off_sel_counters=off_sel_counters, quality=None, off_quality=off_quality)
+            handle = dict(plan=plan, batch=b, sp=sp, cap=cap, out_dev=out_dev, layout=lay, meta=meta,
+                          tab_stride=tab_stride, planes=planes, has_nms=False, has_recall=False,
+                          recall_thresh=tuple(recall_thresh), n_settings=S, quality=None,
+                          args=dict(plan=plan, points_dev=points_dev, nms_thresh=nms_thresh, gt=gt,
+                                    recall_thresh=recall_thresh, slot=slot, points_ready=points_ready,
+                                    settings=settings, quality=quality))
             if S and F:
-                self._select_multi(plan, meta, b, sel, use_occl, gt, recall_thresh, stream, out_dev, off_sel,
-                                   off_sel_counters)
+                self._select_multi(handle, b, sel, use_occl, gt, recall_thresh, stream)
                 if quality is not None and gt is not None:
-                    self._quality(plan, meta, S, gt, quality, stream, out_dev, off_sel, off_quality)
+                    self._quality(handle, gt, quality, stream)
                     handle["quality"] = quality
             if nms_thresh is not None and F:
-                self._stage4_nms(plan, meta, o_boxes, o_best, float(nms_thresh), stream, ob + off_keep)
+                self._stage4_nms(handle, float(nms_thresh), stream)
                 handle["has_nms"] = True
             if gt is not None and F:
-                self._recall(plan, meta, o_boxes, o_best, gt, recall_thresh, stream, out_dev, off_recall)
+                self._recall(handle, gt, recall_thresh, stream)
                 handle["has_recall"] = True
-            host = self.arena.get("out_host%d" % slot, sizes["out"], pinned=True)
-            host[:sizes["out"]].copy_(out_dev[:sizes["out"]], non_blocking=True)
+            host = self.arena.get("out_host%d" % slot, lay.nbytes, pinned=True)
+            host[:lay.nbytes].copy_(out_dev[:lay.nbytes], non_blocking=True)
             handle["out_host"] = host
             handle["event"] = torch.cuda.Event()
             handle["event"].record()
@@ -708,76 +737,79 @@ class SeekerEngine:
 
     N_COUNTERS = 5 + 5 * 3          # generate_recall_record counters for 3 IoU thresholds
 
-    def _stage4_nms(self, plan, meta, o_boxes, o_best, thresh, stream, keep_ptr):
+    def _stage4_nms(self, handle, thresh, stream):
         """Rotated-BEV NMS of each frame's proposals in 2D-score order (the dedup
         PseudoLoader applies later on the CPU, pseudo_loader.py:29-55,755)."""
-        T = self.T
+        plan, meta, lay, ob, T = handle["plan"], handle["meta"], handle["layout"], handle["out_dev"].data_ptr(), self.T
         if plan["max_cands"] * T > _lib.SEG_NMS_MAX:
             raise ValueError("stage-4 NMS handles at most %d proposals per frame" % _lib.SEG_NMS_MAX)
-        rc = _lib.lib.fnp_seg_nms_rotated(o_boxes, None, meta["nms_order" if T == 1 else "prop_order"], o_best,
+        rc = _lib.lib.fnp_seg_nms_rotated(lay.ptr(ob, "boxes"), None, meta["nms_order" if T == 1 else "prop_order"],
+                                          lay.ptr(ob, "best"),
                                           meta["frame_cand_start" if T == 1 else "frame_prop_start"], plan["B"],
                                           int(min(max(plan["max_cands"] * T, 1), _lib.SEG_NMS_MAX)), thresh,
-                                          keep_ptr, stream)
+                                          lay.ptr(ob, "keep"), stream)
         _lib.check(rc, "fnp_seg_nms_rotated")
         self.launches += 1
 
-    def _recall(self, plan, meta, o_boxes, o_best, gt, thresh, stream, out_dev, off):
+    def _recall(self, handle, gt, thresh, stream):
+        plan, meta, lay, out_dev = handle["plan"], handle["meta"], handle["layout"], handle["out_dev"]
+        ob = out_dev.data_ptr()
         gt_boxes, gt_start, max_gt = gt
         assert len(thresh) == 3
-        out_dev[off:off + 8 * self.N_COUNTERS].zero_()
+        out_dev[lay.span("recall")].zero_()
         th = (C.c_float * len(thresh))(*[float(t) for t in thresh])
-        rc = _lib.lib.fnp_recall_counters(o_boxes, o_best, meta["frame_cand_start" if self.T == 1 else "frame_prop_start"],
+        rc = _lib.lib.fnp_recall_counters(lay.ptr(ob, "boxes"), lay.ptr(ob, "best"),
+                                          meta["frame_cand_start" if self.T == 1 else "frame_prop_start"],
                                           gt_boxes.data_ptr(), gt_start.data_ptr(), plan["B"],
                                           max(plan["max_cands"] * self.T, 1), int(max_gt), th, len(thresh),
-                                          out_dev.data_ptr() + off, stream)
+                                          lay.ptr(ob, "recall"), stream)
         _lib.check(rc, "fnp_recall_counters")
         self.launches += 1
 
     N_PRECISION = 1 + 3             # valid proposals, then hits at 3 IoU thresholds (fnp_precision_counters)
 
-    def _select_multi(self, plan, meta, b, sel, use_occl, gt, thresh, stream, out_dev, off, off_counters):
+    def _select_multi(self, handle, b, sel, use_occl, gt, thresh, stream):
         """Stage 3 once per setting over this execution's stages 1-2c, then each setting's recall and precision."""
-        L, F, S = _lib.lib, plan["F"], len(sel)
+        plan, meta, lay, out_dev = handle["plan"], handle["meta"], handle["layout"], handle["out_dev"]
+        L, ob, S = _lib.lib, out_dev.data_ptr(), len(sel)
         if use_occl and not self.use_occl:      # this engine's own cfg leaves stage 2c off
             cfg = _lib.SeekerCfg.from_buffer_copy(self.cfg)
             cfg.flags |= _lib.SEEKER_OCCL_MULT
             _lib.check(L.fnp_seeker_occlusion(C.byref(cfg), C.byref(b), stream), "fnp_seeker_occlusion")
             self.launches += 1
-        ob = out_dev.data_ptr() + off
-        boxes, best = ob, ob + 32 * S * F
         # one launch per FNP_SELECT_MAX_SETTINGS settings (the kernel-parameter block), all over the same stages 1-2c
         for c0 in range(0, S, _lib.SELECT_MAX_SETTINGS):
             n = min(_lib.SELECT_MAX_SETTINGS, S - c0)
             chunk = (_lib.SelectSetting * n)(*sel[c0:c0 + n])
-            _lib.check(L.fnp_seeker_select_multi(C.byref(self.cfg), C.byref(b), chunk, n, boxes + 28 * c0 * F,
-                                                 ob + 28 * S * F + 4 * c0 * F, best + 4 * c0 * F,
-                                                 ob + 36 * S * F + 4 * c0 * F, stream), "fnp_seeker_select_multi")
+            rows = [lay.ptr(ob, k, c0) for k in ("sel_boxes", "sel_score", "sel_best", "sel_count")]
+            _lib.check(L.fnp_seeker_select_multi(C.byref(self.cfg), C.byref(b), chunk, n, *rows, stream),
+                       "fnp_seeker_select_multi")
             self.launches += 1
         if gt is None:
             return
         gt_boxes, gt_start, max_gt = gt
-        out_dev[off_counters:off_counters + 8 * S * (self.N_COUNTERS + self.N_PRECISION)].zero_()
+        out_dev[lay.span("sel_recall", "sel_precision")].zero_()
         th = (C.c_float * len(thresh))(*[float(t) for t in thresh])
         for s in range(S):
-            for fn, n, base in ((L.fnp_recall_counters, self.N_COUNTERS, off_counters),
-                                (L.fnp_precision_counters, self.N_PRECISION, off_counters + 8 * S * self.N_COUNTERS)):
-                rc = fn(boxes + 28 * s * F, best + 4 * s * F, meta["frame_cand_start"], gt_boxes.data_ptr(),
-                        gt_start.data_ptr(), plan["B"], max(plan["max_cands"], 1), int(max_gt), th, len(thresh),
-                        out_dev.data_ptr() + base + 8 * s * n, stream)
+            for fn, counters in ((L.fnp_recall_counters, "sel_recall"), (L.fnp_precision_counters, "sel_precision")):
+                rc = fn(lay.ptr(ob, "sel_boxes", s), lay.ptr(ob, "sel_best", s), meta["frame_cand_start"],
+                        gt_boxes.data_ptr(), gt_start.data_ptr(), plan["B"], max(plan["max_cands"], 1), int(max_gt), th,
+                        len(thresh), lay.ptr(ob, counters, s), stream)
                 _lib.check(rc, fn.__name__)
         self.launches += 2 * S
 
-    def _quality(self, plan, meta, S, gt, spec, stream, out_dev, off, off_quality):
+    def _quality(self, handle, gt, spec, stream):
         """One fnp_quality_counters launch over every setting's proposals (the boxes and flags _select_multi wrote);
         labels are the candidates' 2D labels, shared by the settings."""
         from . import quality
-        F = plan["F"]
+        plan, meta, lay, out_dev = handle["plan"], handle["meta"], handle["layout"], handle["out_dev"]
+        ob, F = out_dev.data_ptr(), plan["F"]
         gt_boxes, gt_start, max_gt = gt
-        out_dev[off_quality:off_quality + 8 * S * spec.n_counters].zero_()
-        ob = out_dev.data_ptr() + off
-        quality.launch(spec, ob, meta["cand_label"], meta["frame_cand_start"], gt_boxes, gt_start, plan["B"],
-                       max(plan["max_cands"], 1), int(max_gt), out_dev.data_ptr() + off_quality, n_settings=S,
-                       pred_valid=ob + 32 * S * F, pred_stride=F, valid_stride=F, stream=stream)
+        out_dev[lay.span("quality")].zero_()
+        quality.launch(spec, lay.ptr(ob, "sel_boxes"), meta["cand_label"], meta["frame_cand_start"], gt_boxes, gt_start,
+                       plan["B"], max(plan["max_cands"], 1), int(max_gt), lay.ptr(ob, "quality"),
+                       n_settings=handle["n_settings"], pred_valid=lay.ptr(ob, "sel_best"), pred_stride=F,
+                       valid_stride=F, stream=stream)
         self.launches += 1
 
     def evaluate_settings(self, plan, points_dev, gt, settings, recall_thresh=(0.3, 0.5, 0.7), quality=None):
@@ -802,13 +834,20 @@ class SeekerEngine:
             from .quality import check_labels
             check_labels(quality, plan["cand_label"], gt[0].cpu().numpy(), gt[1].cpu().numpy())
             quality.check_size(plan["max_cands"], gt[2], "the largest frame of the batch")
+        return self.result(self.execute(plan, points_dev, gt=gt, recall_thresh=recall_thresh, settings=settings,
+                                         quality=quality))
+
+    def result(self, handle):
+        """finish(handle), recovering from a page pool too small for the batch: the pool grows (pts_factor) and the
+        batch runs again with execute()'s original arguments until it fits.  The handle is updated in place, so that
+        afterwards it describes the run whose results are returned."""
         while True:
-            h = self.execute(plan, points_dev, gt=gt, recall_thresh=recall_thresh, settings=settings, quality=quality)
             try:
-                return self.finish(h)
+                return self.finish(handle)
             except OverflowError as e:
                 need = int(e.args[0])
-                self.pts_factor = max(self.pts_factor * 1.5, 1.25 * need / max(plan["total_rows"], 1))
+                self.pts_factor = max(self.pts_factor * 1.5, 1.25 * need / max(handle["plan"]["total_rows"], 1))
+                handle.update(self.execute(**handle["args"]))
 
     def finish(self, handle):
         """Wait for the batch and assemble per-frame results (reference output format)."""
@@ -816,18 +855,9 @@ class SeekerEngine:
         t0 = time.perf_counter()
         plan = handle["plan"]
         F, B = plan["F"], plan["B"]
-        raw = handle["out_host"].numpy()[:handle["out_bytes"]]
-        f32 = raw.view(np.float32)
-        i32 = raw.view(np.int32)
-        T = self.T
-        FT = F * T
-        boxes = f32[0:7 * FT].reshape(FT, 7)
-        score = f32[7 * FT:8 * FT]
-        best = i32[8 * FT:9 * FT]
-        count = i32[9 * FT:10 * FT]
-        npts = i32[10 * FT:10 * FT + F]
-        nvalid = i32[10 * FT + F:10 * FT + 2 * F]
-        status = i32[10 * FT + 2 * F:10 * FT + 2 * F + 4]
+        raw, lay, T = handle["out_host"].numpy(), handle["layout"], self.T
+        boxes, score, best, count, npts, nvalid, status = (lay.view(raw, k) for k in (
+            "boxes", "score", "best", "count", "npts", "nvalid", "status"))
         if status[0] & 1:
             raise OverflowError(int(status[1]))
         if status[0] & 2:
@@ -840,7 +870,7 @@ class SeekerEngine:
         cand_of = idx if T == 1 else idx // T      # slot -> candidate: 2D score and label repeat (:1048-1052)
         c_boxes, c_scores = boxes[idx], plan["cand_score"][cand_of]
         c_labels = plan["cand_label"][cand_of].astype(np.int32)
-        c_keep = raw[handle["off_keep"]:handle["off_keep"] + FT][idx].astype(bool) if handle["has_nms"] else None
+        c_keep = lay.view(raw, "keep")[idx].astype(bool) if handle["has_nms"] else None
         frames = _FrameResults(c_boxes, c_scores, c_labels, c_keep, np.searchsorted(idx, fcs * T))
         # per-candidate views: the best proposal of each (slot 0); cand_topk has every slot
         res = dict(frames=frames, cand_valid=ok[::T].copy(), cand_best=best[::T].copy(), cand_score2=score[::T].copy(),
@@ -850,26 +880,17 @@ class SeekerEngine:
             res["cand_topk"] = dict(best=best.reshape(F, T).copy(), score2=score.reshape(F, T).copy(),
                                     boxes=boxes.reshape(F, T, 7).copy(), count=count.reshape(F, T).copy())
         if handle["has_recall"]:
-            o = handle["off_recall"]
-            res["recall"] = self.recall_dict(raw[o:o + 8 * self.N_COUNTERS].view(np.int64), handle["recall_thresh"])
+            res["recall"] = self.recall_dict(lay.view(raw, "recall"), handle["recall_thresh"])
         S = handle["n_settings"]
         if S:
-            o, oc = handle["off_sel"], handle["off_sel_counters"]
-            sb = raw[o:o + 28 * S * F].view(np.float32).reshape(S, F, 7)
-            ss = raw[o + 28 * S * F:o + 32 * S * F].view(np.float32).reshape(S, F)
-            si = raw[o + 32 * S * F:o + 40 * S * F].view(np.int32).reshape(2, S, F)
-            rec = raw[oc:oc + 8 * S * self.N_COUNTERS].view(np.int64).reshape(S, self.N_COUNTERS)
-            oc += 8 * S * self.N_COUNTERS
-            prec = raw[oc:oc + 8 * S * self.N_PRECISION].view(np.int64).reshape(S, self.N_PRECISION)
+            sb, ss, sbest, scount, rec, prec, qc = (lay.view(raw, k) for k in (
+                "sel_boxes", "sel_score", "sel_best", "sel_count", "sel_recall", "sel_precision", "quality"))
             th = handle["recall_thresh"]
             spec = handle.get("quality")
-            if spec is not None:
-                oq = handle["off_quality"]
-                qc = raw[oq:oq + 8 * S * spec.n_counters].view(np.int64).reshape(S, spec.n_counters)
             res["settings"] = []
             for s in range(S):
-                d = dict(proposals=int((si[0, s] >= 0).sum()), cand_best=si[0, s].copy(), cand_score2=ss[s].copy(),
-                         cand_count=si[1, s].copy(), cand_boxes=sb[s].copy())
+                d = dict(proposals=int((sbest[s] >= 0).sum()), cand_best=sbest[s].copy(), cand_score2=ss[s].copy(),
+                         cand_count=scount[s].copy(), cand_boxes=sb[s].copy())
                 if handle["has_recall"]:
                     d["recall"] = self.recall_dict(rec[s], th)
                     d["precision"] = dict(proposals=int(prec[s, 0]),
@@ -912,13 +933,7 @@ class SeekerEngine:
         if points_dev is None:
             points_dev = self.upload_points(frames)
         gt = self.upload_gt(frames) if with_recall else None
-        while True:
-            h = self.execute(plan, points_dev, nms_thresh=nms_thresh, gt=gt)
-            try:
-                return self.finish(h)
-            except OverflowError as e:
-                need = int(e.args[0])
-                self.pts_factor = max(self.pts_factor * 1.5, 1.25 * need / max(plan["total_rows"], 1))
+        return self.result(self.execute(plan, points_dev, nms_thresh=nms_thresh, gt=gt))
 
     def upload_points(self, frames):
         rows = sum(f.points.shape[0] for f in frames)
@@ -959,7 +974,7 @@ class SeekerEngine:
         # the page pool -> one (x, y, z, d) row per point, frustum by frustum, sorted by source row (stage 1 fills
         # a frustum in whatever order the tiles reach it; no result depends on that order, this view fixes one)
         PG, planes, ts = _lib.PAGE_POINTS, handle["planes"], handle["tab_stride"]
-        npts = handle["out_host"].numpy()[:handle["out_bytes"]].view(np.int32)[10 * F * self.T:10 * F * self.T + F]
+        npts = handle["layout"].view(handle["out_host"].numpy(), "npts")
         tab = view("page_tab", torch.int32, (F, ts))
         n_pages = int(tab.max()) if F else 0
         pool = view("frustum_pts", torch.float32, (max(n_pages, 1), planes, PG))

@@ -296,6 +296,20 @@ def test_evaluate_settings_quality():
             assert np.array_equal(plain[k], res[k])
         assert plain.get("recall") == res.get("recall")
     assert checked > 20
+    # a page pool too small for the batch: it grows and the batch runs again, to what a roomy pool gives
+    starved = SeekerEngine(g["params"], device="cuda:0")
+    starved.pts_factor = 0.05
+    low = starved.evaluate_settings(plan, pts, gt, g["settings"], quality=SPEC)
+    roomy = eng.evaluate_settings(plan, pts, gt, g["settings"], quality=SPEC)
+    assert starved.pts_factor > 0.05 and len(low["settings"]) == len(roomy["settings"]) == len(g["settings"])
+    for k in ("cand_valid", "cand_best", "cand_score2", "cand_count", "cand_npts", "cand_nvalid"):
+        assert np.array_equal(low[k], roomy[k]), k
+    v = roomy["cand_valid"]                     # the boxes of candidates without a proposal are not written
+    assert np.array_equal(low["cand_boxes"][v], roomy["cand_boxes"][v]) and low["recall"] == roomy["recall"]
+    for a, b in zip(low["settings"], roomy["settings"]):
+        assert set(a) == set(b)
+        for k in a:
+            assert np.array_equal(a[k], b[k]) if isinstance(a[k], np.ndarray) else a[k] == b[k], k
 
 
 # ------------------------------------------------------------------------------------------------- 6, 7

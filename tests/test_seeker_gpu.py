@@ -398,6 +398,13 @@ def test_reference_compatible_head_and_extraction(tmp_path):
     assert bidx.dtype == torch.int64 and boxes.shape[0] == labels.shape[0] == scores.shape[0] == bidx.shape[0]
     out = head(bd)["final_box_dicts"]
     assert len(out) == 3 and out[0]["pred_labels"].dtype == torch.int32
+    # a page pool too small for the batch: the head grows it, runs the batch again and gives the same proposals
+    starved = proposer.FrustumProposerOG(model_cfg=dict(PARAMS=params, PREDS_PATH="PreprocessedGLIP", BOX_FORMAT="xyxy"),
+                                         class_names=synth.CLASS_NAMES, image_detector=feeder).eval()
+    starved.engine.pts_factor = 0.05
+    got = starved.get_proposals(bd)
+    assert starved.engine.pts_factor > 0.05
+    assert all(torch.equal(g, w) for g, w in zip(got, (boxes, labels, scores, bidx)))
     eng = SeekerEngine(params, device="cuda:0")
     for b, f in enumerate(sf):
         ora = _oracle(_frame_from_synth(f), params, eng)
@@ -638,6 +645,14 @@ def test_nuscenes_feed_to_pth_pipeline(tmp_path, pack_xyz, loader_xyz):
         assert isinstance(saved, list) and len(saved) == 1
         assert np.array_equal(saved[0]["pred_boxes"].numpy(), merged[i]["pred_boxes"])
         assert saved[0]["pred_labels"].dtype == torch.int32
+    # a page pool too small for a batch: the pipeline runs that batch again in a grown pool, with the same results
+    starved = SeekerEngine(params, device="cuda:0")
+    starved.pts_factor = 0.05
+    merged2, total2, _ = extract.extract_nuscenes(feed, glip, starved, batch_frames=2, nms_thresh=0.1, pack_xyz=pack_xyz,
+                                                  workers=2, loader_xyz=loader_xyz)
+    assert starved.pts_factor > 0.05 and total2 == total
+    for a, b in zip(merged2, merged):
+        assert set(a) == set(b) and all(np.array_equal(a[k], b[k]) for k in a)
     # the feed reproduces the generator's frames: same points after the range filter, same detections
     assert np.array_equal(frames[0].points, sf[0].points[nuscenes_feed.mask_points_by_range(sf[0].points, nuscenes_feed.POINT_CLOUD_RANGE)])
     assert sum(m["pred_boxes"].shape[0] for m in merged) > 0

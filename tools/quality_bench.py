@@ -51,16 +51,10 @@ def main():
     gt_boxes, gt_start, max_gt = gt = eng.upload_gt(frames)
     spec = quality.QualitySpec(synth.CLASS_NAMES)
     quality.check_labels(spec, plan["cand_label"], gt_boxes.cpu().numpy(), gt_start.cpu().numpy())
-    while True:     # the per-setting proposals stay in the engine's output block
-        h = eng.execute(plan, points, gt=gt, settings=settings)
-        try:
-            res = eng.finish(h)
-            break
-        except OverflowError as err:
-            eng.pts_factor = max(eng.pts_factor * 1.5, 1.25 * int(err.args[0]) / plan["total_rows"])
-    F, B, meta = plan["F"], plan["B"], h["meta"]
-    ob = h["out_dev"].data_ptr() + h["off_sel"]
-    boxes, best = ob, ob + 32 * S * F
+    h = eng.execute(plan, points, gt=gt, settings=settings)
+    res = eng.result(h)         # the per-setting proposals stay in the engine's output block
+    F, B, meta, lay, ob = plan["F"], plan["B"], h["meta"], h["layout"], h["out_dev"].data_ptr()
+    boxes, best = lay.ptr(ob, "sel_boxes"), lay.ptr(ob, "sel_best")
     max_k = max(plan["max_cands"], 1)
     stream = _lib.current_stream()
     th = (C.c_float * 3)(*spec.thresh)
@@ -78,8 +72,9 @@ def main():
         prec_out.zero_()
         for s in range(S):
             for fn, out in ((_lib.lib.fnp_recall_counters, rec_out), (_lib.lib.fnp_precision_counters, prec_out)):
-                _lib.check(fn(boxes + 28 * s * F, best + 4 * s * F, meta["frame_cand_start"], gt_boxes.data_ptr(),
-                              gt_start.data_ptr(), B, max_k, int(max_gt), th, 3, out[s].data_ptr(), stream), fn.__name__)
+                _lib.check(fn(lay.ptr(ob, "sel_boxes", s), lay.ptr(ob, "sel_best", s), meta["frame_cand_start"],
+                              gt_boxes.data_ptr(), gt_start.data_ptr(), B, max_k, int(max_gt), th, 3, out[s].data_ptr(),
+                              stream), fn.__name__)
 
     def timed(fn):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

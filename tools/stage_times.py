@@ -69,12 +69,8 @@ def main():
         torch.cuda.synchronize()
         out["stages_ms"][name] = e0.elapsed_time(e1) / a.iters
     # stage 4 + recall, timed through the engine helpers
-    meta = h["meta"]
-    ob = h["out_dev"].data_ptr()
-    F = plan["F"]
-    for name, fn in (("seg_nms", lambda: eng._stage4_nms(plan, meta, ob, ob + 32 * F, 0.1, stream, ob + h["off_keep"])),
-                     ("recall", lambda: eng._recall(plan, meta, ob, ob + 32 * F, gt, (0.3, 0.5, 0.7), stream,
-                                                    h["out_dev"], h["off_recall"]))):
+    for name, fn in (("seg_nms", lambda: eng._stage4_nms(h, 0.1, stream)),
+                     ("recall", lambda: eng._recall(h, gt, (0.3, 0.5, 0.7), stream))):
         fn(); torch.cuda.synchronize()
         e0.record()
         for _ in range(a.iters):

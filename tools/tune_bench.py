@@ -77,12 +77,7 @@ def main():
             out = [None] * len(settings)
             order = [i for g in groups for i in g["members"]]
             for i, (gi, e) in zip(order, separate):
-                while True:
-                    try:
-                        res = e.finish(e.execute(plans[gi], points, gt=gt))
-                        break
-                    except OverflowError as err:      # page pool too small: grow it and run again, as run() does
-                        e.pts_factor = max(e.pts_factor * 1.5, 1.25 * int(err.args[0]) / plans[gi]["total_rows"])
+                res = e.result(e.execute(plans[gi], points, gt=gt))
                 out[i] = (int(res["cand_valid"].sum()), res.get("recall"))
             return out
 
