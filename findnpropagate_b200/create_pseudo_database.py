@@ -17,8 +17,9 @@ database OpenPCDet's ``DataBaseSampler`` reads, in the format of ``create_ground
 The points are ``lidar_with_sweeps(root, info, MAX_SWEEPS, RandomState(--seed))`` without range filter or ego-point
 removal on the key frame (the GT database's rule).  The sweeps are drawn on the main thread once per frame of the info
 list, in order, and the files are read on ``--workers`` threads, so two runs write the same bytes.  Every refusal
-(existing output, missing folder, a label outside the classes, ``WORLD_SIZE`` > 1, a frame over the NMS's box limit)
-exits with status 1 before anything is written.
+(existing output, missing folder, a label outside the classes, ``WORLD_SIZE`` > 1, a frame over the NMS's box limit, a
+KITTI config: KITTI's ``kitti_dbinfos`` / ``gt_database`` layout is another format) exits with status 1 before anything
+is written.
 """
 import argparse
 import os
@@ -101,11 +102,14 @@ def main(argv=None):
         _fail("%s does not exist or is not a folder" % args.folder)
     if args.batch_frames < 1 or args.workers < 1:
         _fail("--batch_frames and --workers must be at least 1")
-    from .extract_pseudo_labels import FAILURES, build_feed, check_frame, load_config
+    from .extract_pseudo_labels import FAILURES, build_feed, check_frame, is_kitti, load_config
     try:
         cfg = load_config(args.cfg_file, args.set_cfgs)
     except (OSError, KeyError, ValueError) as e:
         _fail(e.args[-1] if isinstance(e, KeyError) else e)
+    if is_kitti(cfg):
+        _fail("DATA_CONFIG.DATASET KittiDataset is not supported: this command writes the nuScenes database layout "
+              "(KITTI's kitti_dbinfos / gt_database format is not written)")
     feed = build_feed(cfg)
     names = list(feed.class_names)
     if args.labels is not None:

@@ -8,6 +8,7 @@
 //   stage 2a  :851-911,:1392-1411 hypothesis grid, softmin front shift, distance/IoU filters
 //   stage 2b  :930-932            one points_in_boxes_gpu launch + sum + D2H per hypothesis
 //   stage 3   :994-1053           density+IoU score, sort, nms_normal(thresh 1), top-1
+#include <cstring>
 #include <string>
 
 #include "fnp_common.cuh"
@@ -2016,6 +2017,10 @@ __global__ void __launch_bounds__(128) select_kernel(const fnp_seeker_batch b, c
 // valid set is the compacted hypotheses with iou > its min_cam_iou, the count / occlusion / ego normalisers are
 // maxima over that set, and the arg-max of hyp_score over it breaks ties on the lowest index (compaction keeps the
 // original order, so that is also the lowest original index: select_kernel's choice for a cfg with those values).
+// KITTI = true is FrustumProposerOGKITTI's score (fnp_seeker_select_multi admits it only when every setting keeps the
+// cfg's min_cam_iou, so the valid set, and with it every first-match count, is the one stages 1-2c produced): the
+// count normaliser is the SUM of the compacted counts, exact in any order below 2^24 points as in select_kernel, the
+// distance plane is always staged and the score is hyp_score with kitti = true.
 constexpr int kMultiThreads = 256;
 constexpr int kMultiPlaneDist = 1, kMultiPlaneFail = 2, kMultiPlaneEgo = 4;
 
@@ -2023,6 +2028,7 @@ struct SelectSettings {
     fnp_select_setting s[FNP_SELECT_MAX_SETTINGS];
 };
 
+template <bool KITTI>
 __global__ void __launch_bounds__(kMultiThreads) select_multi_kernel(const fnp_seeker_batch b, const int J, const int H,
                                                                     const SelectSettings set, const int n_set,
                                                                     const int planes, float *out_boxes, float *out_score,
@@ -2035,7 +2041,7 @@ __global__ void __launch_bounds__(kMultiThreads) select_multi_kernel(const fnp_s
     int *s_cnt = reinterpret_cast<int *>(smem);
     float *s_iou = reinterpret_cast<float *>(s_cnt + H);
     float *p_next = s_iou + H;
-    float *s_dist = (planes & kMultiPlaneDist) ? p_next : nullptr;
+    float *s_dist = (KITTI || (planes & kMultiPlaneDist)) ? p_next : nullptr;
     p_next += s_dist ? H : 0;
     float *s_fail = (planes & kMultiPlaneFail) ? p_next : nullptr;
     p_next += s_fail ? H : 0;
@@ -2063,19 +2069,21 @@ __global__ void __launch_bounds__(kMultiThreads) select_multi_kernel(const fnp_s
     for (int si = warp; si < n_set; si += kMultiThreads / 32) {
         const fnp_select_setting p = set.s[si];
         const bool mult = (p.flags & FNP_SEEKER_MULT) != 0, occl_mult = (p.flags & FNP_SEEKER_OCCL_MULT) != 0;
-        const ScoreTerms t = {p.dns_w, p.iou_w, p.dst_w, p.ego_w, p.occl_w, false, mult, occl_mult,
-                              (p.dst_w != 0.f) || mult, p.occl_w > 0.f, p.ego_w > 0.f};
-        const bool use_fail = t.use_occl_w || occl_mult;
+        const ScoreTerms t = KITTI ? ScoreTerms{p.dns_w, p.iou_w, p.dst_w, 0.f, 0.f, true, false, false, true, false, false}
+                                   : ScoreTerms{p.dns_w, p.iou_w, p.dst_w, p.ego_w, p.occl_w, false, mult, occl_mult,
+                                                (p.dst_w != 0.f) || mult, p.occl_w > 0.f, p.ego_w > 0.f};
+        const bool use_fail = t.use_occl_w || t.occl_mult;
         const float thr = p.min_cam_iou;
         int mxi = 0;
         float fmx = 0.f, emx = 0.f;
         for (int r = lane; r < nv; r += 32) {
             if (!(s_iou[r] > thr)) continue;
-            mxi = max(mxi, s_cnt[r]);
+            mxi = KITTI ? mxi + s_cnt[r] : max(mxi, s_cnt[r]);
             if (use_fail) fmx = fmaxf(fmx, s_fail[r]);
             if (t.use_ego) emx = fmaxf(emx, s_ego[r]);
         }
-        const float den = __fadd_rn(warp_max((float)mxi), 1e-8f);
+        const float den = KITTI ? __fadd_rn((float)__reduce_add_sync(0xffffffffu, mxi), 1e-8f)
+                                : __fadd_rn(warp_max((float)mxi), 1e-8f);
         const float fden = use_fail ? __fadd_rn(warp_max(fmx), 1e-6f) : 1.f;
         if (t.use_ego) emx = warp_max(emx);
         float best = -__int_as_float(0x7f800000);
@@ -2346,14 +2354,22 @@ extern "C" int fnp_seeker_select_multi(const fnp_seeker_cfg *cfg, const fnp_seek
     int rc = check_batch(cfg, b);
     if (rc) return rc;
     if (!settings_host || n_settings < 1 || n_settings > FNP_SELECT_MAX_SETTINGS) return FNP_EINVAL;
-    // KITTI: first-match counts depend on the valid set; topk > 1: the suppression pass is not repeated per setting
-    if (cfg->topk > 1 || cfg->variant == FNP_VARIANT_KITTI) return FNP_EINVAL;
+    // topk > 1: the suppression pass is not repeated per setting
+    if (cfg->topk > 1) return FNP_EINVAL;
+    const bool kitti = cfg->variant == FNP_VARIANT_KITTI;
     SelectSettings set = {};
-    int planes = 0;
+    int planes = kitti ? kMultiPlaneDist : 0;
     for (int i = 0; i < n_settings; i++) {
         const fnp_select_setting &s = settings_host[i];
         if (s.flags & ~(FNP_SEEKER_MULT | FNP_SEEKER_OCCL_MULT)) return FNP_EINVAL;
         if (!(s.min_cam_iou >= cfg->min_cam_iou)) return FNP_EINVAL;    // compacted at cfg's threshold
+        if (kitti) {
+            // first-match counts depend on the valid set: only the one stages 1-2c compacted, and only that head's terms
+            uint32_t a, c;
+            memcpy(&a, &s.min_cam_iou, 4);
+            memcpy(&c, &cfg->min_cam_iou, 4);
+            if (a != c || s.flags != 0 || s.ego_w > 0.f || s.occl_w > 0.f) return FNP_EINVAL;
+        }
         if ((s.dst_w != 0.f) || (s.flags & FNP_SEEKER_MULT)) planes |= kMultiPlaneDist;
         if ((s.occl_w > 0.f) || (s.flags & FNP_SEEKER_OCCL_MULT)) planes |= kMultiPlaneFail;
         if (s.ego_w > 0.f) planes |= kMultiPlaneEgo;
@@ -2365,9 +2381,10 @@ extern "C" int fnp_seeker_select_multi(const fnp_seeker_cfg *cfg, const fnp_seek
     const int J = cfg->num_yaw_size, H = J * cfg->num_mags;
     const size_t smem = (size_t)H * 4 * (2 + __builtin_popcount(planes));
     if (smem > 200 * 1024) return FNP_EINVAL;
-    cudaFuncSetAttribute(select_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    select_multi_kernel<<<b->n_cands, kMultiThreads, smem, (cudaStream_t)stream>>>(*b, J, H, set, n_settings, planes,
-                                                                                out_boxes, out_score, out_best, out_count);
+    auto kernel = kitti ? select_multi_kernel<true> : select_multi_kernel<false>;
+    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    kernel<<<b->n_cands, kMultiThreads, smem, (cudaStream_t)stream>>>(*b, J, H, set, n_settings, planes, out_boxes,
+                                                                      out_score, out_best, out_count);
     FNP_LAUNCH_CHECK();
     return FNP_OK;
 }

@@ -4,8 +4,8 @@
 
 reads the ``.pth`` file of every frame of the config's info list (``<folder>/<frame_id with . -> _>.pth``, the format
 ``extract_pseudo_labels`` and the reference's tool write, read as ``pseudo_loader.load_pseudos`` reads it) and scores
-it against the frame's GT as the extraction tool's loader produces it (``NuScenesFeed.gt_boxes``, training mode; the
-LiDAR files are not read).  ``--nms_thresh T ...`` also scores the folder as self-training reads it after
+it against the frame's GT as the extraction tool's loader produces it (``NuScenesFeed.gt_boxes`` or
+``KittiFeed.gt_boxes``, training mode; the LiDAR files are not read), with the classes of the config's CLASS_NAMES.  ``--nms_thresh T ...`` also scores the folder as self-training reads it after
 ``load_pseudos(nms_thresh=T)``; every threshold is one more setting of the same fnp_quality_counters launch.
 
 Per NMS setting it prints one JSON line: ``nms``, ``frames``, ``missing_files``, ``proposals``, ``recall`` (the
@@ -17,7 +17,6 @@ import json
 import os
 import sys
 from concurrent.futures import ThreadPoolExecutor
-from pathlib import Path
 
 import numpy as np
 
@@ -123,7 +122,7 @@ def main(argv=None):
         _fail("%s does not exist or is not a folder" % args.folder)
     if args.every < 1 or args.batch_frames < 1:
         _fail("--every and --batch_frames must be at least 1")
-    from .extract_pseudo_labels import build_feed, load_config
+    from .extract_pseudo_labels import build_feed, frame_id, load_config
     from .quality import QualitySpec
     try:
         cfg = load_config(args.cfg_file, args.set_cfgs)
@@ -144,7 +143,7 @@ def main(argv=None):
     missing = []
 
     def load(i):
-        fid = Path(feed.infos[i]["lidar_path"]).stem
+        fid = frame_id(feed.infos[i])
         got = read_pseudos(pseudo_path(args.folder, fid))
         absent = got is None
         if absent:          # no proposals

@@ -6,12 +6,14 @@ is tools/extract_pseudo_labels.py of the reference with ``extract.extract_nuscen
 loop.  Run it from the directory the reference runs from (``tools/``): the config's relative paths
 (``_BASE_CONFIG_``, ``DATA_PATH``, the GLIP prediction files of ``PreprocessedGLIP``) are read as there.
 
-  * config: ``DATA_CONFIG.DATASET`` NuScenesDataset, ``MODEL.DENSE_HEAD.NAME`` FrustumProposerOG; the head's options
-    are read by ``proposer.FrustumProposerOG``; frames come from ``NuScenesFeed`` in the mode the reference tool runs
-    its loader in (training=True, augmentation list emptied, extract_pseudo_labels.py:47-58);
+  * config: ``DATA_CONFIG.DATASET`` NuScenesDataset with ``MODEL.DENSE_HEAD.NAME`` FrustumProposerOG, or KittiDataset
+    with FrustumProposerOGKITTI; the head's options are read by its own constructor (``proposer``); frames come from
+    ``NuScenesFeed`` / ``KittiFeed`` in the mode the reference tool runs its loader in (training=True, augmentation
+    list emptied, extract_pseudo_labels.py:47-58);
   * output: one ``.pth`` per frame in ``--folder``, which must not exist yet (:80-84);
   * failed frames: a frame whose LiDAR file, one of whose sweep files (MAX_SWEEPS > 1) or one of whose six camera
-    images is missing from the detector's predictions is skipped, logged and counted (``check_frame``);
+    images is missing from the detector's predictions is skipped, logged and counted (``check_frame``); for KITTI a
+    frame whose velodyne or calib file is missing, or whose ``<frame_id>.png`` is not in the predictions;
   * several GPUs: under torchrun (``WORLD_SIZE`` > 1) each process runs on ``cuda:LOCAL_RANK`` over NCCL and takes
     frames ``rank::world``; rank 0 prints.
 """
@@ -23,12 +25,15 @@ from pathlib import Path
 
 from .config import cfg_from_list, cfg_from_yaml_file
 
-DATASETS = ("NuScenesDataset",)
-HEADS = ("FrustumProposerOG",)
+# the dataset each supported head runs on
+PAIRS = {"NuScenesDataset": "FrustumProposerOG", "KittiDataset": "FrustumProposerOGKITTI"}
+DATASETS = tuple(PAIRS)
+HEADS = tuple(PAIRS.values())
 
-LIDAR_MISSING, SWEEP_MISSING, IMAGE_NOT_PREDICTED = 1, 2, 3
+LIDAR_MISSING, SWEEP_MISSING, IMAGE_NOT_PREDICTED, CALIB_MISSING = 1, 2, 3, 4
 FAILURES = {LIDAR_MISSING: "LiDAR file missing", SWEEP_MISSING: "sweep file missing",
-            IMAGE_NOT_PREDICTED: "camera image not in the detector's predictions"}
+            IMAGE_NOT_PREDICTED: "camera image not in the detector's predictions",
+            CALIB_MISSING: "calibration file missing"}
 
 
 def parse_args(argv=None):
@@ -54,17 +59,43 @@ def load_config(cfg_file, set_cfgs=None):
     if dataset not in DATASETS:
         raise ValueError("DATA_CONFIG.DATASET %r is not supported: this command reads %s" % (dataset, ", ".join(DATASETS)))
     head = cfg.get("MODEL", {}).get("DENSE_HEAD", {}).get("NAME")
-    if head not in HEADS:
-        raise ValueError("MODEL.DENSE_HEAD.NAME %r is not supported: this command runs %s on nuScenes"
-                         % (head, ", ".join(HEADS)))
+    if head != PAIRS[dataset]:
+        raise ValueError("DATA_CONFIG.DATASET %r with MODEL.DENSE_HEAD.NAME %r is not supported: this command reads %s, "
+                         "and runs %s" % (dataset, head, " and ".join(DATASETS),
+                                          ", ".join("%s on %s" % (h, d) for d, h in PAIRS.items())))
     return cfg
 
 
-def build_feed(cfg, infos=None):
-    """NuScenesFeed over ``DATA_PATH / VERSION`` (the NuScenesDataset rule) and ``INFO_PATH['train']`` (or ``infos``),
-    training=True; keys the config leaves out keep the feed's defaults."""
-    from .nuscenes_feed import NuScenesFeed
+def is_kitti(cfg) -> bool:
+    return cfg.DATA_CONFIG.DATASET == "KittiDataset"
+
+
+def build_head(cfg, device=None):
+    """The config's head, built by its own constructor from MODEL.DENSE_HEAD and CLASS_NAMES."""
+    from . import proposer
+    cls = proposer.FrustumProposerOGKITTI if is_kitti(cfg) else proposer.FrustumProposerOG
+    return cls(model_cfg=cfg.MODEL.DENSE_HEAD, class_names=cfg.get("CLASS_NAMES"), device=device)
+
+
+def frame_id(info: dict) -> str:
+    """The frame id of an info dict of either dataset (the name of its .pth file, before '.' -> '_')."""
+    return info["point_cloud"]["lidar_idx"] if "point_cloud" in info else Path(info["lidar_path"]).stem
+
+
+def build_feed(cfg, infos=None, device=None):
+    """NuScenesFeed over ``DATA_PATH / VERSION`` (the NuScenesDataset rule), or KittiFeed over ``DATA_PATH`` and
+    ``DATA_SPLIT['train']`` (``device``: where its frames' calibration blocks are formed), of ``INFO_PATH['train']``
+    (or ``infos``), training=True; keys the config leaves out keep the feed's defaults."""
     d = cfg.DATA_CONFIG
+    if is_kitti(cfg):
+        from .kitti_feed import KittiFeed
+        kw = {arg: d[key] for key, arg in (("POINT_CLOUD_RANGE", "point_cloud_range"),
+                                           ("FOV_POINTS_ONLY", "fov_points_only")) if key in d}
+        if "CLASS_NAMES" in cfg:
+            kw["class_names"] = cfg.CLASS_NAMES
+        return KittiFeed(d.DATA_PATH, d.INFO_PATH["train"] if infos is None else infos,
+                         split=d.get("DATA_SPLIT", {}).get("train", "train"), training=True, device=device, **kw)
+    from .nuscenes_feed import NuScenesFeed
     kw = {arg: d[key] for key, arg in (("MAX_SWEEPS", "max_sweeps"), ("POINT_CLOUD_RANGE", "point_cloud_range"),
                                        ("FILTER_MIN_POINTS_IN_GT", "filter_min_points_in_gt"),
                                        ("PRED_VELOCITY", "pred_velocity"),
@@ -83,7 +114,17 @@ def build_feed(cfg, infos=None):
 def check_frame(feed, detector, info) -> int:
     """0, or why the frame cannot run: its LiDAR file is missing; MAX_SWEEPS > 1 and a sweep file its info lists is
     missing (which sweeps the feed reads is drawn only at load time); one of its camera images is not in the
-    detector's predictions (not checked when ``detector`` is None)."""
+    detector's predictions (not checked when ``detector`` is None).  KITTI: its velodyne file or its calib file is
+    missing; ``<frame_id>.png`` is not in the detector's predictions."""
+    if "point_cloud" in info:
+        fid = frame_id(info)
+        if not feed.lidar_path(fid).is_file():
+            return LIDAR_MISSING
+        if not feed.calib_path(fid).is_file():
+            return CALIB_MISSING
+        if detector is not None and not detector.has_image(fid + ".png"):
+            return IMAGE_NOT_PREDICTED
+        return 0
     if not (feed.root / info["lidar_path"]).is_file():
         return LIDAR_MISSING
     if feed.max_sweeps > 1 and not all((feed.root / s["lidar_path"]).is_file() for s in info["sweeps"]):
@@ -128,7 +169,7 @@ def _run(args, rank, world, device):
     import numpy as np
     import torch
     import torch.distributed as dist
-    from . import extract, proposer
+    from . import extract
     log = print if rank == 0 else (lambda *a, **k: None)
     try:
         cfg = load_config(args.cfg_file, args.set_cfgs)
@@ -136,8 +177,8 @@ def _run(args, rank, world, device):
         if rank == 0:
             print(e.args[-1] if isinstance(e, KeyError) else e, file=sys.stderr)
         raise SystemExit(1)
-    head = proposer.FrustumProposerOG(model_cfg=cfg.MODEL.DENSE_HEAD, class_names=cfg.get("CLASS_NAMES"), device=device)
-    all_frames = build_feed(cfg)
+    head = build_head(cfg, device=device)
+    all_frames = build_feed(cfg, device=head.engine.device)
     n = len(all_frames)
     # each rank checks its own shard; the failure codes are then combined so that every rank runs the same frame list
     codes = np.zeros(n, np.int32)
@@ -147,10 +188,10 @@ def _run(args, rank, world, device):
         t = torch.from_numpy(codes).to(device)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         codes = t.cpu().numpy()
-    failed = [(Path(all_frames.infos[i]["lidar_path"]).stem, FAILURES[int(codes[i])]) for i in np.flatnonzero(codes)]
+    failed = [(frame_id(all_frames.infos[i]), FAILURES[int(codes[i])]) for i in np.flatnonzero(codes)]
     for fid, why in failed:
         log("skipped frame %s: %s" % (fid, why))
-    feed = build_feed(cfg, infos=[all_frames.infos[i] for i in np.flatnonzero(codes == 0)])
+    feed = build_feed(cfg, infos=[all_frames.infos[i] for i in np.flatnonzero(codes == 0)], device=head.engine.device)
     _, recall, ar = extract.extract_nuscenes(feed, head.image_detector, head.engine, folder=args.folder,
                                              batch_frames=args.batch_frames, rank=rank, world=world,
                                              nms_thresh=args.nms_thresh, workers=args.workers,

@@ -47,6 +47,22 @@ def head_params(model_cfg, defaults=None):
     return p
 
 
+def kitti_head_params(model_cfg, defaults=None):
+    """The parameters FrustumProposerOGKITTI runs with: ``defaults`` (the constructor's: DEFAULTS with max_dist 70 and
+    clamp_bottom 0 when None), overridden by ``model_cfg.PARAMS`` (frustum_proposals_v1_kitti.py:68-98); aln_w / ego_w /
+    occl_w are read there and never used, so they are 0 here."""
+    p = dict(DEFAULTS, max_dist=70, clamp_bottom=0) if defaults is None else dict(defaults)
+    params = _cfg_get(model_cfg, 'PARAMS')
+    if params is not None:
+        for k in list(DEFAULTS) + list(EXTRA_PARAMS):
+            if k in params:
+                p[k] = params[k]
+    if _cfg_get(model_cfg, 'SAVE_BLEND', False):
+        raise NotImplementedError("SAVE_BLEND (Blender visualisation dumps) is outside the Box Seeker path")
+    p['aln_w'] = p['ego_w'] = p['occl_w'] = 0
+    return p
+
+
 # ----------------------------------------------------------------------------- feeders
 class BoxList:
     """Unpickling shim for maskrcnn_benchmark.structures.bounding_box.BoxList (GLIP's
@@ -400,17 +416,10 @@ class FrustumProposerOGKITTI(nn.Module):
                  size_max=size_max, ry_min=ry_min, ry_max=float(ry_max), cq=cq, num_mags=num_mags, max_dist=max_dist,
                  num_sizes=num_sizes, num_rotations=num_rotations, topk=topk, nms_2d=nms_2d, nms_3d=nms_3d,
                  score_thr=score_thr, nms_normal=nms_normal, clamp_bottom=0)      # the argument is ignored (:62)
-        params = _cfg_get(model_cfg, 'PARAMS')
-        if params is not None:                       # PARAMS override the defaults (:68-98)
-            for k in list(DEFAULTS) + ['aln_w', 'ego_w', 'occl_w', 'rand_center', 'search_depth']:
-                if k in params:
-                    p[k] = params[k]
-        if _cfg_get(model_cfg, 'SAVE_BLEND', False):
-            raise NotImplementedError("SAVE_BLEND (Blender visualisation dumps) is outside the Box Seeker path")
-        assert p['nms_3d'] == 0, 'DO NOT USE!'          # the reference's own assertion (:114)
         # aln_w / ego_w / occl_w and the MULT / OCCL_MULT / MULTICAM_IOU switches are read by that constructor and never
         # used by its get_proposals: ignored here as there
-        p['aln_w'] = p['ego_w'] = p['occl_w'] = 0
+        p = kitti_head_params(model_cfg, p)
+        assert p['nms_3d'] == 0, 'DO NOT USE!'          # the reference's own assertion (:114)
         self.params = p
         self.image_size = [900, 1600]
         self.topk, self.score_thr, self.max_dist = p['topk'], p['score_thr'], p['max_dist']

@@ -52,6 +52,8 @@ FLAG_KEYS = ("MULT", "OCCL_MULT", "MULTICAM_IOU")     # MODEL.DENSE_HEAD switche
 # the parameters only stage 3 reads (with min_cam_iou, which only removes hypotheses): settings that differ in these
 # alone share stages 1-2c (SeekerEngine.evaluate_settings, fnp_seeker_select_multi)
 SELECT_KEYS = ("dns_w", "iou_w", "dst_w", "ego_w", "occl_w", "min_cam_iou", "MULT", "OCCL_MULT")
+# the KITTI head's: its counts are first-match counts over the valid set, which min_cam_iou changes
+SELECT_KEYS_KITTI = ("dns_w", "iou_w", "dst_w")
 
 
 def resolve_params(params: Optional[dict], variant: str = "nuscenes") -> dict:
@@ -817,19 +819,24 @@ class SeekerEngine:
         stage 3 once per setting (fnp_seeker_select_multi), and its recall and precision counters.  settings: dicts of
         SELECT_KEYS (a key a setting leaves out takes this engine's value), any number of them: stage 3 runs for up to
         256 settings per launch; each min_cam_iou must be at least this engine's, whose compaction every setting
-        filters further.  plan / points_dev / gt as for execute (gt from
+        filters further -- for the KITTI variant each must equal this engine's, and a setting holds SELECT_KEYS_KITTI
+        (first-match counts depend on the valid set).  plan / points_dev / gt as for execute (gt from
         upload_gt).  Returns finish()'s dict, whose "settings" holds per setting: proposals, recall (recall_dict),
         precision (proposals, then "hits_<t>": proposals with a GT IoU3D > t), and per candidate cand_best (index among
         the compacted hypotheses, -1: none), cand_score2, cand_count, cand_boxes.  quality (a quality.QualitySpec): one
         more launch, fnp_quality_counters over every setting, and each setting gains "quality", its flat counters
         (quality.tables reads them).  One D2H; on a page-pool overflow the pool grows and the batch runs again."""
-        if self.T != 1 or self.variant != "nuscenes" or self.rand_center:
-            raise NotImplementedError("evaluate_settings runs the nuScenes head with topk = 1 and no rand_center")
+        if self.T != 1 or self.rand_center:
+            raise NotImplementedError("evaluate_settings runs with topk = 1 and no rand_center")
         if not settings:
             raise ValueError("evaluate_settings needs at least one setting")
         for s in settings:
-            if np.float32(s.get("min_cam_iou", self.p["min_cam_iou"])) < np.float32(self.p["min_cam_iou"]):
+            iou = np.float32(s.get("min_cam_iou", self.p["min_cam_iou"]))
+            if iou < np.float32(self.p["min_cam_iou"]):
                 raise ValueError("setting %r: min_cam_iou below the engine's %s" % (s, self.p["min_cam_iou"]))
+            if self.variant == "kitti" and iou != np.float32(self.p["min_cam_iou"]):
+                raise ValueError("setting %r: the KITTI head's min_cam_iou must be the engine's %s (its first-match "
+                                 "counts depend on the valid set)" % (s, self.p["min_cam_iou"]))
         if quality is not None:
             from .quality import check_labels
             check_labels(quality, plan["cand_label"], gt[0].cpu().numpy(), gt[1].cpu().numpy())

@@ -349,12 +349,19 @@ def write_glip_predictions(frames, pred_pth, meta_coco):
         json.dump(dict(images=images, categories=[dict(id=i + 1, name=n) for i, n in enumerate(CLASS_NAMES)]), fh)
 
 
-def make_kitti_frame(index):
+# class names of the synthetic KITTI tree (write_kitti_tree), one per anchor of the KITTI head, in label order
+KITTI_CLASS_NAMES = ['Car', 'Truck', 'Van', 'Tram', 'Pedestrian', 'Cyclist', 'Person_sitting']
+KITTI_IMAGE_SHAPE = (375, 1242)
+
+
+def make_kitti_frame(index, with_gt=False, cfg=None, full_scan=False):
     """A KITTI-shaped frame: points in front of the sensor, P2 / R0 / Tr_velo2cam, x-y-w-h 2D boxes of the visible
-    synthetic objects, labels 1..7 (the KITTI head's seven anchors)."""
-    cfg = SynthConfig("kitti", 32, 900, 1, 12, 4, 6, 1)
+    synthetic objects, labels 1..7 (the KITTI head's seven anchors).  with_gt: also the frame's (G,10) LiDAR-frame GT
+    (make_frame's).  cfg: the scan (default 32 beams x 900 azimuths); full_scan: every point of the scan, not only
+    those in front of the sensor (what a velodyne file holds before the FOV filter)."""
+    cfg = cfg or SynthConfig("kitti", 32, 900, 1, 12, 4, 6, 1)
     f = make_frame(index, cfg)
-    pts = f.points[f.points[:, 0] > 1.0][:, :4].copy()
+    pts = (f.points if full_scan else f.points[f.points[:, 0] > 1.0])[:, :4].copy()
     V2C = np.array([[0.0, -1.0, 0.0, 0.004], [0.0, 0.0, -1.0, -0.076], [1.0, 0.0, 0.0, -0.272]], np.float32)
     a = 0.01
     R0 = np.array([[np.cos(a), -np.sin(a), 0], [np.sin(a), np.cos(a), 0], [0, 0, 1]], np.float32)
@@ -375,5 +382,52 @@ def make_kitti_frame(index):
         boxes.append([x1, y1, x2 - x1, y2 - y1])
         labels.append(1 + int(rng.integers(0, 7)))
         scores.append(float(rng.uniform(0.5, 0.9)))
-    return (pts, {'P2': P2, 'R0': R0, 'Tr_velo2cam': V2C}, np.asarray(boxes, np.float32).reshape(-1, 4),
-            np.asarray(labels, np.int64), np.asarray(scores, np.float32))
+    out = (pts, {'P2': P2, 'R0': R0, 'Tr_velo2cam': V2C}, np.asarray(boxes, np.float32).reshape(-1, 4),
+           np.asarray(labels, np.int64), np.asarray(scores, np.float32))
+    return out + (f.gt_boxes,) if with_gt else out
+
+
+def write_kitti_tree(root, frames, class_names=KITTI_CLASS_NAMES, coco_path=None):
+    """Write make_kitti_frame(i, with_gt=True) frames as an OpenPCDet KITTI tree under ``root`` (DATA_PATH), frame k
+    with id ``%06d % k``: ``training/velodyne/<id>.bin`` (float32 x, y, z, intensity), ``training/calib/<id>.txt``
+    (P0..P3, R0_rect, Tr_velo_to_cam, Tr_imu_to_velo), ``kitti_infos_train.pkl`` (point_cloud.lidar_idx,
+    image.image_shape, annos with name / dimensions (l, h, w) / location / rotation_y in the rectified camera frame:
+    every GT box, out of range ones included, plus one DontCare row per frame) and, at ``coco_path`` (default
+    ``root/kitti_coco_results.json``), the COCO result file of the 2D boxes that proposer.PreprocessedDetector reads
+    (images ``<id>.png``, category k + 1 = class_names[k]).  Returns the info dicts."""
+    import json
+    import os
+    import pickle
+    split = os.path.join(str(root), "training")
+    for sub in ("velodyne", "calib"):
+        os.makedirs(os.path.join(split, sub), exist_ok=True)
+    infos, images, anns = [], [], []
+    for k, (pts, cal, boxes, labels, scores, gt) in enumerate(frames):
+        idx = "%06d" % k
+        np.ascontiguousarray(pts, np.float32).tofile(os.path.join(split, "velodyne", idx + ".bin"))
+        P2, R0, V2C = (np.asarray(cal[n], np.float32) for n in ("P2", "R0", "Tr_velo2cam"))
+        rows = [("P0", P2), ("P1", P2), ("P2", P2), ("P3", P2), ("R0_rect", R0), ("Tr_velo_to_cam", V2C),
+                ("Tr_imu_to_velo", V2C)]
+        with open(os.path.join(split, "calib", idx + ".txt"), "w") as fh:
+            fh.write("".join("%s: %s\n" % (n, " ".join(repr(float(v)) for v in m.reshape(-1))) for n, m in rows))
+        g = np.asarray(gt, np.float64)
+        bottom = np.c_[g[:, 0:2], g[:, 2] - g[:, 5] / 2, np.ones(len(g))]
+        loc = (bottom @ np.vstack([V2C, [0, 0, 0, 1]]).astype(np.float64).T)[:, :3] @ R0.astype(np.float64).T
+        names = [class_names[(int(c) - 1) % len(class_names)] for c in g[:, 9]] + ["DontCare"]
+        annos = dict(name=np.array(names),
+                     dimensions=np.r_[g[:, [3, 5, 4]], [[-1.0, -1.0, -1.0]]].astype(np.float32),
+                     location=np.r_[loc, [[-1000.0, -1000.0, -1000.0]]].astype(np.float32),
+                     rotation_y=np.r_[-g[:, 6] - np.pi / 2, [-10.0]].astype(np.float32))
+        infos.append(dict(point_cloud=dict(num_features=4, lidar_idx=idx),
+                          image=dict(image_idx=idx, image_shape=np.array(KITTI_IMAGE_SHAPE, np.int32)),
+                          calib=dict(P2=P2, R0_rect=R0, Tr_velo_to_cam=V2C), annos=annos))
+        images.append(dict(id=k, file_name=idx + ".png"))
+        for b, lab, sc in zip(boxes, labels, scores):
+            anns.append(dict(id=len(anns), image_id=k, category_id=int(lab), score=float(sc),
+                             bbox=[float(v) for v in b]))
+    with open(os.path.join(str(root), "kitti_infos_train.pkl"), "wb") as fh:
+        pickle.dump(infos, fh)
+    with open(coco_path or os.path.join(str(root), "kitti_coco_results.json"), "w") as fh:
+        json.dump(dict(images=images, annotations=anns,
+                       categories=[dict(id=i + 1, name=n) for i, n in enumerate(class_names)]), fh)
+    return infos

@@ -8,6 +8,11 @@ frame is read and uploaded once.  Settings that differ only in the select-level 
 score weights, ``min_cam_iou``, ``MULT``, ``OCCL_MULT``) form one group and share stages 1-2c of the seeker; only
 stage 3 and the counters run per setting (SeekerEngine.evaluate_settings).  Every other parameter splits groups.
 
+A KITTI config (KittiDataset, FrustumProposerOGKITTI) is tuned the same way, with that head's rule: its counts are
+first-match counts over the valid set, so ``min_cam_iou`` splits groups and only ``dns_w``, ``iou_w`` and ``dst_w``
+(seeker.SELECT_KEYS_KITTI) share stages 1-2c; the keys that head does not read (``ego_w``, ``occl_w``, ``MULT``,
+``OCCL_MULT``, ``MULTICAM_IOU``) are refused, and ``topk`` stays 1.
+
 For each setting the command prints one JSON line -- its values and group, the proposals, the recall counters, AR and
 precision at 0.3 / 0.5 / 0.7 -- sorted by AR@0.5, then the ``--set`` arguments that give the best setting to
 ``extract_pseudo_labels``.  The config, its refusals and the failed-frame rule are those of ``extract_pseudo_labels``.
@@ -22,7 +27,7 @@ import sys
 import yaml
 
 from .config import cfg_from_list
-from .extract_pseudo_labels import build_feed, check_frame, load_config, FAILURES
+from .extract_pseudo_labels import build_feed, build_head, check_frame, frame_id, is_kitti, load_config, FAILURES
 
 HEAD = ("MODEL", "DENSE_HEAD")
 
@@ -91,19 +96,24 @@ def expand_grid(axes):
     return [dict(zip(keys, vals)) for vals in itertools.product(*[a[3] for a in axes])]
 
 
-def group_settings(base_params, settings):
-    """Groups of settings that can share stages 1-2c.  base_params: the head's parameters (proposer.head_params);
-    settings: dicts of parameter overrides.  Each setting is checked by seeker.resolve_params; topk > 1, rand_center
-    and aln_w are refused (ValueError naming the setting).  Settings are grouped on every resolved parameter except
-    seeker.SELECT_KEYS.  Returns a list of dict(params, members): members are indices into settings, params the
-    engine parameters of the group -- its first member's, at the group's loosest min_cam_iou."""
-    from .seeker import SELECT_KEYS, resolve_params
+def group_settings(base_params, settings, variant="nuscenes"):
+    """Groups of settings that can share stages 1-2c.  base_params: the head's parameters (proposer.head_params, or
+    proposer.kitti_head_params for variant "kitti"); settings: dicts of parameter overrides.  Each setting is checked by
+    seeker.resolve_params; topk > 1, rand_center and aln_w are refused, and for the KITTI head the keys it does not
+    read (ValueError naming the setting).  Settings are grouped on every resolved parameter except seeker.SELECT_KEYS
+    (seeker.SELECT_KEYS_KITTI for the KITTI head).  Returns a list of dict(params, members): members are indices into
+    settings, params the engine parameters of the group -- its first member's, at the group's loosest min_cam_iou."""
+    from .seeker import FLAG_KEYS, SELECT_KEYS, SELECT_KEYS_KITTI, resolve_params
+    kitti = variant == "kitti"
     resolved = []
     for s in settings:
+        unused = [k for k in ("ego_w", "occl_w") + FLAG_KEYS if k in s] if kitti else []
+        if unused:
+            raise ValueError("setting %s: %s not read by the KITTI head" % (s, ", ".join(unused)))
         p = dict(base_params)
         p.update(s)
         try:
-            r = resolve_params(p)
+            r = resolve_params(p, variant)
         except NotImplementedError as e:
             raise ValueError("setting %s: %s" % (s, e)) from None
         if int(r["topk"]) > 1:
@@ -111,9 +121,10 @@ def group_settings(base_params, settings):
         if r.get("rand_center"):
             raise ValueError("setting %s: rand_center is not supported by the tuner (the centres are random)" % (s,))
         resolved.append(r)
+    select = SELECT_KEYS_KITTI if kitti else SELECT_KEYS
     groups = {}
     for i, r in enumerate(resolved):
-        key = tuple(sorted((k, repr(v)) for k, v in r.items() if k not in SELECT_KEYS))
+        key = tuple(sorted((k, repr(v)) for k, v in r.items() if k not in select))
         groups.setdefault(key, []).append(i)
     out = []
     for members in groups.values():
@@ -124,17 +135,17 @@ def group_settings(base_params, settings):
 
 
 def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, workers=4, box_format="xyxy", device=None,
-                  quality=None):
-    """Scores every setting over every frame of ``feed``: each batch is read once (NuScenesFeed.prefetch) and uploaded
-    once, then every group of ``group_settings`` runs on it.  Returns (per setting dict(proposals, recall, precision)
+                  quality=None, variant="nuscenes"):
+    """Scores every setting over every frame of ``feed``: each batch is read once (NuScenesFeed / KittiFeed.prefetch)
+    and uploaded once, then every group of ``group_settings`` runs on it (variant: the head's, as for SeekerEngine).  Returns (per setting dict(proposals, recall, precision)
     summed over the frames, groups).  quality (a quality.QualitySpec): each setting's dict also holds "quality", its
     summed fnp_quality_counters counters."""
     import numpy as np
     import torch
     from .extract import THRESH, recall_keys
     from .seeker import SeekerEngine
-    groups = group_settings(base_params, settings)
-    engines = [SeekerEngine(g["params"], device=device, box_format=box_format) for g in groups]
+    groups = group_settings(base_params, settings, variant)
+    engines = [SeekerEngine(g["params"], device=device, box_format=box_format, variant=variant) for g in groups]
     # the groups run one after another and evaluate_settings waits for its results: one scratch arena serves them all,
     # so device memory does not grow with the number of groups
     for e in engines[1:]:
@@ -194,37 +205,41 @@ def main(argv=None):
         _fail("tune_params runs in one process: start it without torchrun")
     if args.every < 1:
         _fail("--every must be at least 1")
-    from .proposer import head_params
+    from .proposer import head_params, kitti_head_params
     try:
         cfg = load_config(args.cfg_file, args.set_cfgs)
         axes = load_grid(args.grid, cfg)
         grid = expand_grid(axes)
         names = {key: name for key, name, _, _ in axes}
         settings = [{names[k]: v for k, v in s.items()} for s in grid]
-        base = head_params(cfg.MODEL.DENSE_HEAD)
-        groups = group_settings(base, settings)
+        kitti = is_kitti(cfg)
+        variant = "kitti" if kitti else "nuscenes"
+        base = (kitti_head_params if kitti else head_params)(cfg.MODEL.DENSE_HEAD)
+        groups = group_settings(base, settings, variant)
         spec = None
         if args.breakdown:
+            from .kitti_feed import CLASS_NAMES as KITTI_CLASS_NAMES
             from .nuscenes_feed import CLASS_NAMES
             from .quality import QualitySpec
-            spec = QualitySpec(cfg.get("CLASS_NAMES") or CLASS_NAMES, range_edges=args.range_edges)
+            spec = QualitySpec(cfg.get("CLASS_NAMES") or (KITTI_CLASS_NAMES if kitti else CLASS_NAMES),
+                               range_edges=args.range_edges)
     except (OSError, KeyError, ValueError, NotImplementedError) as e:
         _fail(e.args[-1] if isinstance(e, KeyError) else e)
     print("%d settings in %d groups" % (len(settings), len(groups)))
-    from . import extract, proposer
-    head = proposer.FrustumProposerOG(model_cfg=cfg.MODEL.DENSE_HEAD, class_names=cfg.get("CLASS_NAMES"))
-    all_frames = build_feed(cfg)
+    from . import extract
+    head = build_head(cfg)
+    device = head.engine.device
+    all_frames = build_feed(cfg, device=device)
     picked = list(range(0, len(all_frames), args.every))
     codes = [check_frame(all_frames, head.image_detector, all_frames.infos[i]) for i in picked]
     for i, c in zip(picked, codes):
         if c:
-            print("skipped frame %s: %s" % (os.path.splitext(os.path.basename(all_frames.infos[i]["lidar_path"]))[0],
-                                            FAILURES[c]))
-    feed = build_feed(cfg, infos=[all_frames.infos[i] for i, c in zip(picked, codes) if c == 0])
+            print("skipped frame %s: %s" % (frame_id(all_frames.infos[i]), FAILURES[c]))
+    feed = build_feed(cfg, infos=[all_frames.infos[i] for i, c in zip(picked, codes) if c == 0], device=device)
     print("frames scored: %d, failed frames: %d" % (len(feed), sum(1 for c in codes if c)))
     totals, groups = evaluate_grid(feed, head.image_detector, base, settings, batch_frames=args.batch_frames,
-                                   workers=args.workers, box_format=head.box_fmt, device=head.engine.device,
-                                   quality=spec)
+                                   workers=args.workers, box_format=head.engine.box_format, device=device,
+                                   quality=spec, variant=variant)
     group_of = {i: gi for gi, g in enumerate(groups) for i in g["members"]}
     lines = []
     for i, (s, t) in enumerate(zip(grid, totals)):

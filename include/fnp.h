@@ -332,12 +332,19 @@ int fnp_seeker_run(const fnp_seeker_cfg *cfg, const fnp_seeker_batch *b, void *s
  * of the 32 KB parameter space; the library allocates nothing).  Each CTA stages a frustum's counts and IoUs, plus
  * the distance, occlusion and centre-norm planes when some setting reads them: 4 H bytes per plane, at most 200 KB
  * (6-15 KB at H = 768).  A caller with more settings makes one call per 256 over the same stages 1-2c.
- * Build record (nvcc 12.9, -Xptxas -v, sm_100a): select_multi_kernel 256 threads, 48 registers, 8-byte stack frame,
- * 4 bytes of spill stores / loads, no static shared memory.
- * FNP_EINVAL: cfg->topk > 1; the KITTI variant (its first-match counts depend on the valid set); a flag other than
+ * FNP_VARIANT_KITTI: that head's counts are first-match counts over the valid set, so they hold for a setting only
+ * when its valid set is the one stages 1-2c compacted: every setting must have cfg->min_cam_iou, bit for bit, no
+ * flags and no ego_w / occl_w (not terms of that score).  The count normaliser is then the SUM of the frustum's
+ * compacted counts + 1e-8, the distance plane is always staged, and the score is that head's additive one
+ * (dns_w + density + iou_w iou + dst_w dist), as fnp_seeker_select forms it for a KITTI cfg.
+ * Build record (nvcc 12.9, -Xptxas -v, sm_100a), 256 threads, no static shared memory: select_multi_kernel<false>
+ * (nuScenes) 48 registers, 8-byte stack frame, 4 bytes of spill stores / loads, 2672 SASS instructions;
+ * select_multi_kernel<true> (KITTI) 40 registers, no stack, no spills, 1760 SASS instructions.
+ * FNP_EINVAL: cfg->topk > 1; a KITTI setting outside the rule above; a flag other than
  * FNP_SEEKER_MULT / FNP_SEEKER_OCCL_MULT; a setting's min_cam_iou below cfg->min_cam_iou (the compaction was done
- * at cfg's threshold); a setting that needs hyp_dist (dst_w != 0, MULT) or hyp_nfar (occl_w > 0, OCCL_MULT) on a
- * batch without it -- hyp_nfar is formed by fnp_seeker_occlusion, which runs only when cfg itself turns occlusion on. */
+ * at cfg's threshold); a setting that needs hyp_dist (dst_w != 0, MULT, the KITTI variant) or hyp_nfar (occl_w > 0,
+ * OCCL_MULT) on a batch without it -- hyp_nfar is formed by fnp_seeker_occlusion, which runs only when cfg itself turns
+ * occlusion on. */
 #define FNP_SELECT_MAX_SETTINGS 256
 typedef struct fnp_select_setting {
     float dns_w, iou_w, dst_w, ego_w, occl_w, min_cam_iou;
