@@ -95,6 +95,11 @@ lib.fnp_crop_points_in_boxes.restype = _i
 lib.fnp_crop_points_in_boxes.argtypes = [_vp, _i, _vp, C.c_longlong, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp,
                                          C.c_size_t, _vp]
 lib.fnp_crop_workspace_bytes.restype = C.c_size_t
+lib.fnp_crop_all_count.restype = _i
+lib.fnp_crop_all_count.argtypes = [_vp, _i, _vp, C.c_longlong, _vp, _vp, _i, _i, _vp, _vp, _vp, C.c_size_t, _vp]
+lib.fnp_crop_all_scatter.restype = _i
+lib.fnp_crop_all_scatter.argtypes = [_vp, _i, _vp, C.c_longlong, _vp, _vp, _vp, _i, _i, _vp, _vp, C.c_longlong, _vp,
+                                     C.c_size_t, _vp]
 lib.fnp_crop_workspace_bytes.argtypes = [_vp, _vp, _i]
 for _n in ("fnp_boxes_overlap_bev", "fnp_boxes_iou_bev"):
     getattr(lib, _n).restype = _i
@@ -167,6 +172,7 @@ lib.fnp_dbg_math.argtypes = [_vp, _vp, _vp, _i, _vp]
 EXPORTED = [
     "fnp_dbg_math", "fnp_upload_from_pinned",
     "fnp_version", "fnp_points_in_boxes", "fnp_count_in_boxes", "fnp_crop_points_in_boxes", "fnp_crop_workspace_bytes",
+    "fnp_crop_all_count", "fnp_crop_all_scatter",
     "fnp_boxes_overlap_bev",
     "fnp_boxes_iou_bev", "fnp_boxes_aligned_overlap_bev", "fnp_nms_workspace_bytes", "fnp_nms_rotated",
     "fnp_nms_normal", "fnp_seeker_cull", "fnp_seeker_frustum_stats", "fnp_seeker_hypotheses",

@@ -64,8 +64,9 @@ def _load_boxes(args, feed, frames, n_classes, pool):
     """Per frame of ``frames`` (info indices): (boxes (K,8) [box7, label], scores (K,)) as load_pseudos returns them,
     or None for a missing file.  Exits for a label outside the classes or a frame too large for the NMS."""
     from ._lib import SEG_NMS_MAX
+    from .extract_pseudo_labels import frame_id
     from .pseudo_loader import pseudo_path, read_pseudos, seg_nms_keep
-    ids = [Path(feed.infos[i]["lidar_path"]).stem for i in frames]
+    ids = [frame_id(feed.infos[i]) for i in frames]
     got = list(pool.map(lambda fid: read_pseudos(pseudo_path(args.folder, fid)), ids))
     out = []
     for fid, g in zip(ids, got):

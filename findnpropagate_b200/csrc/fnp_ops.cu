@@ -93,6 +93,17 @@ __global__ void __launch_bounds__(kCntThreads) count_segments_kernel(const float
 constexpr int kMatThreads = 256;
 constexpr int kMatBoxes = 16;     // boxes per CTA (rows of the output a CTA writes)
 
+// The CPU op's test of one point against one prepared box (q: the 8 floats of box_prep), every product rounded.
+// pib_matrix_kernel and the every-box crop both call it, so the two give the same bits.
+__device__ __forceinline__ bool in_box_cpu(float x, float y, float z, const float *q)
+{
+    const float sz = __fsub_rn(z, q[2]);
+    const float sx = __fsub_rn(x, q[0]), sy = __fsub_rn(y, q[1]);
+    const float lx = __fadd_rn(__fmul_rn(sx, q[4]), __fmul_rn(sy, -q[5]));
+    const float ly = __fadd_rn(__fmul_rn(sx, q[5]), __fmul_rn(sy, q[4]));
+    return !(fabsf(sz) > q[3]) && (fabsf(lx) <= q[6]) && (fabsf(ly) <= q[7]);
+}
+
 __global__ void __launch_bounds__(kMatThreads) pib_matrix_kernel(const float *__restrict__ prep, const float *__restrict__ pts,
                                                                  int32_t *__restrict__ out, int N, int P)
 {
@@ -104,15 +115,8 @@ __global__ void __launch_bounds__(kMatThreads) pib_matrix_kernel(const float *__
     const int j = blockIdx.x * kMatThreads + threadIdx.x;
     if (j >= P) return;
     const float x = pts[(size_t)j * 3], y = pts[(size_t)j * 3 + 1], z = pts[(size_t)j * 3 + 2];
-    for (int k = 0; k < nb; k++) {
-        const float *q = s_box[k];
-        const float sz = __fsub_rn(z, q[2]);
-        const float sx = __fsub_rn(x, q[0]), sy = __fsub_rn(y, q[1]);
-        const float lx = __fadd_rn(__fmul_rn(sx, q[4]), __fmul_rn(sy, -q[5]));
-        const float ly = __fadd_rn(__fmul_rn(sx, q[5]), __fmul_rn(sy, q[4]));
-        const bool in = !(fabsf(sz) > q[3]) && (fabsf(lx) <= q[6]) && (fabsf(ly) <= q[7]);
-        out[(size_t)(n0 + k) * P + j] = in ? 1 : 0;      // coalesced along the points
-    }
+    for (int k = 0; k < nb; k++)
+        out[(size_t)(n0 + k) * P + j] = in_box_cpu(x, y, z, s_box[k]) ? 1 : 0;      // coalesced along the points
 }
 
 // ======================================================================================
@@ -1006,6 +1010,121 @@ __global__ void __launch_bounds__(32) crop_scatter_kernel(const float *__restric
     }
 }
 
+// --------------------------------------------------------------------------------------
+// Every-box crop (points_in_boxes_cpu + points[mask[i] > 0], KittiDataset.create_groundtruth_database): a point is
+// written once for every box of its frame that contains it, by in_box_cpu on fnp_host_prep_boxes_cpu's constants.
+// The plan, the per-(tile, box) matrix, crop_prefix_kernel and crop_starts_kernel are the first-match crop's; only
+// the count and the scatter differ.  crop_all_count_kernel writes each (tile, box) count, summed from warp ballots
+// (no atomic); crop_all_scatter_kernel gives each box of a tile to one warp, which walks the tile's points in row
+// order and ranks the ones in the box with a ballot.
+// --------------------------------------------------------------------------------------
+constexpr int kCropWarps = kCropThreads / 32;
+
+__global__ void __launch_bounds__(kCropThreads) crop_all_count_kernel(const float *__restrict__ pts, int n_cols,
+                                                                      const int64_t *__restrict__ row_start,
+                                                                      const float *__restrict__ box_prep,
+                                                                      const int64_t *__restrict__ box_start,
+                                                                      int n_frames, CropWs ws)
+{
+    __shared__ float s_box[kCropThreads][8];
+    __shared__ int s_cnt[kCropWarps][kCropThreads];
+    int f, n;
+    long long r0;
+    if (!crop_tile(row_start, box_start, n_frames, ws, blockIdx.x, f, r0, n)) return;
+    const long long b0 = box_start[f];
+    const int T = (int)(box_start[f + 1] - b0);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    float x[kCropPerThread], y[kCropPerThread], z[kCropPerThread];
+#pragma unroll
+    for (int j = 0; j < kCropPerThread; j++) {
+        const int i = j * kCropThreads + threadIdx.x;
+        x[j] = y[j] = z[j] = 0.f;
+        if (i < n) {
+            const float *p = pts + (size_t)(r0 + i) * n_cols;
+            x[j] = p[0]; y[j] = p[1]; z[j] = p[2];
+        }
+    }
+    int32_t *row = ws.mat + ws.mat_start[f] + (blockIdx.x - ws.tile_start[f]) * (long long)T;
+    for (int t0 = 0; t0 < T; t0 += kCropThreads) {
+        const int nt = min(kCropThreads, T - t0);
+        __syncthreads();
+        if ((int)threadIdx.x < nt)
+#pragma unroll
+            for (int c = 0; c < 8; c++) s_box[threadIdx.x][c] = box_prep[(size_t)(b0 + t0 + threadIdx.x) * 8 + c];
+        __syncthreads();
+        for (int k = 0; k < nt; k++) {
+            int c = 0;
+#pragma unroll
+            for (int j = 0; j < kCropPerThread; j++) {
+                const bool in = j * kCropThreads + (int)threadIdx.x < n && in_box_cpu(x[j], y[j], z[j], s_box[k]);
+                c += __popc(__ballot_sync(0xffffffffu, in));
+            }
+            if (lane == 0) s_cnt[warp][k] = c;
+        }
+        __syncthreads();
+        if ((int)threadIdx.x < nt) {
+            int c = 0;
+#pragma unroll
+            for (int w = 0; w < kCropWarps; w++) c += s_cnt[w][threadIdx.x];
+            row[t0 + threadIdx.x] = c;
+        }
+    }
+}
+
+// After crop_prefix_kernel the tile's matrix row holds each box's offset within the box, and the next tile's row (or
+// the box's count, for the last tile) where this tile's points of the box end.  A warp stops a box once it has
+// written them all, skips a box with none in the tile, and never writes at or past rows_cap.
+__global__ void __launch_bounds__(kCropThreads) crop_all_scatter_kernel(const float *__restrict__ pts, int n_cols,
+                                                                        const int64_t *__restrict__ row_start,
+                                                                        const float *__restrict__ box_prep,
+                                                                        const double *__restrict__ centres,
+                                                                        const int64_t *__restrict__ box_start,
+                                                                        int n_frames, CropWs ws,
+                                                                        const int64_t *__restrict__ starts,
+                                                                        float *__restrict__ rows, long long rows_cap)
+{
+    __shared__ float s_xyz[3][kCropTile];
+    int f, n;
+    long long r0;
+    if (!crop_tile(row_start, box_start, n_frames, ws, blockIdx.x, f, r0, n)) return;
+    const long long b0 = box_start[f];
+    const int T = (int)(box_start[f + 1] - b0);
+    if (T == 0) return;
+    for (int i = threadIdx.x; i < n; i += kCropThreads) {
+        const float *p = pts + (size_t)(r0 + i) * n_cols;
+        s_xyz[0][i] = p[0]; s_xyz[1][i] = p[1]; s_xyz[2][i] = p[2];
+    }
+    __syncthreads();
+    const unsigned lane = threadIdx.x & 31;
+    const long long t = blockIdx.x - ws.tile_start[f], tiles = ws.tile_start[f + 1] - ws.tile_start[f];
+    const int32_t *off = ws.mat + ws.mat_start[f] + t * T;
+    for (int k = threadIdx.x >> 5; k < T; k += kCropWarps) {
+        const long long g = b0 + k;
+        const long long end = t + 1 < tiles ? (long long)off[k + T] : starts[g + 1] - starts[g];
+        long long left = end - off[k];
+        if (left <= 0) continue;
+        float q[8];
+#pragma unroll
+        for (int c = 0; c < 8; c++) q[c] = box_prep[(size_t)g * 8 + c];
+        long long out = starts[g] + off[k];
+        for (int i0 = 0; i0 < n && left > 0; i0 += 32) {
+            const int i = i0 + (int)lane;
+            const bool in = i < n && in_box_cpu(s_xyz[0][i], s_xyz[1][i], s_xyz[2][i], q);
+            const unsigned m = __ballot_sync(0xffffffffu, in);
+            const long long r = out + __popc(m & ((1u << lane) - 1u));
+            if (in && r >= 0 && r < rows_cap) {
+                const float *p = pts + (size_t)(r0 + i) * n_cols;
+                float *o = rows + (size_t)r * n_cols;
+#pragma unroll
+                for (int c = 0; c < 3; c++) o[c] = __double2float_rn(__dsub_rn((double)p[c], centres[g * 3 + c]));
+                for (int c = 3; c < n_cols; c++) o[c] = p[c];
+            }
+            out += __popc(m);
+            left -= __popc(m);
+        }
+    }
+}
+
 // test hook: the device math routines exactly as this library's kernels see them
 __global__ void dbg_math_kernel(const float *__restrict__ x, const float *__restrict__ y, float *__restrict__ out, int n)
 {
@@ -1073,21 +1192,10 @@ extern "C" size_t fnp_crop_workspace_bytes(const int64_t *row_start_host, const 
     return crop_head_bytes(n_frames ? row_start_host[n_frames] : 0, n_frames) + mat * 4 + 16;
 }
 
-extern "C" int fnp_crop_points_in_boxes(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
-                                        const float *boxes, const double *centres, const int64_t *box_start,
-                                        int n_boxes, int n_frames, int32_t *counts, int64_t *starts, float *rows,
-                                        void *workspace, size_t workspace_bytes, void *stream)
+// The workspace as fnp_crop_workspace_bytes sizes it (the caller has checked it holds the head).
+static CropWs crop_carve(void *workspace, size_t workspace_bytes, long long n_points, int n_boxes, int n_frames)
 {
-    if (n_cols < 3 || n_points < 0 || n_boxes < 0 || n_frames < 0 || n_frames > 65535 * 1024) return FNP_EINVAL;
-    if (n_frames == 0 && (n_points || n_boxes)) return FNP_EINVAL;
-    if (!row_start || !box_start || !starts || !workspace || (n_points && !pts) || (n_boxes && (!boxes || !centres || !counts)) ||
-        (n_points && n_boxes && !rows) || (reinterpret_cast<uintptr_t>(workspace) & 15))
-        return FNP_EINVAL;
-    const long long n_tiles = n_points / kCropTile + n_frames;
-    if (n_tiles > 0x7fffffffLL || divup(n_boxes, 128) > 0x7fffffff) return FNP_EINVAL;
     const size_t head = crop_head_bytes(n_points, n_frames);
-    if (workspace_bytes < head + 16) return FNP_EWORKSPACE;
-    cudaStream_t s = (cudaStream_t)stream;
     char *w = static_cast<char *>(workspace);
     CropWs ws;
     ws.mat_start = reinterpret_cast<int64_t *>(w);
@@ -1097,6 +1205,83 @@ extern "C" int fnp_crop_points_in_boxes(const float *pts, int n_cols, const int6
     ws.mat_cap = (long long)((workspace_bytes - head) / 4);
     ws.n_points = n_points;
     ws.n_boxes = n_boxes;
+    return ws;
+}
+
+// The size and pointer checks the crop entries share: FNP_OK, FNP_EINVAL or FNP_EWORKSPACE.
+static int crop_check(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                      const int64_t *box_start, int n_boxes, int n_frames, const int64_t *starts,
+                      const void *workspace, size_t workspace_bytes)
+{
+    if (n_cols < 3 || n_points < 0 || n_boxes < 0 || n_frames < 0 || n_frames > 65535 * 1024) return FNP_EINVAL;
+    if (n_frames == 0 && (n_points || n_boxes)) return FNP_EINVAL;
+    if (!row_start || !box_start || !starts || !workspace || (n_points && !pts) ||
+        (reinterpret_cast<uintptr_t>(workspace) & 15))
+        return FNP_EINVAL;
+    if (n_points / kCropTile + n_frames > 0x7fffffffLL || divup(n_boxes, 128) > 0x7fffffff) return FNP_EINVAL;
+    if (workspace_bytes < crop_head_bytes(n_points, n_frames) + 16) return FNP_EWORKSPACE;
+    return FNP_OK;
+}
+
+extern "C" int fnp_crop_all_count(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                                  const float *box_prep, const int64_t *box_start, int n_boxes, int n_frames,
+                                  int32_t *counts, int64_t *starts, void *workspace, size_t workspace_bytes,
+                                  void *stream)
+{
+    if (n_boxes > 0 && (!box_prep || !counts)) return FNP_EINVAL;
+    const int rc = crop_check(pts, n_cols, row_start, n_points, box_start, n_boxes, n_frames, starts, workspace,
+                              workspace_bytes);
+    if (rc != FNP_OK) return rc;
+    cudaStream_t s = (cudaStream_t)stream;
+    const CropWs ws = crop_carve(workspace, workspace_bytes, n_points, n_boxes, n_frames);
+    const long long n_tiles = n_points / kCropTile + n_frames;
+    const cudaError_t e = cudaMemsetAsync(ws.mat, 0, workspace_bytes - crop_head_bytes(n_points, n_frames), s);
+    if (e != cudaSuccess) return (int)e;
+    crop_plan_kernel<<<1, kCropScanThreads, 0, s>>>(row_start, box_start, n_frames, ws);
+    FNP_LAUNCH_CHECK();
+    if (n_tiles > 0 && n_boxes > 0)
+        crop_all_count_kernel<<<(unsigned)n_tiles, kCropThreads, 0, s>>>(pts, n_cols, row_start, box_prep, box_start,
+                                                                         n_frames, ws);
+    FNP_LAUNCH_CHECK();
+    if (n_boxes > 0)
+        crop_prefix_kernel<<<divup(n_boxes, 128), 128, 0, s>>>(row_start, box_start, n_frames, n_boxes, ws, counts);
+    FNP_LAUNCH_CHECK();
+    crop_starts_kernel<<<1, kCropScanThreads, 0, s>>>(counts, n_boxes, starts);
+    FNP_LAUNCH_CHECK();
+    return FNP_OK;
+}
+
+extern "C" int fnp_crop_all_scatter(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                                    const float *box_prep, const double *centres, const int64_t *box_start,
+                                    int n_boxes, int n_frames, const int64_t *starts, float *rows, long long rows_cap,
+                                    void *workspace, size_t workspace_bytes, void *stream)
+{
+    if ((n_boxes > 0 && (!box_prep || !centres)) || rows_cap < 0 || (rows_cap > 0 && !rows)) return FNP_EINVAL;
+    const int rc = crop_check(pts, n_cols, row_start, n_points, box_start, n_boxes, n_frames, starts, workspace,
+                              workspace_bytes);
+    if (rc != FNP_OK) return rc;
+    const CropWs ws = crop_carve(workspace, workspace_bytes, n_points, n_boxes, n_frames);
+    const long long n_tiles = n_points / kCropTile + n_frames;
+    if (n_tiles > 0 && n_boxes > 0 && rows_cap > 0)
+        crop_all_scatter_kernel<<<(unsigned)n_tiles, kCropThreads, 0, (cudaStream_t)stream>>>(
+            pts, n_cols, row_start, box_prep, centres, box_start, n_frames, ws, starts, rows, rows_cap);
+    FNP_LAUNCH_CHECK();
+    return FNP_OK;
+}
+
+extern "C" int fnp_crop_points_in_boxes(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                                        const float *boxes, const double *centres, const int64_t *box_start,
+                                        int n_boxes, int n_frames, int32_t *counts, int64_t *starts, float *rows,
+                                        void *workspace, size_t workspace_bytes, void *stream)
+{
+    if ((n_boxes > 0 && (!boxes || !centres || !counts)) || (n_points > 0 && n_boxes > 0 && !rows)) return FNP_EINVAL;
+    const int rc = crop_check(pts, n_cols, row_start, n_points, box_start, n_boxes, n_frames, starts, workspace,
+                              workspace_bytes);
+    if (rc != FNP_OK) return rc;
+    const long long n_tiles = n_points / kCropTile + n_frames;
+    const size_t head = crop_head_bytes(n_points, n_frames);
+    cudaStream_t s = (cudaStream_t)stream;
+    const CropWs ws = crop_carve(workspace, workspace_bytes, n_points, n_boxes, n_frames);
     const cudaError_t e = cudaMemsetAsync(ws.mat, 0, workspace_bytes - head, s);
     if (e != cudaSuccess) return (int)e;
     crop_plan_kernel<<<1, kCropScanThreads, 0, s>>>(row_start, box_start, n_frames, ws);

@@ -13,6 +13,9 @@ calibration_kitti.Calibration (numpy: lidar_to_rect, rect_to_img,  Calibration
 KittiDataset.get_fov_flag (FOV_POINTS_ONLY)                         fov_flag
 common_utils.drop_info_with_name (DontCare)                        KittiFeed._load_gt
 box_utils.boxes3d_kitti_camera_to_lidar                             boxes3d_kitti_camera_to_lidar
+box_utils.boxes3d_lidar_to_kitti_camera,                            boxes3d_lidar_to_kitti_camera,
+  boxes3d_to_corners3d_kitti_camera,                                  boxes3d_to_corners3d_kitti_camera,
+  boxes3d_kitti_camera_to_imageboxes                                  boxes3d_kitti_camera_to_imageboxes
 KittiDataset.__getitem__                                            KittiFeed.__getitem__
 DatasetTemplate.prepare_data, training mode with an empty           KittiFeed._prepare_gt (NuScenesFeed's)
   augmentation list: heading wrap, class filter, class column,        and __getitem__: x / y range mask of the
@@ -95,6 +98,58 @@ def boxes3d_kitti_camera_to_lidar(boxes3d_camera: np.ndarray, calib: Calibration
     xyz_lidar = calib.rect_to_lidar(xyz)
     xyz_lidar[:, 2] += h[:, 0] / 2
     return np.concatenate([xyz_lidar, l, w, h, -(r + np.pi / 2)], axis=-1)
+
+
+def boxes3d_lidar_to_kitti_camera(boxes3d_lidar: np.ndarray, calib: Calibration) -> np.ndarray:
+    """box_utils.boxes3d_lidar_to_kitti_camera, the inverse of boxes3d_kitti_camera_to_lidar: (N,7) [x, y, z, dx, dy,
+    dz, heading] in the LiDAR frame -> (N,7) [x, y, z, l, h, w, ry] in the rectified camera frame, z at the bottom."""
+    b = copy.deepcopy(boxes3d_lidar)
+    xyz_lidar = b[:, 0:3]
+    l, w, h = b[:, 3:4], b[:, 4:5], b[:, 5:6]
+    r = b[:, 6:7]
+    xyz_lidar[:, 2] -= h.reshape(-1) / 2
+    xyz_cam = calib.lidar_to_rect(xyz_lidar)
+    r = -r - np.pi / 2
+    return np.concatenate([xyz_cam, l, h, w, r], axis=-1)
+
+
+def boxes3d_to_corners3d_kitti_camera(boxes3d: np.ndarray) -> np.ndarray:
+    """box_utils.boxes3d_to_corners3d_kitti_camera (bottom_center=True): (N,7) camera boxes -> (N,8,3) float32."""
+    n = boxes3d.shape[0]
+    l, h, w = boxes3d[:, 3], boxes3d[:, 4], boxes3d[:, 5]
+    x_corners = np.array([l / 2., l / 2., -l / 2., -l / 2., l / 2., l / 2., -l / 2., -l / 2], dtype=np.float32).T
+    z_corners = np.array([w / 2., -w / 2., -w / 2., w / 2., w / 2., -w / 2., -w / 2., w / 2.], dtype=np.float32).T
+    y_corners = np.zeros((n, 8), dtype=np.float32)
+    y_corners[:, 4:8] = -h.reshape(n, 1).repeat(4, axis=1)
+    ry = boxes3d[:, 6]
+    zeros, ones = np.zeros(ry.size, dtype=np.float32), np.ones(ry.size, dtype=np.float32)
+    rot_list = np.array([[np.cos(ry), zeros, -np.sin(ry)],
+                         [zeros, ones, zeros],
+                         [np.sin(ry), zeros, np.cos(ry)]])                      # (3, 3, N)
+    R_list = np.transpose(rot_list, (2, 0, 1))                                   # (N, 3, 3)
+    temp_corners = np.concatenate((x_corners.reshape(-1, 8, 1), y_corners.reshape(-1, 8, 1),
+                                   z_corners.reshape(-1, 8, 1)), axis=2)         # (N, 8, 3)
+    rotated = np.matmul(temp_corners, R_list)
+    x = boxes3d[:, 0].reshape(-1, 1) + rotated[:, :, 0].reshape(-1, 8)
+    y = boxes3d[:, 1].reshape(-1, 1) + rotated[:, :, 1].reshape(-1, 8)
+    z = boxes3d[:, 2].reshape(-1, 1) + rotated[:, :, 2].reshape(-1, 8)
+    corners = np.concatenate((x.reshape(-1, 8, 1), y.reshape(-1, 8, 1), z.reshape(-1, 8, 1)), axis=2)
+    return corners.astype(np.float32)
+
+
+def boxes3d_kitti_camera_to_imageboxes(boxes3d: np.ndarray, calib: Calibration, image_shape=None) -> np.ndarray:
+    """box_utils.boxes3d_kitti_camera_to_imageboxes: the (N,4) [u1, v1, u2, v2] image box around the eight corners of
+    each (N,7) camera box; with image_shape (H, W), u clipped to [0, W-1] and v to [0, H-1]."""
+    corners3d = boxes3d_to_corners3d_kitti_camera(boxes3d)
+    pts_img, _ = calib.rect_to_img(corners3d.reshape(-1, 3))
+    corners_in_image = pts_img.reshape(-1, 8, 2)
+    boxes2d_image = np.concatenate([np.min(corners_in_image, axis=1), np.max(corners_in_image, axis=1)], axis=1)
+    if image_shape is not None:
+        boxes2d_image[:, 0] = np.clip(boxes2d_image[:, 0], a_min=0, a_max=image_shape[1] - 1)
+        boxes2d_image[:, 1] = np.clip(boxes2d_image[:, 1], a_min=0, a_max=image_shape[0] - 1)
+        boxes2d_image[:, 2] = np.clip(boxes2d_image[:, 2], a_min=0, a_max=image_shape[1] - 1)
+        boxes2d_image[:, 3] = np.clip(boxes2d_image[:, 3], a_min=0, a_max=image_shape[0] - 1)
+    return boxes2d_image
 
 
 class KittiFeed:

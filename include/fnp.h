@@ -95,6 +95,33 @@ int fnp_crop_points_in_boxes(const float *pts, int n_cols, const int64_t *row_st
  * negative n_frames or a missing pointer. */
 size_t fnp_crop_workspace_bytes(const int64_t *row_start_host, const int64_t *box_start_host, int n_frames);
 
+/* Every-box crop, by the predicate of points_in_boxes_cpu (the crop of KittiDataset.create_groundtruth_database:
+ * points[point_indices[i] > 0], then xyz minus the box centre).  A point is written once for every box of its own
+ * frame that contains it, so the number of rows is known only after counting: two calls, on one stream, with the
+ * same arguments and workspace (sized by fnp_crop_workspace_bytes, left untouched between them).
+ *   pts, row_start, box_start, centres: as for fnp_crop_points_in_boxes.
+ *   box_prep (n_boxes, 8) f32 device = fnp_host_prep_boxes_cpu of the boxes cast to float32; each (point, box)
+ *   test gives the bits of fnp_points_in_boxes_matrix.
+ * fnp_crop_all_count writes counts (n_boxes) int32 and starts (n_boxes+1) int64, starts[n_boxes] = the rows needed.
+ * fnp_crop_all_scatter then writes rows (rows_cap, n_cols) f32: box b's points are rows starts[b] ..
+ * starts[b]+counts[b], in input order, x y z as (float)((double)p - centre), the other columns copied; no row at
+ * or past rows_cap is written.  Positions come from per-(tile, box) counts summed from warp ballots, a scan over
+ * the tiles, and a ballot rank in row order: no atomic picks one, and two runs give the same bytes.  No cap on
+ * points or boxes per frame.  Starts that do not end at n_points / n_boxes, or a workspace too small for the
+ * per-tile part, leave every count 0 and write no row (checked on the device).  FNP_EINVAL / FNP_EWORKSPACE as for
+ * fnp_crop_points_in_boxes, and for a negative rows_cap or a missing rows with rows_cap > 0, before any launch.
+ * Build record (nvcc 12.9, -Xptxas -v, sm_100a), no stack, no spills: crop_all_count_kernel 256 threads,
+ * 33 registers, 16384 bytes of shared memory; crop_all_scatter_kernel 256 threads (one warp per box of the
+ * tile), 40 registers, 12288 bytes of shared memory.  The plan, prefix and starts kernels are
+ * fnp_crop_points_in_boxes'. */
+int fnp_crop_all_count(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                       const float *box_prep, const int64_t *box_start, int n_boxes, int n_frames,
+                       int32_t *counts, int64_t *starts, void *workspace, size_t workspace_bytes, void *stream);
+int fnp_crop_all_scatter(const float *pts, int n_cols, const int64_t *row_start, long long n_points,
+                         const float *box_prep, const double *centres, const int64_t *box_start, int n_boxes,
+                         int n_frames, const int64_t *starts, float *rows, long long rows_cap,
+                         void *workspace, size_t workspace_bytes, void *stream);
+
 /* The (N, P) 0/1 matrix of the reference's CPU op points_in_boxes_cpu (roiaware_pool3d.cpp:121-168): NOT
  * the GPU predicate -- the margin is 1e-2 instead of 1e-5 and the products are rounded individually, with
  * the host libm's cosf / sinf.  box_prep (N,8) device = fnp_host_prep_boxes_cpu(boxes) uploaded (the per-box
