@@ -131,6 +131,10 @@ lib.fnp_seeker_cell_mask_bytes.restype = C.c_size_t
 lib.fnp_seeker_cell_mask_bytes.argtypes = [C.POINTER(SeekerCfg), _i, _i]
 lib.fnp_seg_nms_rotated.restype = _i
 lib.fnp_seg_nms_rotated.argtypes = [_vp, _vp, _vp, _vp, _vp, _i, _i, _f, _vp, _vp]
+SEG_NMS_MAX_THRESH = 8
+lib.fnp_seg_nms_rotated_multi.restype = _i
+lib.fnp_seg_nms_rotated_multi.argtypes = [_vp, C.c_longlong, _vp, C.c_longlong, _vp, _vp, _i, _i, _i, C.POINTER(_f), _i,
+                                          _vp, C.c_longlong, _vp]
 SELECT_MAX_SETTINGS = 256
 lib.fnp_seeker_select_multi.restype = _i
 lib.fnp_seeker_select_multi.argtypes = [C.POINTER(SeekerCfg), C.POINTER(SeekerBatch), C.POINTER(SelectSetting), _i,
@@ -176,7 +180,7 @@ EXPORTED = [
     "fnp_boxes_overlap_bev",
     "fnp_boxes_iou_bev", "fnp_boxes_aligned_overlap_bev", "fnp_nms_workspace_bytes", "fnp_nms_rotated",
     "fnp_nms_normal", "fnp_seeker_cull", "fnp_seeker_frustum_stats", "fnp_seeker_hypotheses",
-    "fnp_seeker_score", "fnp_seeker_score_mode", "fnp_seeker_occlusion", "fnp_seeker_select", "fnp_seeker_run", "fnp_seg_nms_rotated", "fnp_seeker_mask_words", "fnp_seeker_cell_mask_bytes",
+    "fnp_seeker_score", "fnp_seeker_score_mode", "fnp_seeker_occlusion", "fnp_seeker_select", "fnp_seeker_run", "fnp_seg_nms_rotated", "fnp_seg_nms_rotated_multi", "fnp_seeker_mask_words", "fnp_seeker_cell_mask_bytes",
     "fnp_recall_counters", "fnp_precision_counters", "fnp_quality_counters", "fnp_quality_smem_bytes",
     "fnp_seeker_select_multi", "fnp_host_select_candidates", "fnp_host_pack_xyz", "fnp_host_pack_xyz_begin",
     "fnp_host_pack_wait", "fnp_host_nms_order", "fnp_host_pack_xyz_multi_begin", "fnp_host_plan_sizes", "fnp_host_plan",

@@ -462,20 +462,48 @@ __global__ void __launch_bounds__(kScanThreads) nms_scan_kernel(const unsigned l
 // ======================================================================================
 // Stage 4: batched per-segment rotated NMS entirely in shared memory
 // ======================================================================================
-__global__ void __launch_bounds__(256) seg_nms_kernel(const float *__restrict__ boxes, const int32_t *__restrict__ label,
+constexpr int kSegNmsMaxThresh = 8;          // one scan warp per threshold of a 256-thread CTA
+constexpr size_t kSegNmsSmemBudget = 227 * 1024;   // sm_100's opt-in shared memory per block
+struct SegNmsThresh {
+    float t[kSegNmsMaxThresh];
+};
+
+// Dynamic shared memory of seg_nms_kernel for segments of up to n boxes and `chunk` thresholds at a time: the boxes,
+// one n x ceil(n/64)-word bitmask and one removed-row of ceil(n/64) words per threshold, the labels.
+static size_t seg_nms_smem_bytes(int n, int chunk)
+{
+    const size_t cb = (size_t)divup(n, 64);
+    return (size_t)n * sizeof(RBox) + (size_t)chunk * n * cb * 8 + (size_t)(n + 2) * 4 + (size_t)chunk * cb * 8 + 16;
+}
+
+// One CTA per (segment, setting).  Setting s reads its boxes at boxes + 7 s box_stride and its flags at
+// valid + s valid_stride; order, seg_start and label are shared.  Each upper-triangle pair's IoU is computed once and
+// sets its bit in the mask of every threshold of the current chunk it exceeds; then warp w scans threshold c0 + w.
+// keep_mask != NULL (one setting, one threshold): keep_mask[src] = kept ? 1 : 0.  Otherwise
+// keep_valid[(t n_settings + s) keep_stride + src] = kept ? 0 : -1.  MULTI = false folds the threshold loops of
+// that case away at compile time: stage 4 of a 256-frame cfg2 batch (B200, 1000 W limit) took 0.0541 ms with them,
+// 0.0534 without, 0.0529 before the kernel took more than one threshold.
+template <bool MULTI>
+__global__ void __launch_bounds__(256) seg_nms_kernel(const float *__restrict__ boxes, long long box_stride,
+                                                      const int32_t *__restrict__ label,
                                                       const int32_t *__restrict__ order,
-                                                      const int32_t *__restrict__ valid,
-                                                      const int32_t *__restrict__ seg_start, float thresh,
-                                                      uint8_t *__restrict__ keep_mask)
+                                                      const int32_t *__restrict__ valid, long long valid_stride,
+                                                      const int32_t *__restrict__ seg_start, SegNmsThresh thr,
+                                                      int n_thresh, int chunk, uint8_t *__restrict__ keep_mask,
+                                                      int32_t *__restrict__ keep_valid, long long keep_stride)
 {
     extern __shared__ __align__(16) unsigned char smem[];
-    const int seg = blockIdx.x;
+    __shared__ float s_thr[kSegNmsMaxThresh];
+    if (!MULTI) n_thresh = chunk = 1;
+    const int seg = blockIdx.x, set = blockIdx.y;
     const int s0 = seg_start[seg], n = seg_start[seg + 1] - s0;
     if (n <= 0) return;
     const int cb = divup(n, 64);
+    boxes += 7 * set * box_stride;
+    if (valid) valid += set * valid_stride;
     RBox *s_rb = reinterpret_cast<RBox *>(smem);
     unsigned long long *s_mask = reinterpret_cast<unsigned long long *>(s_rb + n);
-    int *s_lab = reinterpret_cast<int *>(s_mask + (size_t)n * cb);
+    int *s_lab = reinterpret_cast<int *>(s_mask + (size_t)chunk * n * cb);
     unsigned long long *s_remv = reinterpret_cast<unsigned long long *>(s_lab + ((n + 1) & ~1));
     // entry i of the segment is box src(i) = order ? order[s0+i] : s0+i; label -1 = not a box
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
@@ -484,29 +512,49 @@ __global__ void __launch_bounds__(256) seg_nms_kernel(const float *__restrict__ 
         const bool ok = !valid || valid[src] >= 0;
         s_lab[i] = ok ? (label ? label[src] : 0) : -1;
     }
-    for (int i = threadIdx.x; i < cb; i += blockDim.x) s_remv[i] = 0ULL;
-    __syncthreads();
-    for (int w = threadIdx.x; w < n * cb; w += blockDim.x) s_mask[w] = 0ULL;
-    __syncthreads();
-    // bitmask, one (i, j) pair per thread iteration (the upper triangle of an n x n grid);
-    // far-apart pairs are dismissed without running the polygon clipper
-    const bool prefilter = thresh >= 0.f;
-    for (int p = threadIdx.x; p < n * n; p += blockDim.x) {
-        const int i = p / n, j = p - i * n;
-        if (j <= i || s_lab[i] < 0 || s_lab[i] != s_lab[j]) continue;
-        if (prefilter && surely_disjoint(s_rb[i], s_rb[j])) continue;
-        if (iou_bev(s_rb[i], s_rb[j]) > thresh) atomicOr(&s_mask[(size_t)i * cb + (j >> 6)], 1ULL << (j & 63));
+    // far-apart pairs (IoU exactly 0) are dismissed without running the polygon clipper when every threshold is >= 0
+    bool prefilter = true;
+#pragma unroll
+    for (int t = 0; t < kSegNmsMaxThresh; t++)
+        if (t < n_thresh) prefilter &= thr.t[t] >= 0.f;
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int t = 0; t < kSegNmsMaxThresh; t++) s_thr[t] = thr.t[t];
     }
-    __syncthreads();
-    if (threadIdx.x < 32) {
-        const int lane = threadIdx.x;
-        for (int i = 0; i < n; i++) {
-            const bool dead = ((s_remv[i >> 6] >> (i & 63)) & 1ULL) || s_lab[i] < 0;
-            if (!dead)
-                for (int j = (i >> 6) + lane; j < cb; j += 32) s_remv[j] |= s_mask[(size_t)i * cb + j];
-            __syncwarp();
-            if (lane == 0) keep_mask[order ? order[s0 + i] : s0 + i] = dead ? 0 : 1;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int c0 = 0; c0 < n_thresh; c0 += chunk) {
+        const int nc = min(chunk, n_thresh - c0);
+        for (int i = threadIdx.x; i < nc * cb; i += blockDim.x) s_remv[i] = 0ULL;
+        for (int w = threadIdx.x; w < nc * n * cb; w += blockDim.x) s_mask[w] = 0ULL;
+        __syncthreads();
+        // bitmasks, one (i, j) pair per thread iteration (the upper triangle of an n x n grid)
+        for (int p = threadIdx.x; p < n * n; p += blockDim.x) {
+            const int i = p / n, j = p - i * n;
+            if (j <= i || s_lab[i] < 0 || s_lab[i] != s_lab[j]) continue;
+            if (prefilter && surely_disjoint(s_rb[i], s_rb[j])) continue;
+            const float iou = iou_bev(s_rb[i], s_rb[j]);
+            unsigned long long *m = s_mask + (size_t)i * cb + (j >> 6);
+            for (int t = 0; t < nc; t++, m += (size_t)n * cb)
+                if (iou > (MULTI ? s_thr[c0 + t] : thr.t[0])) atomicOr(m, 1ULL << (j & 63));
         }
+        __syncthreads();
+        if (warp < nc) {
+            const unsigned long long *mask = s_mask + (size_t)warp * n * cb;
+            unsigned long long *remv = s_remv + warp * cb;
+            int32_t *plane = MULTI ? keep_valid + ((long long)(c0 + warp) * gridDim.y + set) * keep_stride : nullptr;
+            for (int i = 0; i < n; i++) {
+                const bool dead = ((remv[i >> 6] >> (i & 63)) & 1ULL) || s_lab[i] < 0;
+                if (!dead)
+                    for (int j = (i >> 6) + lane; j < cb; j += 32) remv[j] |= mask[(size_t)i * cb + j];
+                __syncwarp();
+                if (lane == 0) {
+                    const int src = order ? order[s0 + i] : s0 + i;
+                    if (MULTI) plane[src] = dead ? -1 : 0;
+                    else keep_mask[src] = dead ? 0 : 1;
+                }
+            }
+        }
+        __syncthreads();
     }
 }
 
@@ -1438,10 +1486,36 @@ extern "C" int fnp_seg_nms_rotated(const float *boxes, const int32_t *label, con
     if (n_segments < 0 || max_seg_boxes < 0 || max_seg_boxes > FNP_SEG_NMS_MAX) return FNP_EINVAL;
     if (n_segments == 0 || max_seg_boxes == 0) return FNP_OK;
     if (!boxes || !seg_start || !keep_mask) return FNP_EINVAL;
-    const int n = max_seg_boxes, cb = divup(n, 64);
-    const size_t smem = (size_t)n * sizeof(RBox) + (size_t)n * cb * 8 + (size_t)(n + 2) * 4 + (size_t)cb * 8 + 16;
-    cudaFuncSetAttribute(seg_nms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    seg_nms_kernel<<<n_segments, 256, smem, (cudaStream_t)stream>>>(boxes, label, order, valid, seg_start, thresh, keep_mask);
+    const size_t smem = seg_nms_smem_bytes(max_seg_boxes, 1);
+    SegNmsThresh thr = {{thresh}};
+    cudaFuncSetAttribute(seg_nms_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    seg_nms_kernel<false><<<n_segments, 256, smem, (cudaStream_t)stream>>>(boxes, 0, label, order, valid, 0, seg_start, thr, 1, 1,
+                                                                    keep_mask, nullptr, 0);
+    FNP_LAUNCH_CHECK();
+    return FNP_OK;
+}
+
+extern "C" int fnp_seg_nms_rotated_multi(const float *boxes, long long box_setting_stride, const int32_t *valid,
+                                         long long valid_setting_stride, const int32_t *order, const int32_t *seg_start,
+                                         int n_segments, int n_settings, int max_seg_boxes, const float *thresh_host,
+                                         int n_thresh, int32_t *keep_valid, long long keep_plane_stride, void *stream)
+{
+    if (n_segments < 0 || n_settings < 0 || max_seg_boxes < 0 || box_setting_stride < 0 || valid_setting_stride < 0 ||
+        keep_plane_stride < 0 || max_seg_boxes > FNP_SEG_NMS_MAX || n_thresh < 1 || n_thresh > kSegNmsMaxThresh ||
+        !thresh_host || n_settings > 65535)
+        return FNP_EINVAL;
+    if (n_segments == 0 || n_settings == 0 || max_seg_boxes == 0) return FNP_OK;
+    if (!boxes || !valid || !order || !seg_start || !keep_valid) return FNP_EINVAL;
+    SegNmsThresh thr = {};
+    for (int t = 0; t < n_thresh; t++) thr.t[t] = thresh_host[t];
+    // as many thresholds per pass over the pairs as the shared memory holds at max_seg_boxes (one always does)
+    int chunk = n_thresh;
+    while (chunk > 1 && seg_nms_smem_bytes(max_seg_boxes, chunk) > kSegNmsSmemBudget) chunk--;
+    const size_t smem = seg_nms_smem_bytes(max_seg_boxes, chunk);
+    cudaFuncSetAttribute(seg_nms_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    seg_nms_kernel<true><<<dim3(n_segments, n_settings), 256, smem, (cudaStream_t)stream>>>(
+        boxes, box_setting_stride, nullptr, order, valid, valid_setting_stride, seg_start, thr, n_thresh, chunk, nullptr,
+        keep_valid, keep_plane_stride);
     FNP_LAUNCH_CHECK();
     return FNP_OK;
 }

@@ -308,17 +308,20 @@ class OutLayout:
     (compacted hypothesis index, -1: unused), count; per candidate: npts, nvalid; status (include/fnp.h: 8 int32);
     the recall counters; the stage-4 keep flags.  Then, for S settings of evaluate_settings: boxes, score, best, count
     per setting and candidate, the recall and the precision counters per setting, and n_quality quality counters per
-    setting (quality.QualitySpec.n_counters)."""
+    setting (quality.QualitySpec.n_counters).  With n_nms NMS thresholds, last: the quality counters of every setting
+    after the NMS at each threshold, (n_nms, S, n_quality)."""
 
-    def __init__(self, F, T=1, S=0, n_quality=0):
+    def __init__(self, F, T=1, S=0, n_quality=0, n_nms=0):
         FT, NC, NP = F * T, SeekerEngine.N_COUNTERS, SeekerEngine.N_PRECISION
         self.regions, end = {}, 0            # name -> (byte offset, dtype, shape)
-        for name, dt, shape in (
-                ("boxes", _F32, (FT, 7)), ("score", _F32, (FT,)), ("best", _I32, (FT,)), ("count", _I32, (FT,)),
-                ("npts", _I32, (F,)), ("nvalid", _I32, (F,)), ("status", _I32, (8,)), ("recall", _I64, (NC,)),
-                ("keep", _U8, (FT,)), ("sel_boxes", _F32, (S, F, 7)), ("sel_score", _F32, (S, F)),
-                ("sel_best", _I32, (S, F)), ("sel_count", _I32, (S, F)), ("sel_recall", _I64, (S, NC)),
-                ("sel_precision", _I64, (S, NP)), ("quality", _I64, (S, n_quality))):
+        regions = [("boxes", _F32, (FT, 7)), ("score", _F32, (FT,)), ("best", _I32, (FT,)), ("count", _I32, (FT,)),
+                   ("npts", _I32, (F,)), ("nvalid", _I32, (F,)), ("status", _I32, (8,)), ("recall", _I64, (NC,)),
+                   ("keep", _U8, (FT,)), ("sel_boxes", _F32, (S, F, 7)), ("sel_score", _F32, (S, F)),
+                   ("sel_best", _I32, (S, F)), ("sel_count", _I32, (S, F)), ("sel_recall", _I64, (S, NC)),
+                   ("sel_precision", _I64, (S, NP)), ("quality", _I64, (S, n_quality))]
+        if n_nms:
+            regions.append(("nms_quality", _I64, (n_nms, S, n_quality)))
+        for name, dt, shape in regions:
             off = _align(end, dt.itemsize)
             self.regions[name] = (off, dt, shape)
             end = off + dt.itemsize * math.prod(shape)
@@ -610,13 +613,13 @@ class SeekerEngine:
         return {k: base + o for k, o in offs.items()}
 
     def execute(self, plan, points_dev, nms_thresh=None, gt=None, recall_thresh=(0.3, 0.5, 0.7), slot=0,
-                points_ready=None, settings=None, quality=None):
+                points_ready=None, settings=None, quality=None, settings_nms=()):
         """Enqueue the whole batch on the current stream.  points_dev: CUDA float32 tensor
         holding the rows of all frames back to back.  points_ready: optional CUDA event the
         kernels must wait for (the H2D copy of the points on another stream); the small
         metadata upload is issued *before* that wait so that it does not queue behind the
-        next step's point copy in the H2D engine.  settings, quality: see evaluate_settings.  Returns a
-        handle for `finish`."""
+        next step's point copy in the H2D engine.  settings, quality and settings_nms (evaluate_settings'
+        nms_thresh): see evaluate_settings.  Returns a handle for `finish`."""
         t0 = time.perf_counter()
         _lib.require_cuda(points_dev)
         assert points_dev.dtype == torch.float32 and points_dev.is_contiguous()
@@ -678,7 +681,7 @@ class SeekerEngine:
             # different streams at the same time (slot 0 keeps the plain names: debug_views reads them)
             sfx = "" if slot == 0 else "@%d" % slot
             ptr = {k: self.arena.get(k + sfx, v).data_ptr() for k, v in sizes.items()}
-            lay = OutLayout(F, self.T, S, quality.n_counters if quality is not None else 0)
+            lay = OutLayout(F, self.T, S, quality.n_counters if quality is not None else 0, len(settings_nms))
             out_dev = self.arena.get("out%d" % slot, lay.nbytes)
             ob = out_dev.data_ptr()
             b = _lib.SeekerBatch(
@@ -714,15 +717,18 @@ class SeekerEngine:
             self.launches += (9 + (mode == _lib.SCORE_SWEEP) + self.use_occl) if F and plan["n_tiles"] else 0
             handle = dict(plan=plan, batch=b, sp=sp, cap=cap, out_dev=out_dev, layout=lay, meta=meta,
                           tab_stride=tab_stride, planes=planes, has_nms=False, has_recall=False,
-                          recall_thresh=tuple(recall_thresh), n_settings=S, quality=None,
+                          recall_thresh=tuple(recall_thresh), n_settings=S, quality=None, settings_nms=(),
                           args=dict(plan=plan, points_dev=points_dev, nms_thresh=nms_thresh, gt=gt,
                                     recall_thresh=recall_thresh, slot=slot, points_ready=points_ready,
-                                    settings=settings, quality=quality))
+                                    settings=settings, quality=quality, settings_nms=settings_nms))
             if S and F:
                 self._select_multi(handle, b, sel, use_occl, gt, recall_thresh, stream)
                 if quality is not None and gt is not None:
                     self._quality(handle, gt, quality, stream)
                     handle["quality"] = quality
+                    if settings_nms:
+                        self._settings_nms(handle, gt, quality, settings_nms, sfx, stream)
+                        handle["settings_nms"] = tuple(settings_nms)
             if nms_thresh is not None and F:
                 self._stage4_nms(handle, float(nms_thresh), stream)
                 handle["has_nms"] = True
@@ -814,7 +820,28 @@ class SeekerEngine:
                        valid_stride=F, stream=stream)
         self.launches += 1
 
-    def evaluate_settings(self, plan, points_dev, gt, settings, recall_thresh=(0.3, 0.5, 0.7), quality=None):
+    def _settings_nms(self, handle, gt, spec, thresh, sfx, stream):
+        """Every setting's proposals after load_pseudos' NMS at each threshold: one fnp_seg_nms_rotated_multi launch in
+        stage-4 order (nms_order: a proposal's score is its candidate's 2D score) into keep planes of arena scratch,
+        then one fnp_quality_counters launch per threshold over that threshold's planes."""
+        from . import quality
+        plan, meta, lay, out_dev = handle["plan"], handle["meta"], handle["layout"], handle["out_dev"]
+        L, ob, F, S, NT = _lib.lib, out_dev.data_ptr(), plan["F"], handle["n_settings"], len(thresh)
+        gt_boxes, gt_start, max_gt = gt
+        keep = self.arena.get("nms_keep" + sfx, 4 * NT * S * F).data_ptr()
+        th = (C.c_float * NT)(*[float(t) for t in thresh])
+        _lib.check(L.fnp_seg_nms_rotated_multi(lay.ptr(ob, "sel_boxes"), F, lay.ptr(ob, "sel_best"), F, meta["nms_order"],
+                                               meta["frame_cand_start"], plan["B"], S, max(plan["max_cands"], 1), th, NT,
+                                               keep, F, stream), "fnp_seg_nms_rotated_multi")
+        out_dev[lay.span("nms_quality")].zero_()
+        for t in range(NT):
+            quality.launch(spec, lay.ptr(ob, "sel_boxes"), meta["cand_label"], meta["frame_cand_start"], gt_boxes,
+                           gt_start, plan["B"], max(plan["max_cands"], 1), int(max_gt), lay.ptr(ob, "nms_quality", t),
+                           n_settings=S, pred_valid=keep + 4 * t * S * F, pred_stride=F, valid_stride=F, stream=stream)
+        self.launches += 1 + NT
+
+    def evaluate_settings(self, plan, points_dev, gt, settings, recall_thresh=(0.3, 0.5, 0.7), quality=None,
+                          nms_thresh=()):
         """Scores several select-level settings on one batch: stages 1-2c run once with this engine's parameters, then
         stage 3 once per setting (fnp_seeker_select_multi), and its recall and precision counters.  settings: dicts of
         SELECT_KEYS (a key a setting leaves out takes this engine's value), any number of them: stage 3 runs for up to
@@ -825,11 +852,22 @@ class SeekerEngine:
         precision (proposals, then "hits_<t>": proposals with a GT IoU3D > t), and per candidate cand_best (index among
         the compacted hypotheses, -1: none), cand_score2, cand_count, cand_boxes.  quality (a quality.QualitySpec): one
         more launch, fnp_quality_counters over every setting, and each setting gains "quality", its flat counters
-        (quality.tables reads them).  One D2H; on a page-pool overflow the pool grows and the batch runs again."""
+        (quality.tables reads them).  nms_thresh (up to 8 thresholds, needs quality): each setting is also scored as
+        self-training reads it after load_pseudos(nms_thresh=t) -- one fnp_seg_nms_rotated_multi launch over every
+        setting and threshold, then one fnp_quality_counters launch per threshold -- and gains "nms", its flat quality
+        counters after the NMS at each threshold, in nms_thresh's order.  One D2H; on a page-pool overflow the pool
+        grows and the batch runs again."""
         if self.T != 1 or self.rand_center:
             raise NotImplementedError("evaluate_settings runs with topk = 1 and no rand_center")
         if not settings:
             raise ValueError("evaluate_settings needs at least one setting")
+        nms_thresh = tuple(float(t) for t in nms_thresh)
+        if nms_thresh and quality is None:
+            raise ValueError("evaluate_settings: nms_thresh needs a quality spec (the post-NMS numbers are quality "
+                             "counters)")
+        if len(nms_thresh) > _lib.SEG_NMS_MAX_THRESH:
+            raise ValueError("evaluate_settings: at most %d NMS thresholds, got %d"
+                             % (_lib.SEG_NMS_MAX_THRESH, len(nms_thresh)))
         for s in settings:
             iou = np.float32(s.get("min_cam_iou", self.p["min_cam_iou"]))
             if iou < np.float32(self.p["min_cam_iou"]):
@@ -842,7 +880,7 @@ class SeekerEngine:
             check_labels(quality, plan["cand_label"], gt[0].cpu().numpy(), gt[1].cpu().numpy())
             quality.check_size(plan["max_cands"], gt[2], "the largest frame of the batch")
         return self.result(self.execute(plan, points_dev, gt=gt, recall_thresh=recall_thresh, settings=settings,
-                                         quality=quality))
+                                         quality=quality, settings_nms=nms_thresh))
 
     def result(self, handle):
         """finish(handle), recovering from a page pool too small for the batch: the pool grows (pts_factor) and the
@@ -894,6 +932,7 @@ class SeekerEngine:
                 "sel_boxes", "sel_score", "sel_best", "sel_count", "sel_recall", "sel_precision", "quality"))
             th = handle["recall_thresh"]
             spec = handle.get("quality")
+            nq = lay.view(raw, "nms_quality") if handle["settings_nms"] else None
             res["settings"] = []
             for s in range(S):
                 d = dict(proposals=int((sbest[s] >= 0).sum()), cand_best=sbest[s].copy(), cand_score2=ss[s].copy(),
@@ -904,6 +943,8 @@ class SeekerEngine:
                                           **{"hits_%s" % t: int(prec[s, 1 + i]) for i, t in enumerate(th)})
                 if spec is not None:
                     d["quality"] = qc[s].copy()
+                if nq is not None:
+                    d["nms"] = [nq[t, s].copy() for t in range(nq.shape[0])]
                 res["settings"].append(d)
         self.host_s["finish"] += time.perf_counter() - t0
         return res

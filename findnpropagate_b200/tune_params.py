@@ -16,11 +16,17 @@ first-match counts over the valid set, so ``min_cam_iou`` splits groups and only
 For each setting the command prints one JSON line -- its values and group, the proposals, the recall counters, AR and
 precision at 0.3 / 0.5 / 0.7 -- sorted by AR@0.5, then the ``--set`` arguments that give the best setting to
 ``extract_pseudo_labels``.  The config, its refusals and the failed-frame rule are those of ``extract_pseudo_labels``.
+
+Self-training reads the proposals through ``load_pseudos(nms_thresh=T)``, a class-agnostic rotated BEV NMS in 2D-score
+order.  ``--nms_thresh T ...`` (up to 8 thresholds) scores every setting that way too: each line gains ``nms``, per
+threshold the proposals, recall counters, AR and precision ``eval_pseudo_labels --nms_thresh`` would print for the
+folder the setting extracts, and the lines are ranked by AR@0.5 after the first threshold's NMS.
 """
 import argparse
 import copy
 import itertools
 import json
+import math
 import os
 import sys
 
@@ -135,11 +141,12 @@ def group_settings(base_params, settings, variant="nuscenes"):
 
 
 def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, workers=4, box_format="xyxy", device=None,
-                  quality=None, variant="nuscenes"):
+                  quality=None, variant="nuscenes", nms_thresh=()):
     """Scores every setting over every frame of ``feed``: each batch is read once (NuScenesFeed / KittiFeed.prefetch)
     and uploaded once, then every group of ``group_settings`` runs on it (variant: the head's, as for SeekerEngine).  Returns (per setting dict(proposals, recall, precision)
     summed over the frames, groups).  quality (a quality.QualitySpec): each setting's dict also holds "quality", its
-    summed fnp_quality_counters counters."""
+    summed fnp_quality_counters counters.  nms_thresh (needs quality): and "nms", its summed counters after the NMS at
+    each threshold (SeekerEngine.evaluate_settings)."""
     import numpy as np
     import torch
     from .extract import THRESH, recall_keys
@@ -156,12 +163,14 @@ def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, worker
     if quality is not None:
         for t in totals:
             t["quality"] = np.zeros(quality.n_counters, np.int64)
+            t["nms"] = np.zeros((len(nms_thresh), quality.n_counters), np.int64)
     for frames, _, _ in feed.prefetch(range(len(feed)), detector, batch_frames=batch_frames, workers=workers,
                                       xyz_only=True):
         points = torch.from_numpy(np.concatenate([f.points for f in frames])).to(engines[0].device)
         gt = engines[0].upload_gt(frames)
         for g, eng in zip(groups, engines):
-            res = eng.evaluate_settings(eng.plan(frames), points, gt, g["settings"], recall_thresh=THRESH, quality=quality)
+            res = eng.evaluate_settings(eng.plan(frames), points, gt, g["settings"], recall_thresh=THRESH, quality=quality,
+                                        nms_thresh=nms_thresh)
             for i, r in zip(g["members"], res["settings"]):
                 t = totals[i]
                 t["proposals"] += r["proposals"]
@@ -171,6 +180,8 @@ def evaluate_grid(feed, detector, base_params, settings, batch_frames=64, worker
                     t["precision"][k] += v
                 if "quality" in r:
                     t["quality"] += r["quality"]
+                if "nms" in r:
+                    t["nms"] += np.stack(r["nms"])
     return totals, groups
 
 
@@ -188,6 +199,9 @@ def parse_args(argv=None):
                    help="add per class and range bin counters to each line (classes; see eval_pseudo_labels)")
     p.add_argument("--range_edges", type=float, nargs="*", default=[20.0, 30.0, 40.0],
                    help="with --breakdown: BEV range bin edges in metres (default: 20 30 40)")
+    p.add_argument("--nms_thresh", type=float, nargs="*", default=[],
+                   help="also score each setting after a rotated BEV NMS at each of these thresholds (as "
+                        "load_pseudos(nms_thresh=T)), at most 8; the lines are then ranked by AR@0.5 after the first")
     p.add_argument("--set", dest="set_cfgs", default=None, nargs=argparse.REMAINDER, metavar="KEY VALUE",
                    help="config overrides applied to every setting, e.g. --set DATA_CONFIG.MAX_SWEEPS 1")
     return p.parse_args(argv)
@@ -205,6 +219,15 @@ def main(argv=None):
         _fail("tune_params runs in one process: start it without torchrun")
     if args.every < 1:
         _fail("--every must be at least 1")
+    nms = [float(t) for t in args.nms_thresh]
+    from ._lib import SEG_NMS_MAX_THRESH
+    if len(nms) > SEG_NMS_MAX_THRESH:
+        _fail("--nms_thresh takes at most %d thresholds, got %d: %s" % (SEG_NMS_MAX_THRESH, len(nms), nms))
+    for i, t in enumerate(nms):
+        if not math.isfinite(t):
+            _fail("--nms_thresh %s: the thresholds must be finite" % t)
+        if t in nms[:i]:
+            _fail("--nms_thresh %s is given twice" % t)
     from .proposer import head_params, kitti_head_params
     try:
         cfg = load_config(args.cfg_file, args.set_cfgs)
@@ -217,7 +240,7 @@ def main(argv=None):
         base = (kitti_head_params if kitti else head_params)(cfg.MODEL.DENSE_HEAD)
         groups = group_settings(base, settings, variant)
         spec = None
-        if args.breakdown:
+        if args.breakdown or nms:
             from .kitti_feed import CLASS_NAMES as KITTI_CLASS_NAMES
             from .nuscenes_feed import CLASS_NAMES
             from .quality import QualitySpec
@@ -239,18 +262,28 @@ def main(argv=None):
     print("frames scored: %d, failed frames: %d" % (len(feed), sum(1 for c in codes if c)))
     totals, groups = evaluate_grid(feed, head.image_detector, base, settings, batch_frames=args.batch_frames,
                                    workers=args.workers, box_format=head.engine.box_format, device=device,
-                                   quality=spec, variant=variant)
+                                   quality=spec, variant=variant, nms_thresh=nms)
     group_of = {i: gi for gi, g in enumerate(groups) for i in g["members"]}
+    from .quality import summary, tables
     lines = []
     for i, (s, t) in enumerate(zip(grid, totals)):
         rec, n_gt, n_prop = t["recall"], max(t["recall"]["gt"], 1), max(t["proposals"], 1)
         lines.append(dict(setting=s, group=group_of[i], proposals=t["proposals"], recall=rec,
                           ar={str(th): rec["rcnn_%s" % th] / n_gt for th in extract.THRESH},
                           precision={str(th): t["precision"]["hits_%s" % th] / n_prop for th in extract.THRESH}))
-        if spec is not None:
-            from .quality import tables
+        if args.breakdown:
             lines[-1]["classes"] = tables(t["quality"], spec)
-    lines.sort(key=lambda d: -d["ar"]["0.5"])       # stable: equal AR keeps grid order
+        if nms:
+            lines[-1]["nms"] = {}
+            for th, c in zip(nms, t["nms"]):
+                d = lines[-1]["nms"][str(th)] = summary(c, spec)
+                if args.breakdown:
+                    d["classes"] = tables(c, spec)
+    # stable: equal AR keeps grid order; with --nms_thresh, the AR self-training sees after the first threshold's NMS
+    if nms:
+        lines.sort(key=lambda d: -d["nms"][str(nms[0])]["ar"]["0.5"])
+    else:
+        lines.sort(key=lambda d: -d["ar"]["0.5"])
     text = [json.dumps(d) for d in lines]
     for t in text:
         print(t)
@@ -265,8 +298,9 @@ def main(argv=None):
         else:
             print("best %s = %r: the config has no %s, add %s: %r to it (--set cannot add a key)"
                   % (key, best[key], key, name, best[key]))
-    print("best setting: python -m findnpropagate_b200.extract_pseudo_labels --cfg_file %s --folder <folder>%s"
-          % (args.cfg_file, (" --set " + " ".join('"%s"' % a for a in set_args)) if set_args else ""))
+    print("best setting%s: python -m findnpropagate_b200.extract_pseudo_labels --cfg_file %s --folder <folder>%s"
+          % (" (ranked by AR@0.5 after the NMS at %s)" % nms[0] if nms else "", args.cfg_file,
+             (" --set " + " ".join('"%s"' % a for a in set_args)) if set_args else ""))
     return lines
 
 

@@ -394,6 +394,29 @@ int fnp_seg_nms_rotated(const float *boxes, const int32_t *label, const int32_t 
                         const int32_t *valid, const int32_t *seg_start, int n_segments,
                         int max_seg_boxes, float thresh, uint8_t *keep_mask, void *stream);
 
+/* Stage 4 for many settings and thresholds in one launch, class-agnostic (the NMS of load_pseudos), for scoring each
+ * setting of fnp_seeker_select_multi after the NMS self-training applies.  Setting s reads its boxes at
+ * boxes + 7 * s * box_setting_stride and its flags at valid + s * valid_setting_stride (entries < 0 are not boxes);
+ * order and seg_start (n_segments+1) are shared by every setting, as in fnp_seg_nms_rotated.  thresh_host is a HOST
+ * array of n_thresh (1..8) thresholds.  For every threshold t, setting s and box i of a segment the call writes
+ *   keep_valid[(t * n_settings + s) * keep_plane_stride + i] = 0 when the box is kept, -1 when it is suppressed or
+ *   is not a box
+ * -- the pred_valid plane fnp_quality_counters reads.  Each plane equals, bit for bit, fnp_seg_nms_rotated(setting s's
+ * boxes, NULL, order, setting s's valid, seg_start, n_segments, max_seg_boxes, thresh_host[t]) with its keep_mask
+ * mapped 1 -> 0, 0 -> -1: the same kernel source (seg_nms_kernel), one CTA per (segment, setting).  Each pair's IoU is
+ * computed once and sets its bit in the mask of every threshold it exceeds; warp w of the CTA scans threshold w.
+ * The masks of all thresholds live in shared memory when they fit 227 KB at max_seg_boxes (8 thresholds up to 448
+ * boxes, 6 at 512, 1 at 1024); otherwise the CTA takes the thresholds in chunks that fit and runs the pair loop once per chunk.
+ * Far-apart pairs skip the polygon clipper only when every threshold is >= 0.  Build record (nvcc 12.9,
+ * -Xptxas -v, sm_100a): seg_nms_kernel<true> (this call; <false> is fnp_seg_nms_rotated's, the same source with the
+ * threshold loops folded away) 256 threads, 64 registers, 192-byte stack frame (box_overlap's vertex arrays), no
+ * spills, 32 bytes of static shared memory (the thresholds); <false> the same without the static shared memory.  FNP_EINVAL: a negative size or stride, max_seg_boxes >
+ * FNP_SEG_NMS_MAX, n_thresh outside 1..8, n_settings > 65535, a missing pointer. */
+int fnp_seg_nms_rotated_multi(const float *boxes, long long box_setting_stride, const int32_t *valid,
+                              long long valid_setting_stride, const int32_t *order, const int32_t *seg_start,
+                              int n_segments, int n_settings, int max_seg_boxes, const float *thresh_host, int n_thresh,
+                              int32_t *keep_valid, long long keep_plane_stride, void *stream);
+
 /* Recall counters (Detector3DTemplate.generate_recall_record): per frame, IoU3D of the
  * proposals vs GT, per-GT max, thresholded.  pred (sum K,7) with pred_start (n_frames+1),
  * pred_valid (nullable): rows with pred_valid[i] < 0 are skipped;
